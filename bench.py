@@ -18,6 +18,11 @@ times and the thing that limits it:
                   verify split by equation over the N GPUs (configs[3])
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--proofs P] [--skip c3,c4,weak] [--impl reference]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed C5 path returned in its last step as DIR/<name>.npy (float32): the per-proof
+verdicts of gs_verify_batch_dev and the one verdict of gs_verify_batch_rand_dev.  Inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 
 Prints ONE JSON line (see the task contract): value = verifies/s with inputs resident in HBM, e2e = the same
 through the C ABI with host buffers (H2D + D2H inside the timed region), roofline = integer-multiply roofline of
@@ -34,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the tree may be read-only: leave no __pycache__ behind
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -351,6 +357,7 @@ def bench_c5(R_, eng, P, distinct, steps, warmup, full):
     sampler.begin()
     ms_total = timed(step_dev, steps)
     sampler.end()
+    out["verdicts"] = (torch.cat(gathered) if R_.world > 1 else ok_dev).cpu().numpy()    # the last timed step's answer
     out["launches"] = eng.launch_count - l0
     out["clocks"] = sampler.stop()
     out["ms_per_step"] = ms_total / steps
@@ -380,12 +387,11 @@ def bench_c5(R_, eng, P, distinct, steps, warmup, full):
     # ---- opt-in randomised batch verification (gs_verify_batch_rand, SURVEY.md 8f.4): ONE verdict per call.  Timed on the
     # honest proofs of this shard (a batch with a bad proof is rejected and then goes through the exact path above).
     try:
-        import secrets
         honest = torch.from_numpy(np.flatnonzero(expected == 1)).to(R_.dev)
         Ph = int(honest.numel())
         devh = [t.index_select(0, honest).contiguous() for t in dev]
         ok1 = torch.zeros(4, dtype=torch.uint8, device=R_.dev)
-        rho = secrets.token_bytes(8 * (2 * P + 1))
+        rho = np.random.default_rng(5 + R_.rank).bytes(8 * (2 * P + 1))   # seeded weights: the same inputs on every run
 
         def step_rand():
             eng.verify_batch_rand_dev(0, Ph, m, n, [t.data_ptr() for t in devh], ok1.data_ptr(), rho=rho[:8 * (2 * Ph + 1)])
@@ -398,6 +404,7 @@ def bench_c5(R_, eng, P, distinct, steps, warmup, full):
         accepts = int(ok1[0].item()) == 1
         l0 = eng.launch_count
         ms_rand = timed(step_rand, steps) / steps
+        verdict_rand = ok1[:1].cpu().numpy()
         launches = (eng.launch_count - l0) // steps
         eng.profile_enable(True)
         step_rand()
@@ -417,7 +424,8 @@ def bench_c5(R_, eng, P, distinct, steps, warmup, full):
         accepts = accepts and int(ok1h[0]) == 1
         e2e_rand = R_.wall_ms(step_rand_e2e, steps, warmup=0)
         out["rand"] = {"proofs": Ph, "ms_per_step": ms_rand, "e2e_ms": e2e_rand, "accepts_honest_batch": accepts,
-                       "rejects_batch_with_tampered": rejects, "launches_per_step": int(launches), "prof": prof_r}
+                       "rejects_batch_with_tampered": rejects, "launches_per_step": int(launches), "prof": prof_r,
+                       "verdict": verdict_rand}
         del devh, hosth
     except Exception as ex:  # noqa: BLE001 -- the opt-in leg must not take the headline down
         out["rand"] = {"error": f"{type(ex).__name__}: {ex}"}
@@ -626,11 +634,35 @@ def cpu_baseline_record(m, n):
     return rec
 
 
+DUMP_BYTES = 64 << 20
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"{s} is not a positive integer")
+    return v
+
+
+def dump_outputs(d, arrays):
+    """Each array as float32 d/<name>.npy, all of them within DUMP_BYTES: an array over its share is replaced by a fixed,
+    seeded sample of its elements, and d/<name>_index.npy (float64) holds the positions sampled."""
+    import numpy as np
+    share = DUMP_BYTES // len(arrays) - 4096                  # (room for the .npy headers)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32).ravel()
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // 12, replace=False))
+            np.save(os.path.join(d, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(d, f"{name}.npy"), a)
+
+
 # ---------------------------------------------------------------- GPU arm
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=positive_int, default=3, help="timed steps of every leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--proofs", type=int, default=65536, help="proofs per step in TOTAL (sharded over the GPUs)")
     ap.add_argument("--distinct", type=int, default=0, help="distinct proved instances per rank (0 = every proof distinct)")
@@ -640,9 +672,14 @@ def main():
     ap.add_argument("--skip", default="", help="comma list of sub-records to skip: weak,c3,c4")
     ap.add_argument("--c3-size", type=int, default=1024)
     ap.add_argument("--c4-eqs", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's C5 outputs as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the GPU path; it does not apply to --impl reference")
         return run_reference(args)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)       # fail before the run, not after it
 
     import groth_sahai_rs_b200 as gsb
     R_ = Ranks()
@@ -734,16 +771,16 @@ def main():
 
     if world > 1 and "weak" not in skip:
         def weak():
-            w = bench_c5(R_, eng, args.proofs, 4096, max(1, args.steps - 1), 1, full=False)
+            w = bench_c5(R_, eng, args.proofs, 4096, args.steps, 1, full=False)
             return {"workload": f"C5 weak: {args.proofs} proofs PER GPU (the round-1 headline)", "scaling": "weak", "n_gpus": world,
                     "value": round(world * args.proofs / (w["ms_per_step"] * 1e-3), 1), "unit": "verifies/s",
                     "ms_per_step": round(w["ms_per_step"], 3), "distinct_instances_per_gpu": 4096,
                     "limiter": "none: independent proofs, verdict bytes all-gathered"}
         sub("c5_weak", weak)
     if "c3" not in skip:
-        sub("c3_sharded", lambda: bench_c3_sharded(R_, eng, args.c3_size, max(2, args.steps)))
+        sub("c3_sharded", lambda: bench_c3_sharded(R_, eng, args.c3_size, args.steps))
     if "c4" not in skip:
-        sub("c4_by_equation", lambda: bench_c4_by_equation(R_, eng, args.c4_eqs, 2))
+        sub("c4_by_equation", lambda: bench_c4_by_equation(R_, eng, args.c4_eqs, args.steps))
 
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -791,6 +828,11 @@ def main():
         line.update(extras)
         if cpu is not None:
             line["cpu_baseline"] = cpu
+        if args.dump_outputs:
+            outs = {"c5_verdicts": c5["verdicts"]}
+            if rnd and "verdict" in rnd:
+                outs["c5_randomised_verdict"] = rnd["verdict"]
+            dump_outputs(args.dump_outputs, outs)
         print(json.dumps(line))
     if world > 1:
         R_.dist.destroy_process_group()
