@@ -49,7 +49,6 @@ struct gs_ctx {
                             // stream, so that partial waves of one half are filled by the other (GS_SPLIT_MIN; 0 = never)
   int lone_walk_jac = 1;    // lone statements walk their G2 points in Jacobian coordinates + one batched inversion
                             // (GS_LONE_WALK_JAC = 0: the affine walk with an inversion per step)
-  bool in_pass = false;     // set by a caller that already cut the batch into passes (verify_host): no second split inside
   int pass_streams = 2;   // verify passes of a big batch alternate between this many streams (GS_PASS_STREAMS = 1 | 2)
   int prep_variant = 5;   // resident blocks per SM the line-walk kernel is compiled for (GS_PREP_VARIANT = 4 | 5, experiments)
   size_t rand_pip_min = 4096;   // gs_verify_batch_rand: batches of at least this many proofs sum their pi / theta slots over the
@@ -117,37 +116,54 @@ struct Scratch {
     for (void* q : ptrs) cudaFreeAsync(q, home);
   }
 };
-// orders `main_s` after everything queued on `other` so far, on every exit path of the scope
-struct StreamJoin {
-  cudaStream_t main_s, other;
-  bool on;
-  ~StreamJoin() {
-    if (!on) return;
-    cudaEvent_t j;
-    if (cudaEventCreateWithFlags(&j, cudaEventDisableTiming) != cudaSuccess) {
-      cudaStreamSynchronize(other);
-      return;
-    }
-    cudaEventRecord(j, other);
-    cudaStreamWaitEvent(main_s, j, 0);
-    cudaEventDestroy(j);
-  }
-};
 // instances per verify pass: verify_batch_max for big batches; half of a medium batch (two streams fill each other's
-// partial waves -- the strong-scaling regime of C5: 8,192 proofs per GPU are 3.46 waves of k_miller4); else everything
-static inline size_t verify_pass_size(const gs_ctx* ctx, size_t count, bool shared_x) {
-  if (ctx->in_pass) return count;
+// partial waves -- the strong-scaling regime of C5: 8,192 proofs per GPU are 3.46 waves of k_miller4); else everything.
+// `one_pass`: the caller has already cut the batch into passes (verify_host), no second split inside
+static inline size_t verify_pass_size(const gs_ctx* ctx, size_t count, bool shared_x, bool one_pass) {
+  if (one_pass) return count;
   if (count > ctx->verify_batch_max) return ctx->verify_batch_max;
   if (ctx->pass_streams == 2 && !ctx->profile && !shared_x && ctx->split_min && count >= ctx->split_min)
     return (((count + 1) / 2) + 31) / 32 * 32;
   return count;
 }
-// restores ctx->stream on every exit path of a function that switches it
-struct StreamGuard {
+// The passes of a big batch, alternating between ctx->stream and the context's second stream.  On every exit path of the
+// scope ctx->stream is restored and, once split() has run, ordered after everything queued on the second stream.
+struct PassStreams {
   gs_ctx* ctx;
-  cudaStream_t saved;
-  explicit StreamGuard(gs_ctx* c) : ctx(c), saved(c->stream) {}
-  ~StreamGuard() { ctx->stream = saved; }
+  cudaStream_t s[2];
+  bool two = false;
+  explicit PassStreams(gs_ctx* c) : ctx(c), s{c->stream, c->stream} {}
+  // odd passes run on the second stream (created on first use); with `fork` it first waits for everything queued on the
+  // main stream so far (inputs uploaded or produced there)
+  cudaError_t split(bool fork) {
+    if (!ctx->stream2) {
+      cudaError_t e = cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking);
+      if (e != cudaSuccess) return e;
+    }
+    s[1] = ctx->stream2;
+    two = true;
+    if (!fork) return cudaSuccess;
+    cudaEvent_t ev;
+    cudaError_t e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e != cudaSuccess) return e;
+    cudaEventRecord(ev, s[0]);
+    cudaStreamWaitEvent(s[1], ev, 0);
+    cudaEventDestroy(ev);
+    return cudaSuccess;
+  }
+  void use(size_t pass) { ctx->stream = s[pass & 1]; }
+  ~PassStreams() {
+    ctx->stream = s[0];
+    if (!two) return;
+    cudaEvent_t j;
+    if (cudaEventCreateWithFlags(&j, cudaEventDisableTiming) != cudaSuccess) {
+      cudaStreamSynchronize(s[1]);
+      return;
+    }
+    cudaEventRecord(j, s[1]);
+    cudaStreamWaitEvent(s[0], j, 0);
+    cudaEventDestroy(j);
+  }
 };
 
 template <class T>

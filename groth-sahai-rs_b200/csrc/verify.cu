@@ -780,6 +780,7 @@ __global__ void k_rand_place_pi(const g2_jac* __restrict__ sums, size_t stride, 
 
 }  // namespace gs
 
+
 // what the shape alone says about the G2 side of every slot (k_verify_assemble): CRS points have stored lines, iota_2
 // images have no first coordinate
 static std::vector<uint8_t> slot_kinds(const verify_shape& s) {
@@ -791,35 +792,44 @@ static std::vector<uint8_t> slot_kinds(const verify_shape& s) {
   return kind_all;
 }
 
-// The G1-side statement MSM of `nprob` problems into the X slots (k_verify_assemble has filled the others).
-static int statement_msm(gs_ctx* ctx, Scratch& sc, verify_shape s, const verify_args& v, size_t nprob, bool shared_x, g1_aff* X) {
+// the kinds of the slots k = rank, rank + world, ... that a sharded statement's rank owns
+static std::vector<uint8_t> owned_kinds(const std::vector<uint8_t>& kind_all, int rank, int world) {
+  std::vector<uint8_t> kind;
+  for (size_t k = rank; k < kind_all.size(); k += world) kind.push_back(kind_all[k]);
+  return kind;
+}
+
+// The G1-side statement MSM of `nprob` problems up to its chunk partials (this rank's bases, s.nb_own(), into the outputs
+// it owns): sets s.chunk and s.nchunk, *part = the s.nchunk partial sums.  The caller sums them with its last kernel.
+static int statement_msm_partials(gs_ctx* ctx, Scratch& sc, verify_shape& s, const verify_args& v, size_t nprob, bool shared_x,
+                                  const g1_jac** part_out) {
   // outputs that share one base coordinate: this rank's MSM outputs x the problems that use the same commitments
   const size_t owned_out = (size_t)s.n_out_owned();
   const size_t na = (size_t)s.na;
+  const size_t nb = (size_t)s.nb_own() * na;
   const bool use_wtab = (nprob == 1 || shared_x) && owned_out * nprob >= 320;  // table build ~ 14.6 ms at m = 1024
   {
     // bases per thread: few threads (one statement, or one rank's share of it) -> smaller chunks, so that the
     // grid is ~8 waves of the ~296 resident blocks instead of 1.7 (measured: 20.8 ms for half of C3's sums against
     // 30.8 ms for all of them; C4's shared-table batches 91 -> 67 ms); the table kernel has no doublings to
-    // amortise, Straus keeps >= 8.  Many chunks are folded 16 at a time (k_vmsm_fold) before k_vmsm_reduce.
+    // amortise, Straus keeps >= 8.  Many chunks are folded 16 at a time (k_vmsm_fold) before the last kernel.
     int chunk = GS_MSM_CHUNK;
     // (a lone small statement is pure latency: one base per thread there)
-    const bool tiny = nprob * owned_out * na * ((s.nbases + 7) / 8) < 16384;
+    const bool tiny = nprob * owned_out * na * ((s.nb_own() + 7) / 8) < 16384;
     const int floor_chunk = use_wtab ? 4 : (tiny ? 1 : 8);
-    while (chunk > floor_chunk && nprob * owned_out * na * ((s.nbases + chunk - 1) / chunk) < (size_t)128 * 2368) chunk /= 2;
+    while (chunk > floor_chunk && nprob * owned_out * na * ((s.nb_own() + chunk - 1) / chunk) < (size_t)128 * 2368) chunk /= 2;
     set_msm_chunk(s, chunk);
   }
   g1_jac* part;
   CUDA_TRY(sc.alloc(&part, (size_t)s.nchunk * s.n_out * na * nprob));
   if (use_wtab) {
-    const int nb = s.nb_own() * na;
     const wt_geom g = wt_choose(owned_out * nprob);
-    const size_t nrows = (size_t)nb * g.W;
+    const size_t nrows = nb * g.W;
     g1_aff* wtab;
     g1_jac* J;
     CUDA_TRY(sc.alloc(&wtab, nrows * g.H));
     CUDA_TRY(sc.alloc(&J, nrows * g.H));
-    LAUNCH(k_wtab_bases, (size_t)nb, s, v, ctx->crs, J, nb, g);
+    LAUNCH(k_wtab_bases, nb, s, v, ctx->crs, J, (int)nb, g);
     LAUNCH(k_jac_to_affine_blocks<1>, nrows, J, wtab, nrows, (size_t)g.H);
     LAUNCH(k_wtab_fill, nrows * (g.H / GS_WT_RUN), wtab, J, nrows, g.H);
     LAUNCH(k_jac_to_affine_blocks<8>, nrows * g.H / 8, J, wtab, nrows * g.H, (size_t)1);
@@ -827,42 +837,120 @@ static int statement_msm(gs_ctx* ctx, Scratch& sc, verify_shape s, const verify_
   } else {
     g1_aff* vtab;
     fp* vtabx;
-    CUDA_TRY(sc.alloc(&vtab, (size_t)s.nb_own() * na * GS_VTAB * nprob));
-    CUDA_TRY(sc.alloc(&vtabx, (size_t)s.nb_own() * na * GS_VTAB * nprob));
-    LAUNCH(k_vmsm_tables, nprob * (size_t)s.nb_own() * na, s, v, ctx->crs, vtab, vtabx, nprob);
+    CUDA_TRY(sc.alloc(&vtab, nb * GS_VTAB * nprob));
+    CUDA_TRY(sc.alloc(&vtabx, nb * GS_VTAB * nprob));
+    LAUNCH(k_vmsm_tables, nprob * nb, s, v, ctx->crs, vtab, vtabx, nprob);
     LAUNCH(k_vmsm_partial, nprob * owned_out * na * s.nchunk, s, v, vtab, vtabx, part, nprob);
   }
-  const g1_jac* partr = part;
-  if (s.nchunk > 32) {  // fold 16 chunks at a time in parallel; k_vmsm_reduce then walks the few that are left
+  *part_out = part;
+  if (s.nchunk > 32) {  // fold 16 chunks at a time in parallel; the last kernel then walks the few that are left
     const int F = 16, ng = (s.nchunk + F - 1) / F;
     g1_jac* part2;
     CUDA_TRY(sc.alloc(&part2, (size_t)ng * s.n_out * na * nprob));
     LAUNCH(k_vmsm_fold, (size_t)s.n_out * na * nprob * ng, s, part, part2, nprob, s.nchunk, F, ng);
-    partr = part2;
+    *part_out = part2;
     s.nchunk = ng;
   }
-  LAUNCH(k_vmsm_reduce, nprob * owned_out * na, s, v, partr, X, nprob);
   return GS_OK;
+}
+
+// ---- the eight input arrays of a verify call as one verify_args (host or device addresses)
+static verify_args args_of(const void* a_consts, const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
+                           const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta) {
+  verify_args v;
+  v.a_consts = a_consts;
+  v.b_consts = b_consts;
+  v.gamma = (const fr*)gamma;
+  v.target = target;
+  v.xcoms = (const g1_aff*)xcoms;
+  v.ycoms = (const g2_aff*)ycoms;
+  v.pi = (const g2_aff*)pi;
+  v.theta = (const g1_aff*)theta;
+  return v;
+}
+
+// the arrays from problem `off` on (Gamma holds s.gm rows per problem)
+static verify_args args_at(const verify_shape& s, const verify_args& v, size_t off) {
+  verify_args o = v;
+  o.a_consts = (const char*)v.a_consts + off * s.n * elem_size_A(s.type);
+  o.b_consts = (const char*)v.b_consts + off * s.m * elem_size_B(s.type);
+  o.gamma = v.gamma + off * s.gm * s.n;
+  o.target = (const char*)v.target + off * elem_size_T(s.type);
+  o.xcoms = v.xcoms + off * s.m * 2;
+  o.ycoms = v.ycoms + off * s.n * 2;
+  o.pi = v.pi + off * s.cx * 2;
+  o.theta = v.theta + off * s.cy * 2;
+  return o;
+}
+
+// device copies of problems [off, off + cnt) of the host arrays `h`, on ctx->stream
+static int upload_args(gs_ctx* ctx, Scratch& sc, const verify_shape& s, const verify_args& h, size_t off, size_t cnt, verify_args* d) {
+  const verify_args a = args_at(s, h, off);
+  uint8_t *dA, *dB, *dT;
+  fr* dG;
+  g1_aff *dc, *dth;
+  g2_aff *dd, *dpi;
+  CUDA_TRY(upload(ctx, sc, &dA, a.a_consts, cnt * s.n * elem_size_A(s.type)));
+  CUDA_TRY(upload(ctx, sc, &dB, a.b_consts, cnt * s.m * elem_size_B(s.type)));
+  CUDA_TRY(upload(ctx, sc, &dG, a.gamma, cnt * s.gm * s.n));
+  CUDA_TRY(upload(ctx, sc, &dT, a.target, cnt * elem_size_T(s.type)));
+  CUDA_TRY(upload(ctx, sc, &dc, a.xcoms, cnt * s.m * 2));
+  CUDA_TRY(upload(ctx, sc, &dd, a.ycoms, cnt * s.n * 2));
+  CUDA_TRY(upload(ctx, sc, &dpi, a.pi, cnt * s.cx * 2));
+  CUDA_TRY(upload(ctx, sc, &dth, a.theta, cnt * s.cy * 2));
+  *d = args_of(dA, dB, (const gs_fr*)dG, dT, (const gs_com1*)dc, (const gs_com2*)dd, (const gs_com2*)dpi, (const gs_com1*)dth);
+  return GS_OK;
+}
+
+// every input array is set (Gamma may be left out: the rank of gs_verify_sharded that holds no row of it)
+static bool inputs_set(const verify_args& v, bool need_gamma = true) {
+  return v.a_consts && v.b_consts && (v.gamma || !need_gamma) && v.target && v.xcoms && v.ycoms && v.pi && v.theta;
+}
+
+// all `count` rows of `bytes` bytes are equal, count > 1 (equations over ONE set of commitments: a multi-equation statement)
+static bool same_rows(const void* rows, size_t count, size_t bytes) {
+  for (size_t i = 1; i < count; i++)
+    if (memcmp(rows, (const char*)rows + i * bytes, bytes) != 0) return false;
+  return count > 1;
+}
+
+// ---- argument checks.  Their order decides the code of a call with several bad arguments, and it is not the same for
+// every entry point: each one calls these at the point where it has always made that check.
+static int check_crs(gs_ctx* ctx) {
+  if (!ctx->crs_loaded) FAIL(GS_EARG, "verify: no CRS loaded");
+  return GS_OK;
+}
+// the context, the equation type, the shard (rank, world) and, with `need_crs`, a loaded CRS
+static int check_call(gs_ctx* ctx, int type, int rank, int world, bool need_crs) {
+  if (!ctx) return GS_EARG;
+  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
+  if (world < 1 || rank < 0 || rank >= world) FAIL(GS_EARG, "verify: bad shard (rank, world)");
+  return need_crs ? check_crs(ctx) : GS_OK;
+}
+
+// a non-empty call: both variable lists non-empty and at most 2^20 long, then all inputs set.  The host front end of
+// gs_verify_batch / gs_verify_partial checks its inputs and the CRS ahead of the length limit (`inputs_first`).
+static int check_lists(gs_ctx* ctx, size_t m, size_t n, bool inputs, bool inputs_first = false) {
+  // the reference panics on empty variable lists (SURVEY.md §3.7): keep it an error
+  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
+  if (inputs_first) {
+    if (!inputs) return GS_EARG;
+    if (int rc = check_crs(ctx)) return rc;
+  }
+  if (m > 1 << 20 || n > 1 << 20) FAIL(GS_EDIM, "verify: too many variables");
+  return inputs ? GS_OK : GS_EARG;
 }
 
 extern "C" {
 
 // Shared body of gs_verify_batch_dev (rank 0 of 1, verdicts) and gs_verify_partial_dev (rank r of w: the
-// un-exponentiated Miller products of the slots that rank owns, out_partial[p][4]).
-static int verify_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                       const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
-                       const gs_com1* theta, int rank, int world, uint8_t* out_ok_dev, fp12* out_partial_dev, bool shared_x,
-                       bool shared_y = false) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
-  if (world < 1 || rank < 0 || rank >= world) FAIL(GS_EARG, "verify: bad shard (rank, world)");
-  if (!ctx->crs_loaded) FAIL(GS_EARG, "verify: no CRS loaded");
+// un-exponentiated Miller products of the slots that rank owns, out_partial[p][4]).  `one_pass`: the caller has cut the
+// batch into passes already (verify_host).
+static int verify_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args, int rank, int world,
+                       uint8_t* out_ok_dev, fp12* out_partial_dev, bool shared_x, bool shared_y = false, bool one_pass = false) {
+  if (int rc = check_call(ctx, type, rank, world, true)) return rc;
   if (count == 0) return GS_OK;
-  // the reference panics on empty variable lists (SURVEY.md §3.7): keep it an error
-  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
-  if (m > 1 << 20 || n > 1 << 20) FAIL(GS_EDIM, "verify: too many variables");
-  if (!a_consts || !b_consts || !gamma || !target || !xcoms || !ycoms || !pi || !theta) return GS_EARG;
-  if (!out_ok_dev && !out_partial_dev) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(args))) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
   s.rank = rank;
@@ -875,34 +963,16 @@ static int verify_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, 
   // A batch that needs several passes alternates them between the context's two streams: the passes are independent,
   // so whenever a kernel of one pass leaves SMs idle (the partial last wave of the MSM, a line walk that fills 3/4 of a
   // wave, kernel boundaries) blocks of the other pass take them.  Everything is joined back into gs_stream() at the end.
-  const size_t pass_n = verify_pass_size(ctx, count, shared_x);
-  const bool pipelined = count > pass_n && ctx->pass_streams == 2 && !ctx->profile;  // (per-kernel event times need one stream)
-  StreamGuard guard(ctx);
-  cudaStream_t pass_stream[2] = {ctx->stream, ctx->stream};
-  if (pipelined) {
-    if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-    pass_stream[1] = ctx->stream2;
-    cudaEvent_t fork;
-    CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-    cudaEventRecord(fork, pass_stream[0]);
-    cudaStreamWaitEvent(pass_stream[1], fork, 0);  // the inputs (uploaded / produced on the main stream) are complete
-    cudaEventDestroy(fork);
-  }
-  StreamJoin join{pass_stream[0], pass_stream[1], pipelined};  // the main stream is ordered after the second one on every exit path
+  const size_t pass_n = verify_pass_size(ctx, count, shared_x, one_pass);
+  PassStreams streams(ctx);
+  if (count > pass_n && ctx->pass_streams == 2 && !ctx->profile)  // (per-kernel event times need one stream)
+    CUDA_TRY(streams.split(true));  // the second stream waits for the inputs (uploaded / produced on the main stream)
   size_t pass = 0;
   for (size_t off = 0; off < count; off += pass_n, pass++) {
     size_t nprob = count - off < pass_n ? count - off : pass_n;
-    ctx->stream = pass_stream[pass & 1];
+    streams.use(pass);
     Scratch sc(ctx);
-    verify_args v;
-    v.a_consts = (const char*)a_consts + off * n * elem_size_A(type);
-    v.b_consts = (const char*)b_consts + off * m * elem_size_B(type);
-    v.gamma = (const fr*)gamma + off * m * n;
-    v.target = (const char*)target + off * elem_size_T(type);
-    v.xcoms = (const g1_aff*)xcoms + off * m * 2;
-    v.ycoms = (const g2_aff*)ycoms + off * n * 2;
-    v.pi = (const g2_aff*)pi + off * s.cx * 2;
-    v.theta = (const g1_aff*)theta + off * s.cy * 2;
+    const verify_args v = args_at(s, args, off);
     g1_aff* X;
     g2_aff* Y;
     uint8_t* ok4;
@@ -910,14 +980,12 @@ static int verify_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, 
     CUDA_TRY(sc.alloc(&Y, 2 * (size_t)s.K * nprob));
     CUDA_TRY(sc.alloc(&ok4, 4 * nprob));
     LAUNCH(k_verify_assemble, nprob * (size_t)s.K, s, v, ctx->crs, X, Y, nprob);
-    // what the shape alone says about the G2 side of every slot (k_verify_assemble): CRS points have stored lines,
-    // iota_2 images have no first coordinate
-    std::vector<uint8_t> kind_all = slot_kinds(s), kind;
+    std::vector<uint8_t> kind_all = slot_kinds(s);
     // equations over ONE set of y-commitments (a multi-equation statement): the (P_j, d_j) slots have the same G2 side in
     // every problem, so lines walked ahead are walked once (C4, 256 PPE equations: 50 k walked points -> 17 k)
     if (shared_y && nprob > 1)
       for (int k = 0; k < s.n; k++) kind_all[k] = gsi::GS_SLOT_WALK_SHARED;
-    for (int k = world > 1 ? rank : 0; k < s.K; k += world > 1 ? world : 1) kind.push_back(kind_all[k]);
+    const std::vector<uint8_t> kind = owned_kinds(kind_all, rank, world);
     // the G2 side is final now: a lone statement starts its line walks on the second stream, next to the MSM below
     g1_aff* Xo = nullptr;
     g2_aff* Yo = nullptr;
@@ -934,8 +1002,10 @@ static int verify_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, 
       if (rcw) return rcw;
     }
     {
-      int rcm = statement_msm(ctx, sc, s, v, nprob, shared_x, X);
+      const g1_jac* part;
+      int rcm = statement_msm_partials(ctx, sc, s, v, nprob, shared_x, &part);
       if (rcm) return rcm;
+      LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
     }
     const g1_aff* Xp = X;
     if (world > 1) {
@@ -960,7 +1030,8 @@ int gs_verify_batch_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n,
                         const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
                         const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, uint8_t* out_ok_dev) {
   if (!out_ok_dev) return GS_EARG;
-  return verify_impl(ctx, type, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, 0, 1, out_ok_dev, nullptr, false);
+  return verify_impl(ctx, type, count, m, n, args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), 0, 1, out_ok_dev,
+                     nullptr, false);
 }
 
 int gs_verify_partial_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
@@ -968,15 +1039,19 @@ int gs_verify_partial_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t 
                           const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, int rank, int world,
                           gs_gt* out_partial_dev) {
   if (!out_partial_dev) return GS_EARG;
-  return verify_impl(ctx, type, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, rank, world, nullptr,
-                     (fp12*)out_partial_dev, false);
+  return verify_impl(ctx, type, count, m, n, args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), rank, world,
+                     nullptr, (fp12*)out_partial_dev, false);
+}
+
+static int check_finish(gs_ctx* ctx, int type, int nparts) {
+  if (int rc = check_call(ctx, type, 0, 1, false)) return rc;
+  if (nparts < 1 || nparts > 4096) FAIL(GS_EARG, "verify_finish: bad number of partial products");
+  return GS_OK;
 }
 
 int gs_verify_finish_dev(gs_ctx* ctx, int type, size_t count, int nparts, const gs_gt* partials_dev, const void* target_dev,
                          uint8_t* out_ok_dev) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify_finish: bad equation type");
-  if (nparts < 1 || nparts > 4096) FAIL(GS_EARG, "verify_finish: bad number of partial products");
+  if (int rc = check_finish(ctx, type, nparts)) return rc;
   if (count == 0) return GS_OK;
   if (!partials_dev || !out_ok_dev || (type == GS_PPE && !target_dev)) return GS_EARG;
   CUDA_TRY(cudaSetDevice(ctx->device));
@@ -993,62 +1068,39 @@ int gs_verify_finish_dev(gs_ctx* ctx, int type, size_t count, int nparts, const 
 }
 
 // host-buffer front end shared by gs_verify_batch and gs_verify_partial: upload, run, download
-static int verify_host(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                       const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
-                       const gs_com1* theta, int rank, int world, uint8_t* out_ok, gs_gt* out_partial) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
+static int verify_host(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& h, int rank, int world,
+                       uint8_t* out_ok, gs_gt* out_partial) {
+  if (ctx && count && !out_ok && !out_partial) return GS_EARG;
+  if (int rc = check_call(ctx, type, rank, world, false)) return rc;
   if (count == 0) return GS_OK;
-  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
-  if (!a_consts || !b_consts || !gamma || !target || !xcoms || !ycoms || !pi || !theta || (!out_ok && !out_partial)) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(h), true)) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  verify_shape s = make_verify_shape(type, (int)m, (int)n);
+  const verify_shape s = make_verify_shape(type, (int)m, (int)n);
   // a batch of equations over ONE set of x-commitments (a multi-equation statement): detected on the host copy
-  bool shared_x = count > 1;
-  for (size_t i = 1; i < count && shared_x; i++)
-    shared_x = memcmp(xcoms, (const char*)xcoms + i * m * sizeof(gs_com1), m * sizeof(gs_com1)) == 0;
-  bool shared_y = count > 1;
-  for (size_t i = 1; i < count && shared_y; i++)
-    shared_y = memcmp(ycoms, (const char*)ycoms + i * n * sizeof(gs_com2), n * sizeof(gs_com2)) == 0;
+  const bool shared_x = same_rows(h.xcoms, count, m * sizeof(gs_com1));
+  const bool shared_y = same_rows(h.ycoms, count, n * sizeof(gs_com2));
   // Passes of verify_batch_max instances; with two pass streams the H2D copies of pass i + 1 run under the kernels of
   // pass i (pinned host buffers; pageable ones are staged by the driver and serialise on the host side).
-  const size_t B = verify_pass_size(ctx, count, shared_x);
+  const size_t B = verify_pass_size(ctx, count, shared_x, false);
   const bool pipelined = count > B && ctx->pass_streams == 2 && !ctx->profile && !shared_x;
   const size_t step = pipelined ? B : count;
   {
-    StreamGuard guard(ctx);
-    cudaStream_t pass_stream[2] = {ctx->stream, ctx->stream};
-    if (pipelined) {
-      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-      pass_stream[1] = ctx->stream2;
-    }
-    StreamJoin join{pass_stream[0], pass_stream[1], pipelined};
+    PassStreams streams(ctx);
+    if (pipelined) CUDA_TRY(streams.split(false));
     size_t pass = 0;
     for (size_t off = 0; off < count; off += step, pass++) {
       const size_t cnt = count - off < step ? count - off : step;
-      ctx->stream = pass_stream[pass & 1];
+      streams.use(pass);
       Scratch sc(ctx);
-      uint8_t *dA, *dB, *dT, *dok = nullptr;
+      verify_args d;
+      uint8_t* dok = nullptr;
       fp12* dpart = nullptr;
-      fr* dG;
-      g1_aff *dc, *dth;
-      g2_aff *dd, *dpi;
-      CUDA_TRY(upload(ctx, sc, &dA, (const char*)a_consts + off * n * elem_size_A(type), cnt * n * elem_size_A(type)));
-      CUDA_TRY(upload(ctx, sc, &dB, (const char*)b_consts + off * m * elem_size_B(type), cnt * m * elem_size_B(type)));
-      CUDA_TRY(upload(ctx, sc, &dG, gamma + off * m * n, cnt * m * n));
-      CUDA_TRY(upload(ctx, sc, &dT, (const char*)target + off * elem_size_T(type), cnt * elem_size_T(type)));
-      CUDA_TRY(upload(ctx, sc, &dc, xcoms + off * m, cnt * m * 2));
-      CUDA_TRY(upload(ctx, sc, &dd, ycoms + off * n, cnt * n * 2));
-      CUDA_TRY(upload(ctx, sc, &dpi, pi + off * s.cx, cnt * s.cx * 2));
-      CUDA_TRY(upload(ctx, sc, &dth, theta + off * s.cy, cnt * s.cy * 2));
+      if (int rc = upload_args(ctx, sc, s, h, off, cnt, &d)) return rc;
       if (out_ok)
         CUDA_TRY(sc.alloc(&dok, cnt));
       else
         CUDA_TRY(sc.alloc(&dpart, cnt * 4));
-      ctx->in_pass = pipelined;  // this loop IS the pass loop: verify_impl must not cut a pass in two again
-      int rc = verify_impl(ctx, type, cnt, m, n, dA, dB, (const gs_fr*)dG, dT, (const gs_com1*)dc, (const gs_com2*)dd,
-                           (const gs_com2*)dpi, (const gs_com1*)dth, rank, world, dok, dpart, shared_x, shared_y);
-      ctx->in_pass = false;
+      int rc = verify_impl(ctx, type, cnt, m, n, d, rank, world, dok, dpart, shared_x, shared_y, pipelined);
       if (rc) return rc;
       if (out_ok)
         CUDA_TRY(cudaMemcpyAsync(out_ok + off, dok, cnt, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1071,9 +1123,8 @@ static int verify_host(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, 
 // The transport is the caller's (NCCL through torch.distributed, raw NCCL, MPI ...): `allgather(user, send_dev, recv_dev,
 // bytes)` must gather `bytes` from every rank into recv_dev (rank-major) and return 0 when recv_dev is complete; both are
 // DEVICE pointers and the context's stream is idle while it runs.
-static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* dA, const void* dB, const fr* dGrows,
-                               const void* dT, const g1_aff* dc, const g2_aff* dd, const g2_aff* dpi, const g1_aff* dth, int rank,
-                               int world, bool shared_x, gs_allgather_fn allgather, void* user, uint8_t* dok) {
+static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& v, int rank, int world,
+                               bool shared_x, gs_allgather_fn allgather, void* user, uint8_t* dok) {
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
   s.rank = rank;
   s.world = world;
@@ -1086,15 +1137,6 @@ static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, si
   if (nprob > ctx->verify_batch_max) FAIL(GS_EDIM, "verify_sharded: too many statements for one pass");
   const int Ko = (s.K - rank + world - 1) / world;  // slots this rank owns
   Scratch sc(ctx);
-  verify_args v;
-  v.a_consts = dA;
-  v.b_consts = dB;
-  v.gamma = dGrows;
-  v.target = dT;
-  v.xcoms = dc;
-  v.ycoms = dd;
-  v.pi = dpi;
-  v.theta = dth;
   // ---- slots, owned G2 side, walk-ahead on the second stream (hidden behind the MSM and the first exchange)
   g1_aff *X, *Xo;
   g2_aff *Y, *Yo;
@@ -1103,12 +1145,7 @@ static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, si
   CUDA_TRY(sc.alloc(&Xo, 2 * (size_t)(Ko ? Ko : 1) * nprob));
   CUDA_TRY(sc.alloc(&Yo, 2 * (size_t)(Ko ? Ko : 1) * nprob));
   LAUNCH(k_verify_assemble, nprob * (size_t)s.K, s, v, ctx->crs, X, Y, nprob);
-  std::vector<uint8_t> kind_all(s.K, gsi::GS_SLOT_WALK), kind;
-  for (int k = s.sB; k < s.sPi; k++) kind_all[k] = s.groupB ? gsi::GS_SLOT_WALK_B1 : (uint8_t)(gsi::GS_SLOT_FIXED + 2);
-  for (int j = 0; j < s.cy; j++) kind_all[s.sTh + j] = (uint8_t)(gsi::GS_SLOT_FIXED + j);
-  if (type == 1 || type == 3) kind_all[s.sT] = (uint8_t)(gsi::GS_SLOT_FIXED + 2);
-  if (type == 2) kind_all[s.sT] = gsi::GS_SLOT_WALK_B1;
-  for (int k = rank; k < s.K; k += world) kind.push_back(kind_all[k]);
+  const std::vector<uint8_t> kind = owned_kinds(slot_kinds(s), rank, world);
   LAUNCH(k_gather_owned_slots, nprob * (size_t)Ko * 2, X, Y, Xo, Yo, nprob, s.K, Ko, rank, world, 0, 1);
   gsi::walk_ahead wa;  // after `sc`: destroyed first
   if (Ko > 0) {
@@ -1120,50 +1157,14 @@ static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, si
   sa.rank = 0;
   sa.world = 1;
   const size_t all_out = (size_t)sa.n_out;
-  const int nbo = sa.nb_own();
   g1_aff *myparts, *allparts;
   CUDA_TRY(sc.alloc(&myparts, nprob * all_out * 2));
   CUDA_TRY(sc.alloc(&allparts, (size_t)world * nprob * all_out * 2));
-  if (nbo > 0) {
-    const bool use_wtab = (nprob == 1 || shared_x) && all_out * nprob >= 320;
-    int chunk = GS_MSM_CHUNK;
-    const bool tiny = nprob * all_out * 2 * ((nbo + 7) / 8) < 16384;
-    const int floor_chunk = use_wtab ? 4 : (tiny ? 1 : 8);
-    while (chunk > floor_chunk && nprob * all_out * 2 * ((nbo + chunk - 1) / chunk) < (size_t)128 * 2368) chunk /= 2;
-    set_msm_chunk(sa, chunk);
-    g1_jac* part;
-    CUDA_TRY(sc.alloc(&part, (size_t)sa.nchunk * sa.n_out * 2 * nprob));
-    if (use_wtab) {
-      const int nb = nbo * 2;
-      const wt_geom g = wt_choose(all_out * nprob);
-      const size_t nrows = (size_t)nb * g.W;
-      g1_aff* wtab;
-      g1_jac* J;
-      CUDA_TRY(sc.alloc(&wtab, nrows * g.H));
-      CUDA_TRY(sc.alloc(&J, nrows * g.H));
-      LAUNCH(k_wtab_bases, (size_t)nb, sa, v, ctx->crs, J, nb, g);
-      LAUNCH(k_jac_to_affine_blocks<1>, nrows, J, wtab, nrows, (size_t)g.H);
-      LAUNCH(k_wtab_fill, nrows * (g.H / GS_WT_RUN), wtab, J, nrows, g.H);
-      LAUNCH(k_jac_to_affine_blocks<8>, nrows * g.H / 8, J, wtab, nrows * g.H, (size_t)1);
-      LAUNCH(k_vmsm_wsum, nprob * all_out * 2 * sa.nchunk, sa, v, wtab, part, nprob, g);
-    } else {
-      g1_aff* vtab;
-      fp* vtabx;
-      CUDA_TRY(sc.alloc(&vtab, (size_t)nbo * 2 * GS_VTAB * nprob));
-      CUDA_TRY(sc.alloc(&vtabx, (size_t)nbo * 2 * GS_VTAB * nprob));
-      LAUNCH(k_vmsm_tables, nprob * (size_t)nbo * 2, sa, v, ctx->crs, vtab, vtabx, nprob);
-      LAUNCH(k_vmsm_partial, nprob * all_out * 2 * sa.nchunk, sa, v, vtab, vtabx, part, nprob);
-    }
-    const g1_jac* partr = part;
-    if (sa.nchunk > 32) {
-      const int F = 16, ng = (sa.nchunk + F - 1) / F;
-      g1_jac* part2;
-      CUDA_TRY(sc.alloc(&part2, (size_t)ng * sa.n_out * 2 * nprob));
-      LAUNCH(k_vmsm_fold, (size_t)sa.n_out * 2 * nprob * ng, sa, part, part2, nprob, sa.nchunk, F, ng);
-      partr = part2;
-      sa.nchunk = ng;
-    }
-    LAUNCH(k_vmsm_parts_out, nprob * all_out * 2, sa, partr, myparts, nprob);
+  if (sa.nb_own() > 0) {
+    const g1_jac* part;
+    int rcm = statement_msm_partials(ctx, sc, sa, v, nprob, shared_x, &part);
+    if (rcm) return rcm;
+    LAUNCH(k_vmsm_parts_out, nprob * all_out * 2, sa, part, myparts, nprob);
   } else {
     CUDA_TRY(cudaMemsetAsync(myparts, 0, nprob * all_out * 2 * sizeof(g1_aff), ctx->stream));  // no base: identities
   }
@@ -1181,42 +1182,26 @@ static int verify_sharded_impl(gs_ctx* ctx, int type, size_t count, size_t m, si
   // ---- second exchange: 4 un-exponentiated GT values per statement and rank
   CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   if (allgather(user, mine, allp, nprob * 4 * sizeof(fp12)) != 0) FAIL(GS_EARG, "verify_sharded: all-gather of the Miller partial products failed");
-  return gs_verify_finish_dev(ctx, type, nprob, world, (const gs_gt*)allp, dT, dok);
+  return gs_verify_finish_dev(ctx, type, nprob, world, (const gs_gt*)allp, v.target, dok);
 }
 
 int gs_verify_sharded(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                       const gs_fr* gamma_rows, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                       const gs_com1* theta, int rank, int world, gs_allgather_fn allgather, void* user, uint8_t* out_ok) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
-  if (world < 1 || rank < 0 || rank >= world) FAIL(GS_EARG, "verify: bad shard (rank, world)");
-  if (!ctx->crs_loaded) FAIL(GS_EARG, "verify: no CRS loaded");
+  const verify_args h = args_of(a_consts, b_consts, gamma_rows, target, xcoms, ycoms, pi, theta);
+  if (int rc = check_call(ctx, type, rank, world, true)) return rc;
   if (count == 0) return GS_OK;
-  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
-  if (m > 1 << 20 || n > 1 << 20) FAIL(GS_EDIM, "verify: too many variables");
-  if (!a_consts || !b_consts || !target || !xcoms || !ycoms || !pi || !theta || !out_ok || !allgather) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(h, false) && out_ok && allgather)) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
   set_base_shard(s, rank, world);
   if (s.gm > 0 && !gamma_rows) return GS_EARG;
   Scratch sc(ctx);
-  uint8_t *dA, *dB, *dT, *dok;
-  fr* dG;
-  g1_aff *dc, *dth;
-  g2_aff *dd, *dpi;
-  CUDA_TRY(upload(ctx, sc, &dA, a_consts, count * n * elem_size_A(type)));
-  CUDA_TRY(upload(ctx, sc, &dB, b_consts, count * m * elem_size_B(type)));
-  CUDA_TRY(upload(ctx, sc, &dG, gamma_rows, count * (size_t)s.gm * n));   // ONLY this rank's rows of Gamma
-  CUDA_TRY(upload(ctx, sc, &dT, target, count * elem_size_T(type)));
-  CUDA_TRY(upload(ctx, sc, &dc, xcoms, count * m * 2));
-  CUDA_TRY(upload(ctx, sc, &dd, ycoms, count * n * 2));
-  CUDA_TRY(upload(ctx, sc, &dpi, pi, count * s.cx * 2));
-  CUDA_TRY(upload(ctx, sc, &dth, theta, count * s.cy * 2));
+  verify_args d;
+  uint8_t* dok;
+  if (int rc = upload_args(ctx, sc, s, h, 0, count, &d)) return rc;  // ONLY this rank's rows of Gamma
   CUDA_TRY(sc.alloc(&dok, count));
-  bool shared_x = count > 1;
-  for (size_t i = 1; i < count && shared_x; i++)
-    shared_x = memcmp(xcoms, (const char*)xcoms + i * m * sizeof(gs_com1), m * sizeof(gs_com1)) == 0;
-  int rc = verify_sharded_impl(ctx, type, count, m, n, dA, dB, dG, dT, dc, dd, dpi, dth, rank, world, shared_x, allgather, user, dok);
+  int rc = verify_sharded_impl(ctx, type, count, m, n, d, rank, world, same_rows(xcoms, count, m * sizeof(gs_com1)), allgather, user, dok);
   if (rc) return rc;
   CUDA_TRY(cudaMemcpyAsync(out_ok, dok, count, cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(cudaStreamSynchronize(ctx->stream));
@@ -1226,25 +1211,20 @@ int gs_verify_sharded(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, c
 int gs_verify_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
                     const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
                     const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, uint8_t* out_ok) {
-  if (ctx && count && !out_ok) return GS_EARG;
-  return verify_host(ctx, type, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, 0, 1, out_ok, nullptr);
+  return verify_host(ctx, type, count, m, n, args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), 0, 1, out_ok, nullptr);
 }
 
 int gs_verify_partial(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
                       const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
                       const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, int rank, int world,
                       gs_gt* out_partial) {
-  if (ctx && count && !out_partial) return GS_EARG;
-  if (ctx && (world < 1 || rank < 0 || rank >= world)) FAIL(GS_EARG, "verify: bad shard (rank, world)");
-  return verify_host(ctx, type, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, rank, world, nullptr,
-                     out_partial);
+  return verify_host(ctx, type, count, m, n, args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), rank, world,
+                     nullptr, out_partial);
 }
 
 int gs_verify_finish(gs_ctx* ctx, int type, size_t count, int nparts, const gs_gt* partials, const void* target,
                      uint8_t* out_ok) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify_finish: bad equation type");
-  if (nparts < 1 || nparts > 4096) FAIL(GS_EARG, "verify_finish: bad number of partial products");
+  if (int rc = check_finish(ctx, type, nparts)) return rc;
   if (count == 0) return GS_OK;
   if (!partials || !out_ok || (type == GS_PPE && !target)) return GS_EARG;
   CUDA_TRY(cudaSetDevice(ctx->device));
@@ -1279,9 +1259,8 @@ static int rand_slots_per_acc(size_t npairs) {
   return best;
 }
 
-static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                           const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
-                           const gs_com1* theta, const uint64_t* rho_host, bool shared_x, uint8_t* out_ok_dev) {
+static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args, const uint64_t* rho_host,
+                           bool shared_x, uint8_t* out_ok_dev) {
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
   const std::vector<uint8_t> kind_all = slot_kinds(s);
   // per-proof pairs (G2 side walked) and CRS slots (G1 sides summed over the proofs)
@@ -1388,15 +1367,7 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
       side_stream& s;      // main stream is ordered after the side work before `sc` releases buffers that work still uses
       ~join_on_exit() { s.join(); }
     } joined{side};
-    verify_args v;
-    v.a_consts = (const char*)a_consts + off * n * elem_size_A(type);
-    v.b_consts = (const char*)b_consts + off * m * elem_size_B(type);
-    v.gamma = (const fr*)gamma + off * m * n;
-    v.target = (const char*)target + off * elem_size_T(type);
-    v.xcoms = (const g1_aff*)xcoms + off * m * 2;
-    v.ycoms = (const g2_aff*)ycoms + off * n * 2;
-    v.pi = (const g2_aff*)pi + off * s.cx * 2;
-    v.theta = (const g1_aff*)theta + off * s.cy * 2;
+    const verify_args v = args_at(s, args, off);
     g1_aff *X, *X1, *Xfix;
     g2_aff *Y, *Y1;
     uint64_t* drho;
@@ -1487,14 +1458,18 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
       vf.fold_Kw = Kw;
       vf.fold_X1 = X1;
       vf.fold_Xfix = Xfix;
-      int rcm = statement_msm(ctx, sc, sf, vf, nprob, false, nullptr);
+      const g1_jac* part;
+      int rcm = statement_msm_partials(ctx, sc, sf, vf, nprob, false, &part);
       if (rcm) return rcm;
+      LAUNCH(k_vmsm_reduce, nprob * (size_t)sf.n_out_owned() * sf.na, sf, vf, part, (g1_aff*)nullptr, nprob);
       LAUNCH(k_rand_fold_g1, nprob * rest_slots.size(), X, nprob, s.K, drho, drest, (int)rest_slots.size(), dmap, Kw, X1, Xfix);
     } else {
       // one set of commitments under many equations: the statement MSM keeps its shared-base tables (both coordinates),
       // every slot is folded afterwards
-      int rcm = statement_msm(ctx, sc, s, v, nprob, shared_x, X);
+      const g1_jac* part;
+      int rcm = statement_msm_partials(ctx, sc, s, v, nprob, shared_x, &part);
       if (rcm) return rcm;
+      LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
       LAUNCH(k_rand_fold_g1, nprob * all_slots.size(), X, nprob, s.K, drho, dall, (int)all_slots.size(), dmap, Kw, X1, Xfix);
     }
     LAUNCH(k_rand_fold_g2, nprob * (size_t)Kw, Y, nprob, s.K, beta, dwalk_slot, Kw, Y1, (size_t)Kw, (size_t)1);
@@ -1529,38 +1504,21 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
 int gs_verify_batch_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                          const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                          const gs_com1* theta, const uint64_t* rho, uint8_t* out_all_ok) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
-  if (!ctx->crs_loaded) FAIL(GS_EARG, "verify: no CRS loaded");
+  const verify_args h = args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta);
+  if (int rc = check_call(ctx, type, 0, 1, true)) return rc;
   if (!out_all_ok) return GS_EARG;
   if (count == 0) {
     *out_all_ok = 1;
     return GS_OK;
   }
-  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
-  if (m > 1 << 20 || n > 1 << 20) FAIL(GS_EDIM, "verify: too many variables");
-  if (!a_consts || !b_consts || !gamma || !target || !xcoms || !ycoms || !pi || !theta || !rho) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(h) && rho)) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  verify_shape s = make_verify_shape(type, (int)m, (int)n);
-  bool shared_x = count > 1;
-  for (size_t i = 1; i < count && shared_x; i++)
-    shared_x = memcmp(xcoms, (const char*)xcoms + i * m * sizeof(gs_com1), m * sizeof(gs_com1)) == 0;
   Scratch sc(ctx);
-  uint8_t *dA, *dB, *dT, *dok;
-  fr* dG;
-  g1_aff *dc, *dth;
-  g2_aff *dd, *dpi;
-  CUDA_TRY(upload(ctx, sc, &dA, a_consts, count * n * elem_size_A(type)));
-  CUDA_TRY(upload(ctx, sc, &dB, b_consts, count * m * elem_size_B(type)));
-  CUDA_TRY(upload(ctx, sc, &dG, gamma, count * m * n));
-  CUDA_TRY(upload(ctx, sc, &dT, target, count * elem_size_T(type)));
-  CUDA_TRY(upload(ctx, sc, &dc, xcoms, count * m * 2));
-  CUDA_TRY(upload(ctx, sc, &dd, ycoms, count * n * 2));
-  CUDA_TRY(upload(ctx, sc, &dpi, pi, count * s.cx * 2));
-  CUDA_TRY(upload(ctx, sc, &dth, theta, count * s.cy * 2));
+  verify_args d;
+  uint8_t* dok;
+  if (int rc = upload_args(ctx, sc, make_verify_shape(type, (int)m, (int)n), h, 0, count, &d)) return rc;
   CUDA_TRY(sc.alloc(&dok, 4));
-  int rc = verify_rand_dev(ctx, type, count, m, n, dA, dB, (const gs_fr*)dG, dT, (const gs_com1*)dc, (const gs_com2*)dd,
-                           (const gs_com2*)dpi, (const gs_com1*)dth, rho, shared_x, dok);
+  int rc = verify_rand_dev(ctx, type, count, m, n, d, rho, same_rows(xcoms, count, m * sizeof(gs_com1)), dok);
   if (rc) return rc;
   CUDA_TRY(cudaMemcpyAsync(out_all_ok, dok, 1, cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(cudaStreamSynchronize(ctx->stream));
@@ -1570,15 +1528,12 @@ int gs_verify_batch_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n
 int gs_verify_batch_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                              const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                              const gs_com1* theta, const uint64_t* rho, uint8_t* out_all_ok_dev) {
-  if (!ctx) return GS_EARG;
-  if (type < 0 || type > 3) FAIL(GS_EARG, "verify: bad equation type");
-  if (!ctx->crs_loaded) FAIL(GS_EARG, "verify: no CRS loaded");
+  const verify_args v = args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta);
+  if (int rc = check_call(ctx, type, 0, 1, true)) return rc;
   if (count == 0 || !out_all_ok_dev) return GS_EARG;
-  if (m == 0 || n == 0) FAIL(GS_EDIM, "verify: empty variable list");
-  if (m > 1 << 20 || n > 1 << 20) FAIL(GS_EDIM, "verify: too many variables");
-  if (!a_consts || !b_consts || !gamma || !target || !xcoms || !ycoms || !pi || !theta || !rho) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(v) && rho)) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  return verify_rand_dev(ctx, type, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, rho, false, out_all_ok_dev);
+  return verify_rand_dev(ctx, type, count, m, n, v, rho, false, out_all_ok_dev);
 }
 
 }  // extern "C"

@@ -252,10 +252,12 @@ class Engine:
         return pi.raw[: count * cx * COM2], th.raw[: count * cy * COM1]
 
     @staticmethod
-    def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta):
-        """The C side reads count * (shape) bytes from every buffer: a short one would be read past its end."""
+    def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, gamma_rows=None):
+        """The C side reads count * (shape) bytes from every buffer: a short one would be read past its end.  Gamma holds
+        `gamma_rows` rows per problem (default m; gs_verify_sharded: this rank's rows only)."""
         cx, cy = _cx(ty), _cy(ty)
-        want = [count * n * _a_size(ty), count * m * _b_size(ty), count * m * n * FR, count * _t_size(ty),
+        gm = m if gamma_rows is None else gamma_rows
+        want = [count * n * _a_size(ty), count * m * _b_size(ty), count * gm * n * FR, count * _t_size(ty),
                 count * m * COM1, count * n * COM2, count * cx * COM2, count * cy * COM1]
         names = ["a_consts", "b_consts", "gamma", "target", "xcoms", "ycoms", "pi", "theta"]
         for nm, buf, w in zip(names, (a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), want):
@@ -333,14 +335,8 @@ class Engine:
         """gs_verify_sharded: the statement MSM split by base, the Miller pairs by slot, two all-gathers through
         `allgather(send_ptr, recv_ptr, nbytes) -> None` (device pointers; shard.make_allgather builds one over
         torch.distributed).  gamma_rows = this rank's rows of Gamma only (shard.gamma_rows_of)."""
-        cx, cy = _cx(ty), _cy(ty)
-        gm = len(range(rank, m, world))
-        want = [count * n * _a_size(ty), count * m * _b_size(ty), count * gm * n * FR, count * _t_size(ty), count * m * COM1,
-                count * n * COM2, count * cx * COM2, count * cy * COM1]
-        for nm, buf, w in zip(("a_consts", "b_consts", "gamma_rows", "target", "xcoms", "ycoms", "pi", "theta"),
-                              (a_consts, b_consts, gamma_rows, target, xcoms, ycoms, pi, theta), want):
-            if len(buf) != w:
-                raise GsError(1, f"verify_sharded: {nm} is {len(buf)} bytes, expected {w}")
+        self._check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma_rows, target, xcoms, ycoms, pi, theta,
+                                 gamma_rows=len(range(rank, m, world)))
         err = []
 
         def cb(_user, send, recv, nbytes):
