@@ -201,6 +201,11 @@ class _Equation:
         yc = (batch_commit_G2 if self.equ_type in (0, 2) else batch_commit_scalar_to_B2)(yvars, crs, rng)
         return CProof(xc, yc, [self.prove(xvars, yvars, xc, yc, crs, rng)])
 
+    def rerandomize(self, com_proof: CProof, crs: CRS, rng) -> CProof:
+        """A fresh-looking CProof of the same statement from `com_proof` alone, without the witnesses or the old randomness
+        (not in the reference; see rerandomize_batch).  RNG order: R' rows, S' rows, then T', row-major."""
+        return rerandomize_batch([self], [com_proof], crs, rng)[0]
+
     def verify(self, com_proof: CProof, crs: CRS) -> bool:              # verifier.rs:23-157
         assert len(com_proof.equ_proofs) == 1
         ep = com_proof.equ_proofs[0]
@@ -247,6 +252,57 @@ def prove_batch(equations, xvars, yvars, xcoms, ycoms, crs: CRS, rng) -> List[Eq
                                     b"".join(_flat(r) for r in rands), shared_vars=True)
     ps, ts = _split(pi, 384 * cx), _split(th, 192 * cy)
     return [EquProof(_split(p, 384), _split(t, 192), ty, r) for p, t, r in zip(ps, ts, rands)]
+
+
+def rerandomize_batch(equations, proofs, crs: CRS, rng, shared_commitments: bool = False) -> List[CProof]:
+    """Rerandomisation of committed proofs (Belenkiy et al., CRYPTO 2009; not in the reference): every (equation, CProof)
+    pair becomes a CProof of the same statement that is distributed exactly as a fresh commit_and_prove, computed from the
+    proof alone in one GPU pass (gs_rerandomize_batch).  One type and one shape per batch.
+
+    Fresh randomness is drawn per proof in commit_and_prove's order: R' (m x cx) rows, then S' (n x cy) rows, then T'
+    (cy x cx), row-major.  With shared_commitments every CProof must hold the same commitments (a multi-equation statement
+    over one set of variables): R' and S' are drawn once, then T' equation by equation, and the returned CProofs share the
+    new commitments.  The openings are not known to the rerandomiser, so the returned Commit*.rand and EquProof.rand are
+    empty matrices."""
+    assert len(equations) == len(proofs) and equations
+    ty = equations[0].equ_type
+    m, n = len(proofs[0].xcoms.coms), len(proofs[0].ycoms.coms)
+    for e, p in zip(equations, proofs):
+        if e.equ_type != ty or len(p.xcoms.coms) != m or len(p.ycoms.coms) != n:
+            raise ValueError("rerandomize_batch: every (equation, proof) must have the same type and shape")
+        if len(p.equ_proofs) != 1 or p.equ_proofs[0].equ_type != ty:
+            raise ValueError("rerandomize_batch: exactly one EquProof of the equation's type per CProof")
+        if len(e.a_consts) != n or len(e.b_consts) != m or len(e.gamma) != m or any(len(r) != n for r in e.gamma):
+            raise ValueError("rerandomize_batch: constants / Gamma do not match the number of variables")
+        if shared_commitments and (p.xcoms.coms != proofs[0].xcoms.coms or p.ycoms.coms != proofs[0].ycoms.coms):
+            raise ValueError("rerandomize_batch: shared_commitments needs the same commitments in every CProof")
+    cx, cy = equations[0]._cx(), equations[0]._cy()
+    draw = lambda rows, cols: [[rng.fr() for _ in range(cols)] for _ in range(rows)]
+    if shared_commitments:
+        R, S = draw(m, cx), draw(n, cy)
+        Rs, Ss, Ts = [R], [S], [draw(cy, cx) for _ in equations]
+    else:
+        Rs, Ss, Ts = [], [], []
+        for _ in equations:
+            Rs.append(draw(m, cx))
+            Ss.append(draw(n, cy))
+            Ts.append(draw(cy, cx))
+    coms = proofs[:1] if shared_commitments else proofs
+    cat = lambda f, items: b"".join(f(x) for x in items)
+    xc, yc, pi, th = crs._use().rerandomize_batch(
+        ty, len(equations), m, n, cat(lambda e: b"".join(e.a_consts), equations), cat(lambda e: b"".join(e.b_consts), equations),
+        cat(lambda e: _flat(e.gamma), equations), cat(lambda p: b"".join(p.xcoms.coms), coms),
+        cat(lambda p: b"".join(p.ycoms.coms), coms), cat(lambda p: b"".join(p.equ_proofs[0].pi), proofs),
+        cat(lambda p: b"".join(p.equ_proofs[0].theta), proofs), cat(_flat, Rs), cat(_flat, Ss), cat(_flat, Ts),
+        shared_coms=shared_commitments)
+    xcs, ycs = _split(xc, 192 * m), _split(yc, 384 * n)
+    pis, ths = _split(pi, 384 * cx), _split(th, 192 * cy)
+    out = []
+    for k in range(len(equations)):
+        j = 0 if shared_commitments else k
+        out.append(CProof(Commit1(_split(xcs[j], 192), []), Commit2(_split(ycs[j], 384), []),
+                          [EquProof(_split(pis[k], 384), _split(ths[k], 192), ty, [])]))
+    return out
 
 
 def verify_batch(equations, proofs, crs: CRS, randomized: bool = False, rho: bytes = None) -> List[bool]:

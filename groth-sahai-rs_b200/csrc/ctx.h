@@ -255,6 +255,14 @@ template <class F>
 int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_typed, const fr* sv, const void* dconst,
                   size_t nconst, const void* dvars, size_t nvars, bool vars_shared, int ncoef, const fr* coef, size_t coef_rs,
                   const fr* e, Aff<F>* dout);
+// rerandomisation of committed proofs (prover.cu gs_rerandomize_batch): c' = c + R' key for n commitments, and one
+// rerandomised proof element vector per proof (sv / rg: the scalar rows, see prover_impl.cuh)
+template <class F>
+int rerand_commit(gs_ctx* ctx, size_t n, int ns, const fr* dR, const Aff<F>* dcom, Aff<F>* dout);
+template <class F>
+int rerand_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_typed, const fr* sv, const fr* rg,
+                   const void* dconst, size_t nconst, const Aff<F>* dcom, size_t ncom, bool coms_shared, int ncoef,
+                   const fr* coef, const fr* e, const Aff<F>* dold, Aff<F>* dout);
 template <class F>
 int com_matmul_impl(gs_ctx* ctx, size_t r, size_t k, size_t c, const gs_fr* lhs, const void* mat, void* out);
 

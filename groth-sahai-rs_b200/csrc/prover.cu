@@ -388,6 +388,153 @@ int gs_prove_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, cons
                     out_pi, out_theta);
 }
 
+// `count` rerandomisations of committed proofs, laid out as prove_impl's arrays (shared_coms: one set of commitments and
+// of R', S' for every equation).  With fresh R', S', T':
+//   c' = c + R' u_x                     d' = d + S' v_y
+//   pi'    = pi    + R'^T iota_y(B) + (R'^T Gamma) d + (R'^T Gamma S' - T'^T) v_y
+//   theta' = theta + S'^T iota_x(A) + (S'^T Gamma^T) c + T' u_x
+// -- exactly commit_and_prove of the same witnesses under R + R', S + S', T + T' + S'^T Gamma^T R.  The Fr algebra is
+// prove_impl's; the variable-base sums run over the commitments (both coordinates) instead of iota(variables).
+static int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                            const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                            const gs_com1* theta, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
+                            gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta) {
+  if (!ctx) return GS_EARG;
+  if (type < 0 || type > 3) FAIL(GS_EARG, "rerandomize: bad equation type");
+  if (!ctx->crs_loaded) FAIL(GS_EARG, "rerandomize: no CRS loaded");
+  if (count == 0) return GS_OK;
+  if (m == 0 || n == 0) FAIL(GS_EDIM, "rerandomize: empty variable list");
+  if (m > 1 << 22 || n > 1 << 22) FAIL(GS_EDIM, "rerandomize: too many variables");
+  if (!a_consts || !b_consts || !gamma || !xcoms || !ycoms || !pi || !theta || !x_rand || !y_rand || !pf_rand || !out_xcoms ||
+      !out_ycoms || !out_pi || !out_theta)
+    return GS_EARG;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  verify_shape s = make_verify_shape(type, (int)m, (int)n);
+  const int cx = s.cx, cy = s.cy;
+  const size_t szA = elem_size_A(type), szB = elem_size_B(type);
+  const size_t MAXB = 32768;  // gridDim.y limit is 65,535
+  for (size_t off = 0; off < count; off += MAXB) {
+    const size_t nb = count - off < MAXB ? count - off : MAXB;
+    const size_t voff = shared ? 0 : off, nv = shared ? 1 : nb;
+    Scratch sc(ctx);
+    uint8_t *dA, *dB;
+    fr *dG, *dR, *dS, *dT;
+    g1_aff *dXc, *dTh;
+    g2_aff *dYc, *dPi;
+    CUDA_TRY(upload(ctx, sc, &dA, (const char*)a_consts + off * n * szA, nb * n * szA));
+    CUDA_TRY(upload(ctx, sc, &dB, (const char*)b_consts + off * m * szB, nb * m * szB));
+    CUDA_TRY(upload(ctx, sc, &dG, gamma + off * m * n, nb * m * n));
+    CUDA_TRY(upload(ctx, sc, &dXc, xcoms + voff * m, nv * m * 2));
+    CUDA_TRY(upload(ctx, sc, &dYc, ycoms + voff * n, nv * n * 2));
+    CUDA_TRY(upload(ctx, sc, &dPi, pi + off * cx, nb * cx * 2));
+    CUDA_TRY(upload(ctx, sc, &dTh, theta + off * cy, nb * cy * 2));
+    CUDA_TRY(upload(ctx, sc, &dR, x_rand + voff * m * cx, nv * m * cx));
+    CUDA_TRY(upload(ctx, sc, &dS, y_rand + voff * n * cy, nv * n * cy));
+    CUDA_TRY(upload(ctx, sc, &dT, pf_rand + off * cx * cy, nb * cx * cy));
+    // the new commitments (once for a shared set), on the main stream before the proof elements fork: a first call under
+    // a key may (re)build the fixed-base tables that the elements read
+    const bool do_coms = !shared || off == 0;
+    g1_aff* dXo = nullptr;
+    g2_aff* dYo = nullptr;
+    if (do_coms) {
+      CUDA_TRY(sc.alloc(&dXo, nv * m * 2));
+      CUDA_TRY(sc.alloc(&dYo, nv * n * 2));
+      int rc = rerand_commit<FpOps>(ctx, nv * m, cx, dR, dXc, dXo);
+      if (rc) return rc;
+      rc = rerand_commit<Fp2Ops>(ctx, nv * n, cy, dS, dYc, dYo);
+      if (rc) return rc;
+    }
+    const size_t r_bs = shared ? 0 : m * cx, s_bs = shared ? 0 : n * cy;  // instance strides of R', S'
+    fr *RG, *SG, *coef_pi, *sv_pi, *sv_th;
+    CUDA_TRY(sc.alloc(&RG, nb * cx * n));
+    CUDA_TRY(sc.alloc(&SG, nb * cy * m));
+    CUDA_TRY(sc.alloc(&coef_pi, nb * cx * cy));
+    CUDA_TRY(sc.alloc(&sv_pi, nb * cx * (m + n)));
+    CUDA_TRY(sc.alloc(&sv_th, nb * cy * (m + n)));
+    // RG = R'^T Gamma (cx x n), SG = S'^T Gamma^T (cy x m), coef_pi = R'^T Gamma S' - T'^T: as in prove_impl
+    const int l_rg = fr_lanes(m, (size_t)cx * n * nb), l_sg = fr_lanes(n, (size_t)cy * m * nb), l_cp = fr_lanes(n, (size_t)cx * cy * nb);
+    LAUNCH_B(k_fr_matmul, (size_t)cx * n * l_rg, nb, RG, dR, (size_t)1, (size_t)cx, dG, n, (size_t)1, (size_t)cx, m, n, r_bs, m * n, l_rg);
+    LAUNCH_B(k_fr_matmul, (size_t)cy * m * l_sg, nb, SG, dS, (size_t)1, (size_t)cy, dG, (size_t)1, n, (size_t)cy, n, m, s_bs, m * n, l_sg);
+    LAUNCH_B(k_coef_pi, (size_t)cx * cy * l_cp, nb, coef_pi, RG, dS, dT, cx, cy, n, s_bs, l_cp);
+    LAUNCH_B(k_concat_scalars, (size_t)cx * (m + n), nb, sv_pi, dR, RG, cx, m, n, r_bs);
+    LAUNCH_B(k_concat_scalars, (size_t)cy * (m + n), nb, sv_th, dS, SG, cy, n, m, s_bs);
+    // scalar-typed constants collapse onto W: e_i = sum_k R'[k][i] b_k (pi'), sum_j S'[j][i] a_j (theta')
+    fr *e_pi = nullptr, *e_th = nullptr;
+    if (!s.groupB) {
+      fr* rt;
+      CUDA_TRY(sc.alloc(&rt, nb * cx * m));
+      CUDA_TRY(sc.alloc(&e_pi, nb * cx));
+      const int l_d = fr_lanes(m, (size_t)cx * nb);
+      LAUNCH_B(k_concat_scalars, (size_t)cx * m, nb, rt, dR, RG, cx, m, (size_t)0, r_bs);
+      LAUNCH_B(k_fr_dot, (size_t)cx * l_d, nb, e_pi, rt, (const fr*)dB, m, (const fr*)nullptr, (size_t)0, cx, (size_t)0, l_d);
+    }
+    if (!s.groupA) {
+      fr* st;
+      CUDA_TRY(sc.alloc(&st, nb * cy * n));
+      CUDA_TRY(sc.alloc(&e_th, nb * cy));
+      const int l_d = fr_lanes(n, (size_t)cy * nb);
+      LAUNCH_B(k_concat_scalars, (size_t)cy * n, nb, st, dS, SG, cy, n, (size_t)0, s_bs);
+      LAUNCH_B(k_fr_dot, (size_t)cy * l_d, nb, e_th, st, (const fr*)dA, n, (const fr*)nullptr, (size_t)0, cy, (size_t)0, l_d);
+    }
+    g2_aff* dpo;
+    g1_aff* dto;
+    CUDA_TRY(sc.alloc(&dpo, nb * 2 * cx));
+    CUDA_TRY(sc.alloc(&dto, nb * 2 * cy));
+    // theta' on the second stream next to pi' in the latency regime, as in prove_impl
+    const bool two_streams = nb * (m + n) * 2 < 32768;
+    cudaStream_t main_stream = ctx->stream;
+    cudaEvent_t fork = nullptr, join = nullptr;
+    if (two_streams) {
+      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
+      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
+      if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
+        cudaEventDestroy(fork);
+        FAIL(GS_ECUDA, "rerandomize: event creation failed");
+      }
+      cudaEventRecord(fork, main_stream);
+      cudaStreamWaitEvent(ctx->stream2, fork, 0);
+      ctx->stream = ctx->stream2;
+    }
+    int rc_th = rerand_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, SG, dA, n, dXc, m, shared, cx, dT, e_th, dTh, dto);
+    if (two_streams) {
+      cudaEventRecord(join, ctx->stream2);
+      ctx->stream = main_stream;
+    }
+    int rc_pi = rerand_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, RG, dB, m, dYc, n, shared, cy, coef_pi, e_pi, dPi, dpo);
+    if (two_streams) {
+      cudaStreamWaitEvent(main_stream, join, 0);  // also orders the scratch frees (main stream) after theta's kernels
+      cudaEventDestroy(fork);
+      cudaEventDestroy(join);
+    }
+    if (rc_th) return rc_th;
+    if (rc_pi) return rc_pi;
+    if (do_coms) {
+      CUDA_TRY(cudaMemcpyAsync(out_xcoms + voff * m, dXo, nv * m * 2 * sizeof(g1_aff), cudaMemcpyDeviceToHost, ctx->stream));
+      CUDA_TRY(cudaMemcpyAsync(out_ycoms + voff * n, dYo, nv * n * 2 * sizeof(g2_aff), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CUDA_TRY(cudaMemcpyAsync(out_pi + off * cx, dpo, nb * 2 * cx * sizeof(g2_aff), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_theta + off * cy, dto, nb * 2 * cy * sizeof(g1_aff), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  }
+  return GS_OK;
+}
+
+int gs_rerandomize(gs_ctx* ctx, int type, size_t m, size_t n, const void* a_consts, const void* b_consts, const gs_fr* gamma,
+                   const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const gs_fr* x_rand,
+                   const gs_fr* y_rand, const gs_fr* pf_rand, gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi,
+                   gs_com1* out_theta) {
+  return rerandomize_impl(ctx, type, 1, m, n, a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand, false,
+                          out_xcoms, out_ycoms, out_pi, out_theta);
+}
+
+int gs_rerandomize_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                         const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                         const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, int shared_coms, gs_com1* out_xcoms,
+                         gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta) {
+  return rerandomize_impl(ctx, type, count, m, n, a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand,
+                          shared_coms != 0, out_xcoms, out_ycoms, out_pi, out_theta);
+}
+
 int gs_com1_matmul(gs_ctx* ctx, size_t r, size_t k, size_t c, const gs_fr* lhs, const gs_com1* mat, gs_com1* out) {
   return com_matmul_impl<FpOps>(ctx, r, k, c, lhs, mat, out);
 }

@@ -350,6 +350,132 @@ __global__ void k_proof_finish2(Aff<F>* __restrict__ out, int rows, const Jac<F>
   out[id] = r;
 }
 
+// ------------------------------------------------------------------ rerandomisation of a committed proof
+// c' = c + R' u_x (and d' = d + S' v_y): out[i].p[a] = com[i].p[a] + sum_{k < ns} s[i][k] key_k.a from the fixed-base tables.
+// Unlike k_fixed_commit the addend is a whole commitment (both coordinates); k_fixed_commit keeps its C2 register budget.
+template <class F>
+__global__ void __launch_bounds__(GS_TAB_NT) k_rerand_commit(const Aff<F>* __restrict__ tab, int c, int W, size_t H, const fr* __restrict__ s,
+                                                             int ns, const Aff<F>* __restrict__ com, Aff<F>* __restrict__ out, size_t n) {
+  __shared__ fp sm[2 * GS_TAB_NT];
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  bool active = id < 2 * n;
+  size_t i = active ? id >> 1 : 0;
+  int a = (int)(id & 1);
+  Jac<F> acc;
+  acc.set_inf();
+  if (active) {
+    acc.from_affine(com[i * 2 + a]);
+    for (int k = 0; k < ns; k++) {
+      uint32_t kk[8];
+      fr_from_mont(kk, s[i * ns + k]);
+      fixed_base_accumulate<F>(acc, tab + ((size_t)(k * 2 + a) * W) * H, kk, c, W, H);
+    }
+  }
+  Aff<F> r;
+  block_to_affine<GS_TAB_NT>(r, acc, sm);
+  if (active) out[i * 2 + a] = r;
+}
+
+// Variable-base products of a rerandomised proof element (pi': G2 over the constants B and the commitments d; theta': G1
+// over A and c).  Output row i has two coordinate rows:
+//   a = 1:  sum_{k < n0} sv[i][k] B_k + sum_j sv[i][c0 + j] com_j.1        (n0 = 0 on a scalar-typed side)
+//   a = 0:                              sum_j sv[i][c0 + j] com_j.0
+// terms[((y*rows + i)*2 + a)*ns*PARTS + slot*PARTS + part], ns = n0 + ncom slots (slot k < n0: B_k; n0 + j: com_j).
+// Only the n0 + 2 ncom real products of a row are computed, product q of [q0, q1):  q < n0: B_q (a = 1);
+// q < n0 + ncom: com_{q-n0}.1; else com_{q-n0-ncom}.0.  The n0 constant slots of an a = 0 row are zeroed by the caller.
+template <class F>
+__global__ void __launch_bounds__(128) k_rerand_terms(Jac<F>* __restrict__ terms, const fr* __restrict__ sv, size_t svs, size_t c0,
+                                                      const Aff<F>* __restrict__ b0, size_t n0, const Aff<F>* __restrict__ com, size_t ncom,
+                                                      size_t com_bs, int rows, size_t q0, size_t q1, int PARTS) {
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t nq = q1 - q0;
+  if (id >= nq * rows * PARTS) return;
+  const int j = (int)(id % PARTS);
+  const size_t qr = id / PARTS;
+  const size_t q = q0 + qr % nq, i = qr / nq;
+  const size_t ntp = (n0 + ncom) * PARTS;
+  terms += (size_t)blockIdx.y * rows * 2 * ntp;
+  sv += (size_t)blockIdx.y * rows * svs;
+  b0 += (size_t)blockIdx.y * n0;
+  com += (size_t)blockIdx.y * com_bs;
+  Aff<F> B;
+  size_t col, slot;
+  int a = 1;
+  if (q < n0) {
+    B = b0[q];
+    col = q;
+    slot = q;
+  } else {
+    const size_t t = q - n0;
+    const size_t jc = t < ncom ? t : t - ncom;
+    a = t < ncom ? 1 : 0;
+    B = com[jc * 2 + a];
+    col = c0 + jc;
+    slot = n0 + jc;
+  }
+  uint32_t k[8];
+  fr_from_mont(k, sv[i * svs + col]);
+  Jac<F> r;
+  if (PARTS == 1)
+    scalar_mul<F>(r, B, k);
+  else
+    EndoSplit<F>::part(r, B, k, j);
+  terms[(i * 2 + a) * ntp + slot * PARTS + j] = r;
+}
+
+// Shared commitments (one set for every equation): thread -> (i, a, j) of equation blockIdx.y,
+// terms[((y*rows + i)*2 + a)*ns + n0 + j] = sv[i][c0 + j] * com_j.a from the shared-base tables (table row 2j + a).
+template <class F>
+__global__ void __launch_bounds__(128) k_rerand_com_terms_tab(Jac<F>* __restrict__ terms, const fr* __restrict__ sv, size_t svs, size_t c0,
+                                                              const Aff<F>* __restrict__ tab, size_t n0, size_t ncom, int rows) {
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= (size_t)rows * 2 * ncom) return;
+  const size_t jc = id % ncom, ia = id / ncom;
+  const size_t i = ia >> 1;
+  const int a = (int)(ia & 1);
+  const size_t ns = n0 + ncom;
+  constexpr int W = ptab_windows<F>(), PARTS = PipSplit<F>::PARTS;
+  uint32_t k[8], sub[PARTS][4];
+  fr_from_mont(k, sv[(size_t)blockIdx.y * rows * svs + i * svs + c0 + jc]);
+  PipSplit<F>::split(sub, k);
+  Jac<F> acc;
+  acc.set_inf();
+  for (int p = PARTS - 1; p >= 0; p--) {
+    if (p != PARTS - 1 && !acc.is_inf()) endo_neg_jac(acc);
+    uint32_t kk[8] = {sub[p][0], sub[p][1], sub[p][2], sub[p][3], 0, 0, 0, 0};
+    fixed_base_accumulate<F>(acc, tab + ((jc * 2 + a) * W) * GS_PT_H, kk, GS_PT_C, W, (size_t)GS_PT_H);
+  }
+  terms[(((size_t)blockIdx.y * rows + i) * 2 + a) * ns + n0 + jc] = acc;
+}
+
+// where the variable-base sum of coordinate a of output row i of proof y is: p[a][y * inst[a] + i * row[a]] (p[a] null: none)
+template <class F>
+struct rerand_sums {
+  const Jac<F>* p[2];
+  size_t inst[2], row[2];
+};
+// out[i].p[a] = old[i].p[a] + the key / W terms (reduced kt, as for k_proof_finish2) + the variable-base sum of coordinate a
+template <class F>
+__global__ void k_rerand_finish(Aff<F>* __restrict__ out, int rows, const Jac<F>* __restrict__ kt, int KT, const Aff<F>* __restrict__ old,
+                                rerand_sums<F> vs) {
+  int id = blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= rows * 2) return;
+  int i = id >> 1, a = id & 1;
+  const size_t y = blockIdx.y;
+  out += y * rows * 2;
+  old += y * rows * 2;
+  kt += y * rows * 2 * KT;
+  Jac<F> acc = kt[(size_t)id * KT];
+  Jac<F>::add_mixed(acc, acc, old[id]);
+  if (vs.p[a] != nullptr) {
+    Jac<F> v = vs.p[a][y * vs.inst[a] + (size_t)i * vs.row[a]];
+    Jac<F>::add(acc, acc, v);
+  }
+  Aff<F> r;
+  Jac<F>::to_affine(r, acc);
+  out[id] = r;
+}
+
 // ------------------------------------------------------------------ Mat::left_mul on Com matrices
 // terms[(i*c + j)*2 + a][t] = lhs[i][t] * mat[t][j].a      (data_structures.rs:696-742)
 template <class F>
@@ -428,6 +554,16 @@ int fixed_table_rebuild(gs_ctx* ctx, int c) {
   return GS_OK;
 }
 
+// the fixed-base tables for a batch of n commitments: big batches amortise bigger windows, 16 windows of 16 bits instead
+// of 32 of 8 (never downgraded: once the c = 16 tables exist, small batches use them too instead of rebuilding c = 8)
+template <class F>
+int fixed_table_for(gs_ctx* ctx, size_t n) {
+  gs_fixed_table<F>& T = table_of<F>(ctx);
+  int want_c = n >= 8192 ? 16 : 8;
+  if (!T.t || (want_c == 16 && T.c != 16)) return fixed_table_rebuild<F>(ctx, want_c);
+  return GS_OK;
+}
+
 // out[i] = s0[i] Base0 + s1[i] Base1 (+ iota(addend[i]))    -- all four batch_commit_* variants
 template <class F>
 int batch_commit_impl(gs_ctx* ctx, size_t n, int base0, int base1, const gs_fr* s0, size_t s0_stride, const gs_fr* s1,
@@ -436,14 +572,9 @@ int batch_commit_impl(gs_ctx* ctx, size_t n, int base0, int base1, const gs_fr* 
   if (!ctx->crs_loaded) FAIL(GS_EARG, "commit: no CRS loaded");
   if (n == 0) return GS_OK;  // reference: empty input -> empty Commit (left_mul returns vec![])
   CUDA_TRY(cudaSetDevice(ctx->device));
-  // big batches amortise bigger windows: 16 windows of 16 bits instead of 32 of 8
+  int rct = fixed_table_for<F>(ctx, n);
+  if (rct) return rct;
   gs_fixed_table<F>& T = table_of<F>(ctx);
-  // (never downgraded: once the c = 16 tables exist, small batches use them too instead of rebuilding c = 8)
-  int want_c = n >= 8192 ? 16 : 8;
-  if (!T.t || (want_c == 16 && T.c != 16)) {
-    int rc = fixed_table_rebuild<F>(ctx, want_c);
-    if (rc) return rc;
-  }
   // Big batches (C2: 2^20 variables = 160 MB in, 192 MB out for G1) are cut into chunks that alternate between two
   // streams: while the host stages chunk i+1 in and chunk i-1 out (pageable copies block the host, not the GPU),
   // the kernel of chunk i runs.  Only the interleaved-randomness layout (batch_commit_G1/G2) is chunked.
@@ -530,18 +661,45 @@ int reduce_rows(gs_ctx* ctx, Jac<F>* terms, size_t stride, size_t cnt, int rows,
   return GS_OK;
 }
 
-// final assembly of the proof elements of `count` proofs (k_proof_key_terms -> tree -> k_proof_finish2)
+// the CRS-key terms of the proof elements of `count` proofs (k_proof_key_terms -> tree): the sum of (i, a) lands in
+// (*kt)[(i*2 + a) * *KT] of each proof
+template <class F>
+int proof_key_sums(gs_ctx* ctx, Scratch& sc, size_t count, int rows, int ncoef, const fr* coef, const gs_fixed_table<F>& T,
+                   const fr* e, Jac<F>** kt, int* KT) {
+  const int nscal = ncoef + (e != nullptr ? 1 : 0);
+  *KT = nscal * PF_NCH;
+  CUDA_TRY(sc.alloc(kt, count * (size_t)rows * 2 * *KT));
+  LAUNCH_B((k_proof_key_terms<F>), (size_t)rows * 2 * *KT, count, *kt, rows, ncoef, coef, T.t, T.c, T.W, T.H, e, nscal);
+  return reduce_rows<F>(ctx, *kt, (size_t)*KT, (size_t)*KT, rows * 2, count);
+}
+
+// final assembly of the proof elements of `count` proofs (key sums -> k_proof_finish2)
 template <class F>
 int proof_finish(gs_ctx* ctx, Scratch& sc, size_t count, int rows, int ncoef, const fr* coef, const gs_fixed_table<F>& T,
                  const Jac<F>* varsum, size_t var_stride, const fr* e, Aff<F>* dout) {
-  const int nscal = ncoef + (e != nullptr ? 1 : 0);
-  const int KT = nscal * PF_NCH;
   Jac<F>* kt;
-  CUDA_TRY(sc.alloc(&kt, count * (size_t)rows * 2 * KT));
-  LAUNCH_B((k_proof_key_terms<F>), (size_t)rows * 2 * KT, count, kt, rows, ncoef, coef, T.t, T.c, T.W, T.H, e, nscal);
-  int rc = reduce_rows<F>(ctx, kt, (size_t)KT, (size_t)KT, rows * 2, count);
+  int KT;
+  int rc = proof_key_sums<F>(ctx, sc, count, rows, ncoef, coef, T, e, &kt, &KT);
   if (rc) return rc;
   LAUNCH_B((k_proof_finish2<F>), (size_t)rows * 2, count, dout, rows, kt, KT, varsum, var_stride);
+  return GS_OK;
+}
+
+// shared-base window tables of nb points (see k_ptab_bases): ptab = nb * ptab_windows rows of GS_PT_H affine multiples,
+// J = Jacobian scratch of the same size
+template <class F>
+cudaError_t shared_base_alloc(Scratch& sc, size_t nb, Aff<F>** ptab, Jac<F>** J) {
+  const size_t nrows = nb * ptab_windows<F>();
+  cudaError_t e = sc.alloc(ptab, nrows * GS_PT_H);
+  return e == cudaSuccess ? sc.alloc(J, nrows * GS_PT_H) : e;
+}
+template <class F>
+int shared_base_tables(gs_ctx* ctx, const Aff<F>* bases, size_t nb, Aff<F>* ptab, Jac<F>* J) {
+  const size_t nrows = nb * ptab_windows<F>();
+  LAUNCH((k_ptab_bases<F>), nb, bases, J, (int)nb);
+  LAUNCH((k_ptab_to_affine<F>), nrows, J, ptab, nrows, (size_t)GS_PT_H);
+  LAUNCH((k_ptab_fill<F>), nrows * (GS_PT_H / GS_PT_RUN), ptab, J, nrows);
+  LAUNCH((k_ptab_to_affine<F>), nrows * GS_PT_H, J, ptab, nrows * GS_PT_H, (size_t)1);
   return GS_OK;
 }
 
@@ -587,11 +745,9 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
     } else {
       // the tables are built on the second stream while the constant terms (latency-bound scalar multiplications)
       // run on the main one
-      const size_t nrows = nvars * ptab_windows<F>();
       Aff<F>* ptab;
       Jac<F>* J;
-      CUDA_TRY(sc.alloc(&ptab, nrows * GS_PT_H));
-      CUDA_TRY(sc.alloc(&J, nrows * GS_PT_H));
+      CUDA_TRY(shared_base_alloc<F>(sc, nvars, &ptab, &J));
       if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
       cudaEvent_t fork, join;
       CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
@@ -601,10 +757,8 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
       cudaStream_t main_stream = ctx->stream;
       ctx->stream = ctx->stream2;
       int rct = [&]() -> int {
-        LAUNCH((k_ptab_bases<F>), nvars, (const Aff<F>*)dvars, J, (int)nvars);
-        LAUNCH((k_ptab_to_affine<F>), nrows, J, ptab, nrows, (size_t)GS_PT_H);
-        LAUNCH((k_ptab_fill<F>), nrows * (GS_PT_H / GS_PT_RUN), ptab, J, nrows);
-        LAUNCH((k_ptab_to_affine<F>), nrows * GS_PT_H, J, ptab, nrows * GS_PT_H, (size_t)1);
+        int rcb = shared_base_tables<F>(ctx, (const Aff<F>*)dvars, nvars, ptab, J);
+        if (rcb) return rcb;
         LAUNCH_B((k_msm_var_terms_tab<F>), nvars * rows, count, terms, sv, ptab, nconst, nvars, rows);
         return GS_OK;
       }();
@@ -637,6 +791,118 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
     // scalar-typed side: the caller collapsed the terms into e_i = <sv_i, (consts | vars)> (k_fr_dot, prover.cu)
     return proof_finish<F>(ctx, sc, count, rows, ncoef, coef, T, (const Jac<F>*)nullptr, (size_t)0, e, dout);
   }
+}
+
+// c' = c + R' key for n commitments of one group, R' n x ns (ns = 2: u1 u2 / v1 v2; 1: u1 / v1); device buffers
+template <class F>
+int rerand_commit(gs_ctx* ctx, size_t n, int ns, const fr* dR, const Aff<F>* dcom, Aff<F>* dout) {
+  int rc = fixed_table_for<F>(ctx, n);
+  if (rc) return rc;
+  const gs_fixed_table<F>& T = table_of<F>(ctx);
+  LAUNCH((k_rerand_commit<F>), 2 * n, T.t, T.c, T.W, T.H, dR, ns, dcom, dout, n);
+  return GS_OK;
+}
+
+// One rerandomised proof element vector per proof (pi': F = G2, theta': F = G1), batched over `count` proofs:
+//   out[i] = old[i] + (variable-base sums, see k_rerand_terms) + sum_l coef[i][l] key_l (+ e_i W)
+// sv = [count][rows][nconst + ncom]: the scalars of the constants, then those of the commitments; rg = the commitment
+// columns alone, [count][rows][ncom]; dcom = [count][ncom] Com, or one set for every proof with coms_shared.
+// The paths are proof_element's: bucket MSMs for one big statement, shared-base tables over the 2 ncom commitment
+// points when many equations share them, else one (split) scalar multiplication per product.
+template <class F>
+int rerand_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_typed, const fr* sv, const fr* rg,
+                   const void* dconst, size_t nconst, const Aff<F>* dcom, size_t ncom, bool coms_shared, int ncoef,
+                   const fr* coef, const fr* e, const Aff<F>* dold, Aff<F>* dout) {
+  if (!table_of<F>(ctx).t) {
+    int rct = fixed_table_rebuild<F>(ctx, 8);
+    if (rct) return rct;
+  }
+  const gs_fixed_table<F>& T = table_of<F>(ctx);
+  const Aff<F>* B = (const Aff<F>*)dconst;
+  const size_t n0 = group_typed ? nconst : 0, svs = nconst + ncom;
+  const size_t nprod = n0 + 2 * ncom, ns = n0 + ncom;  // products and term slots of a coordinate row
+  const bool var_tables = coms_shared && count * rows >= 64;
+  rerand_sums<F> vs;
+  if (count == 1 && !var_tables && ns >= ctx->pip_min) {
+    Aff<F>*c0, *c1;
+    CUDA_TRY(sc.alloc(&c0, ncom));
+    CUDA_TRY(sc.alloc(&c1, ncom));
+    const size_t A = sizeof(Aff<F>);
+    CUDA_TRY(cudaMemcpy2DAsync(c0, A, dcom, 2 * A, A, ncom, cudaMemcpyDeviceToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpy2DAsync(c1, A, dcom + 1, 2 * A, A, ncom, cudaMemcpyDeviceToDevice, ctx->stream));
+    Jac<F>*s0, *s1;
+    size_t st0, st1;
+    int rc = group_typed ? pippenger_rows<F>(ctx, sc, sv, rows, B, n0, c1, ncom, &s1, &st1, ctx->pip_c)
+                         : pippenger_rows<F>(ctx, sc, rg, rows, c1, ncom, (const Aff<F>*)nullptr, 0, &s1, &st1, ctx->pip_c);
+    if (rc) return rc;
+    rc = pippenger_rows<F>(ctx, sc, rg, rows, c0, ncom, (const Aff<F>*)nullptr, 0, &s0, &st0, ctx->pip_c);
+    if (rc) return rc;
+    vs = {{s0, s1}, {0, 0}, {st0, st1}};
+  } else {
+    const int PARTS = (!var_tables && count * nprod * rows < 32768) ? EndoSplit<F>::PARTS : 1;
+    const size_t ntp = ns * PARTS;
+    Jac<F>* terms;
+    CUDA_TRY(sc.alloc(&terms, count * rows * 2 * ntp));
+    // shared commitment randomness: the constants of all equations along one bucket structure (as in proof_element),
+    // the sum in slot 0 of the a = 1 row
+    const bool const_sums = var_tables && n0 * PipSplit<F>::PARTS >= 64 && count >= 16;
+    // identities in the constant slots no product writes: those of the a = 0 rows, with const_sums those of every row
+    if (n0 > 0)
+      CUDA_TRY(cudaMemset2DAsync(terms, (const_sums ? 1 : 2) * ntp * sizeof(Jac<F>), 0, n0 * PARTS * sizeof(Jac<F>),
+                                 count * rows * (const_sums ? 2 : 1), ctx->stream));
+    if (!var_tables) {
+      LAUNCH_B((k_rerand_terms<F>), (size_t)rows * nprod * PARTS, count, terms, sv, svs, nconst, B, n0, dcom, ncom,
+               coms_shared ? (size_t)0 : 2 * ncom, rows, (size_t)0, nprod, PARTS);
+    } else {
+      // the commitment tables are built on the second stream while the constant terms run on the main one
+      Aff<F>* ptab;
+      Jac<F>* J;
+      CUDA_TRY(shared_base_alloc<F>(sc, 2 * ncom, &ptab, &J));
+      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
+      cudaEvent_t fork, join;
+      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
+      if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
+        cudaEventDestroy(fork);
+        FAIL(GS_ECUDA, "rerandomize: event creation failed");
+      }
+      cudaEventRecord(fork, ctx->stream);
+      cudaStreamWaitEvent(ctx->stream2, fork, 0);
+      cudaStream_t main_stream = ctx->stream;
+      ctx->stream = ctx->stream2;
+      int rct = [&]() -> int {
+        int rcb = shared_base_tables<F>(ctx, dcom, 2 * ncom, ptab, J);
+        if (rcb) return rcb;
+        LAUNCH_B((k_rerand_com_terms_tab<F>), (size_t)rows * 2 * ncom, count, terms, sv, svs, nconst, ptab, n0, ncom, rows);
+        return GS_OK;
+      }();
+      cudaEventRecord(join, ctx->stream2);
+      ctx->stream = main_stream;
+      int rcc = [&]() -> int {
+        if (n0 == 0) return GS_OK;
+        if (const_sums) return shared_scalar_sums<F>(ctx, sc, sv, svs, rows, B, n0, count, terms + ntp, 2 * ntp);
+        LAUNCH_B((k_rerand_terms<F>), (size_t)rows * n0, count, terms, sv, svs, nconst, B, n0, dcom, ncom, (size_t)0, rows,
+                 (size_t)0, n0, 1);
+        return GS_OK;
+      }();
+      cudaStreamWaitEvent(ctx->stream, join, 0);
+      cudaEventDestroy(fork);
+      cudaEventDestroy(join);
+      if (rct) return rct;
+      if (rcc) return rcc;
+    }
+    int rc = reduce_rows<F>(ctx, terms, ntp, ntp, rows * 2, count);
+    if (rc) return rc;
+    vs.p[0] = terms;
+    vs.p[1] = terms + ntp;
+    vs.inst[0] = vs.inst[1] = (size_t)rows * 2 * ntp;
+    vs.row[0] = vs.row[1] = 2 * ntp;
+  }
+  Jac<F>* kt;
+  int KT;
+  int rc = proof_key_sums<F>(ctx, sc, count, rows, ncoef, coef, T, e, &kt, &KT);
+  if (rc) return rc;
+  LAUNCH_B((k_rerand_finish<F>), (size_t)rows * 2, count, dout, rows, kt, KT, dold, vs);
+  return GS_OK;
 }
 
 template <class F>

@@ -16,7 +16,7 @@ EXPORTED_SYMBOLS = [
     "gs_profile_enable", "gs_profile_read", "gs_diag_fpmul_rate",
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
-    "gs_prove", "gs_prove_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
     "gs_com1_matmul", "gs_com2_matmul", "gs_fr_matmul",
@@ -73,6 +73,8 @@ def load_library():
             getattr(lib, f).argtypes = [vp, sz, vp, vp, vp]
         lib.gs_prove.argtypes = [vp, ci, sz, sz] + [vp] * 10
         lib.gs_prove_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 8 + [ci, vp, vp]
+        lib.gs_rerandomize.argtypes = [vp, ci, sz, sz] + [vp] * 14
+        lib.gs_rerandomize_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10 + [ci] + [vp] * 4
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
@@ -250,6 +252,39 @@ class Engine:
         self._chk(self.lib.gs_prove_batch(self.h, ty, count, m, n, *[k[1] for k in ks], 1 if shared_vars else 0,
                                           ctypes.cast(pi, ctypes.c_void_p), ctypes.cast(th, ctypes.c_void_p)))
         return pi.raw[: count * cx * COM2], th.raw[: count * cy * COM1]
+
+    def rerandomize_batch(self, ty, count, m, n, a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand,
+                          shared_coms=False):
+        """`count` committed proofs rerandomised in one pass (gs_rerandomize_batch) with fresh R' = x_rand, S' = y_rand,
+        T' = pf_rand; returns (xcoms, ycoms, pi, theta) bytes, proof-major.  With shared_coms the commitments and R', S'
+        are one set for every equation, and so are the returned commitments."""
+        cx, cy = _cx(ty), _cy(ty)
+        reps = 1 if shared_coms else count
+        if count and m and n:
+            assert len(a_consts) == count * n * _a_size(ty) and len(b_consts) == count * m * _b_size(ty)
+            assert len(gamma) == count * m * n * FR and len(pf_rand) == count * cx * cy * FR
+            assert len(pi) == count * cx * COM2 and len(theta) == count * cy * COM1
+            assert len(xcoms) == reps * m * COM1 and len(ycoms) == reps * n * COM2
+            assert len(x_rand) == reps * m * cx * FR and len(y_rand) == reps * n * cy * FR
+        outs = [ctypes.create_string_buffer(max(1, k)) for k in
+                (reps * m * COM1, reps * n * COM2, count * cx * COM2, count * cy * COM1)]
+        ks = [_buf(x) for x in (a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand)]
+        self._chk(self.lib.gs_rerandomize_batch(self.h, ty, count, m, n, *[k[1] for k in ks], 1 if shared_coms else 0,
+                                                *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
+        return (outs[0].raw[: reps * m * COM1], outs[1].raw[: reps * n * COM2], outs[2].raw[: count * cx * COM2],
+                outs[3].raw[: count * cy * COM1])
+
+    def rerandomize(self, ty, m, n, a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand):
+        """One committed proof rerandomised (gs_rerandomize); returns (xcoms, ycoms, pi, theta) bytes."""
+        cx, cy = _cx(ty), _cy(ty)
+        if m and n:
+            assert len(a_consts) == n * _a_size(ty) and len(b_consts) == m * _b_size(ty) and len(gamma) == m * n * FR
+            assert len(xcoms) == m * COM1 and len(ycoms) == n * COM2 and len(pi) == cx * COM2 and len(theta) == cy * COM1
+            assert len(x_rand) == m * cx * FR and len(y_rand) == n * cy * FR and len(pf_rand) == cx * cy * FR
+        outs = [ctypes.create_string_buffer(max(1, k)) for k in (m * COM1, n * COM2, cx * COM2, cy * COM1)]
+        ks = [_buf(x) for x in (a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand)]
+        self._chk(self.lib.gs_rerandomize(self.h, ty, m, n, *[k[1] for k in ks], *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
+        return outs[0].raw[: m * COM1], outs[1].raw[: n * COM2], outs[2].raw[: cx * COM2], outs[3].raw[: cy * COM1]
 
     @staticmethod
     def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, gamma_rows=None):

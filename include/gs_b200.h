@@ -132,7 +132,31 @@ int gs_prove_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, cons
                    const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, int shared_vars,
                    gs_com2* out_pi, gs_com1* out_theta);
 
-/* ---- verification (src/verifier.rs) ----------------------------------------------------- */
+/* ---- rerandomisation of committed proofs (not in the reference) ---------------------------------- */
+/* Turns a CProof (commitments + proof) into a fresh-looking one for the same statement without the witnesses or the
+ * old randomness (Belenkiy et al., CRYPTO 2009; PAPERS.md).  With fresh R' = x_rand (m x cx), S' = y_rand (n x cy)
+ * and T' = pf_rand (cy x cx, as for gs_prove):
+ *   c' = c + R' u_x                     d' = d + S' v_y
+ *   pi'    = pi    + R'^T iota_y(B) + (R'^T Gamma) d + (R'^T Gamma S' - T'^T) v_y
+ *   theta' = theta + S'^T iota_x(A) + (S'^T Gamma^T) c + T' u_x
+ * (u_x = u[..cx], v_y = v[..cy]; iota = iota_1/2 on a group-typed side, x W1 / y W2 on a scalar-typed one).  The
+ * result is byte for byte commit + prove of the same witnesses under R + R', S + S', T + T' + S'^T Gamma^T R: with
+ * uniform R', S', T' it is distributed exactly as a fresh proof.  Arrays as gs_prove_batch / gs_verify_batch:
+ * a_consts[count][n], b_consts[count][m], gamma[count][m][n], pi[count][cx], theta[count][cy], pf_rand[count][cy][cx],
+ * out_pi[count][cx], out_theta[count][cy]; xcoms, ycoms, x_rand, y_rand, out_xcoms, out_ycoms are [count][...], or ONE
+ * set used by every equation when shared_coms != 0 (a multi-equation statement over one set of commitments).
+ * Return codes as gs_prove_batch.  gs_rerandomize is the batch of one. */
+int gs_rerandomize(gs_ctx* ctx, int type, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                   const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                   const gs_com1* theta, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand,
+                   gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta);
+int gs_rerandomize_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
+                         const void* b_consts, const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms,
+                         const gs_com2* pi, const gs_com1* theta, const gs_fr* x_rand, const gs_fr* y_rand,
+                         const gs_fr* pf_rand, int shared_coms, gs_com1* out_xcoms, gs_com2* out_ycoms,
+                         gs_com2* out_pi, gs_com1* out_theta);
+
+/* ---- verification (src/verifier.rs)----------------------------------------------------- */
 /* Verifiable::verify :23-157 for `count` independent (equation, proof) instances of the same
  * type and shape, each laid out contiguously with the given element counts:
  *   a_consts[count][n], b_consts[count][m], gamma[count][m][n], target[count],

@@ -50,6 +50,16 @@ extern "C" {
     pub fn gs_prove_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                           gamma: *const GsFr, x: *const u8, y: *const u8, x_rand: *const GsFr, y_rand: *const GsFr,
                           pf_rand: *const GsFr, shared: i32, out_pi: *mut GsCom2, out_theta: *mut GsCom1) -> i32;
+    // not in the reference: a committed proof rerandomised without the witnesses (shared_coms != 0: one set of commitments)
+    pub fn gs_rerandomize(ctx: *mut GsCtx, ty: i32, m: usize, n: usize, a: *const u8, b: *const u8, gamma: *const GsFr,
+                          xcoms: *const GsCom1, ycoms: *const GsCom2, pi: *const GsCom2, theta: *const GsCom1,
+                          x_rand: *const GsFr, y_rand: *const GsFr, pf_rand: *const GsFr, out_xcoms: *mut GsCom1,
+                          out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1) -> i32;
+    pub fn gs_rerandomize_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
+                                gamma: *const GsFr, xcoms: *const GsCom1, ycoms: *const GsCom2, pi: *const GsCom2,
+                                theta: *const GsCom1, x_rand: *const GsFr, y_rand: *const GsFr, pf_rand: *const GsFr,
+                                shared_coms: i32, out_xcoms: *mut GsCom1, out_ycoms: *mut GsCom2, out_pi: *mut GsCom2,
+                                out_theta: *mut GsCom1) -> i32;
     // verifier.rs:23-157
     pub fn gs_verify_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                            gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,

@@ -117,3 +117,36 @@ pub fn prove_statement_ppe<E: Gpu, CR: Rng>(equations: &[PPE<E>], xvars: &[E::G1
         pi: pi[2 * i..2 * i + 2].iter().map(Com2::from_abi).collect(), theta: theta[2 * i..2 * i + 2].iter().map(Com1::from_abi).collect(),
         equ_type: EquType::PairingProduct, rand }).collect()
 }
+
+/// Not in the reference: a fresh-looking CProof of the same PPE statement from `proof` alone, without the witnesses or the
+/// old randomness (`gs_rerandomize`; Belenkiy et al., CRYPTO 2009).  RNG order: R' (m x 2) rows, S' (n x 2) rows, then T'
+/// (2 x 2), row-major -- commit_and_prove's.  The openings are unknown to the caller, so the returned `rand` matrices are empty.
+pub fn rerandomize_ppe<E: Gpu, CR: Rng>(equ: &PPE<E>, proof: &CProof<E>, crs: &CRS<E>, rng: &mut CR) -> CProof<E> {
+    let (m, n) = (proof.xcoms.coms.len(), proof.ycoms.coms.len());
+    assert_eq!(proof.equ_proofs.len(), 1);
+    assert_eq!((equ.a_consts.len(), equ.b_consts.len(), equ.gamma.len()), (n, m, m));
+    let mut draw = |rows: usize| -> Matrix<E::ScalarField> { (0..rows).map(|_| (0..2).map(|_| E::ScalarField::rand(rng)).collect()).collect() };
+    let (r2, s2, t2) = (draw(m), draw(n), draw(2));
+    let ep = &proof.equ_proofs[0];
+    let (a, b, g) = (g1s::<E>(&equ.a_consts), g2s::<E>(&equ.b_consts), fr_matrix::<E>(&equ.gamma));
+    let xc: Vec<GsCom1> = proof.xcoms.coms.iter().map(|c| c.abi()).collect();
+    let yc: Vec<GsCom2> = proof.ycoms.coms.iter().map(|c| c.abi()).collect();
+    let pi: Vec<GsCom2> = ep.pi.iter().map(|c| c.abi()).collect();
+    let th: Vec<GsCom1> = ep.theta.iter().map(|c| c.abi()).collect();
+    let (r, s, t) = (fr_matrix::<E>(&r2), fr_matrix::<E>(&s2), fr_matrix::<E>(&t2));
+    let mut oxc = vec![Com1::<E>::zero().abi(); m];
+    let mut oyc = vec![Com2::<E>::zero().abi(); n];
+    let mut opi = vec![Com2::<E>::zero().abi(); 2];
+    let mut oth = vec![Com1::<E>::zero().abi(); 2];
+    with_crs(&crs.abi(), |c| check(c, unsafe {
+        gs_rerandomize(c.raw(), 0, m, n, bytes_of(&a).as_ptr(), bytes_of(&b).as_ptr(), g.as_ptr(), xc.as_ptr(), yc.as_ptr(),
+                       pi.as_ptr(), th.as_ptr(), r.as_ptr(), s.as_ptr(), t.as_ptr(), oxc.as_mut_ptr(), oyc.as_mut_ptr(),
+                       opi.as_mut_ptr(), oth.as_mut_ptr())
+    }));
+    CProof {
+        xcoms: Commit1 { coms: oxc.iter().map(Com1::from_abi).collect(), rand: vec![] },
+        ycoms: Commit2 { coms: oyc.iter().map(Com2::from_abi).collect(), rand: vec![] },
+        equ_proofs: vec![EquProof { pi: opi.iter().map(Com2::from_abi).collect(), theta: oth.iter().map(Com1::from_abi).collect(),
+                                    equ_type: EquType::PairingProduct, rand: vec![] }],
+    }
+}
