@@ -18,7 +18,7 @@ reference's order, which makes every output reproducible bit-for-bit.
 The reference signals misuse by assert!/panic; here those are AssertionError / GsError.
 """
 from dataclasses import dataclass, field
-from typing import List
+from typing import List, Tuple
 
 from . import ffi
 from .ffi import Engine, GsError
@@ -51,6 +51,23 @@ def _flat(m):
 
 # ---------------------------------------------------------------- CRS  (generator.rs)
 @dataclass
+class ExtractionKey:
+    """The trapdoor of a binding CRS: a1, a2 of generate_crs (Fr bytes), with u[0] = (p1, a1 p1), v[0] = (p2, a2 p2).
+    Whoever holds it opens every commitment made under that CRS (extract_G1 and the other extract functions)."""
+    a1: bytes
+    a2: bytes
+
+    def to_bytes(self) -> bytes:
+        return self.a1 + self.a2
+
+    @staticmethod
+    def from_bytes(b: bytes) -> "ExtractionKey":
+        if len(b) != 2 * FR:
+            raise ValueError(f"ExtractionKey: {len(b)} bytes, expected {2 * FR}")
+        return ExtractionKey(b[:FR], b[FR:])
+
+
+@dataclass
 class CRS:
     u: List[bytes]       # 2 x Com1
     v: List[bytes]       # 2 x Com2
@@ -62,10 +79,16 @@ class CRS:
     @staticmethod
     def generate_crs(rng, engine: Engine = None) -> "CRS":
         """generator.rs:81-118; RNG order p1 <- G1, p2 <- G2, a1, a2, t1, t2 <- Fr (:86-93)."""
+        return CRS.generate_crs_with_trapdoor(rng, engine)[0]
+
+    @staticmethod
+    def generate_crs_with_trapdoor(rng, engine: Engine = None) -> "Tuple[CRS, ExtractionKey]":
+        """generate_crs that also returns the binding key's trapdoor (a1, a2) instead of dropping it (not in the reference;
+        ExtGen of Groth & Sahai, EUROCRYPT 2008).  Exactly generate_crs's draws: the same rng state gives the same CRS."""
         eng = engine or default_engine()
         p1, p2 = rng.g1(), rng.g2()
         a1, a2, t1, t2 = rng.fr(), rng.fr(), rng.fr(), rng.fr()
-        return CRS.from_bytes(eng.crs_generate(p1, p2, a1, a2, t1, t2), eng, loaded=True)
+        return CRS.from_bytes(eng.crs_generate(p1, p2, a1, a2, t1, t2), eng, loaded=True), ExtractionKey(a1, a2)
 
     @staticmethod
     def generate_hiding_crs(rng, engine: Engine = None) -> "CRS":
@@ -303,6 +326,45 @@ def rerandomize_batch(equations, proofs, crs: CRS, rng, shared_commitments: bool
         out.append(CProof(Commit1(_split(xcs[j], 192), []), Commit2(_split(ycs[j], 384), []),
                           [EquProof(_split(pis[k], 384), _split(ths[k], 192), ty, [])]))
     return out
+
+
+# ---------------------------------------------------------------- extraction with the binding key (not in the reference)
+# X = c.1 - a1 c.0 for a commitment under a binding CRS (u[0] = (p1, a1 p1), u[1] = t1 u[0]); scalar commitments give x p1
+# (x itself cannot be recovered), the G2 side likewise with a2 (gs_extract).  The key is checked against the engine's
+# current CRS -- `crs` when given, else the one loaded last -- and a mismatch raises GsError; a hiding CRS has no key.
+def _coms_of(coms): return coms.coms if isinstance(coms, _Commit) else list(coms)
+
+
+def _extract_engine(crs): return crs._use() if crs is not None else default_engine()
+
+
+def extract_G1(coms, key: ExtractionKey, crs: CRS = None) -> List[bytes]:
+    """The committed G1 values of a Commit1 (batch_commit_G1) or of a list of Com1."""
+    return _split(_extract_engine(crs).extract(b"".join(_coms_of(coms)), key.a1)[0], G1)
+
+
+def extract_G2(coms, key: ExtractionKey, crs: CRS = None) -> List[bytes]:
+    """The committed G2 values of a Commit2 (batch_commit_G2) or of a list of Com2."""
+    return _split(_extract_engine(crs).extract(ycoms=b"".join(_coms_of(coms)), ykey=key.a2)[1], G2)
+
+
+def extract_scalar_B1(coms, key: ExtractionKey, crs: CRS = None) -> List[bytes]:
+    """x * g1 for every commitment of a scalar x (batch_commit_scalar_to_B1)."""
+    return extract_G1(coms, key, crs)
+
+
+def extract_scalar_B2(coms, key: ExtractionKey, crs: CRS = None) -> List[bytes]:
+    """y * g2 for every commitment of a scalar y (batch_commit_scalar_to_B2)."""
+    return extract_G2(coms, key, crs)
+
+
+def extract(com_proof: CProof, equ_type: int, key: ExtractionKey, crs: CRS = None) -> Tuple[List[bytes], List[bytes]]:
+    """Both sides of a CProof in one GPU call: (x values, y values).  Group-typed sides (x of PPE / MSMEG1, y of PPE /
+    MSMEG2) give the witnesses themselves; scalar-typed sides give x * g1 / y * g2."""
+    if equ_type not in (0, 1, 2, 3):
+        raise ValueError(f"extract: bad equation type {equ_type}")
+    xs, ys = _extract_engine(crs).extract(b"".join(com_proof.xcoms.coms), key.a1, b"".join(com_proof.ycoms.coms), key.a2)
+    return _split(xs, G1), _split(ys, G2)
 
 
 def verify_batch(equations, proofs, crs: CRS, randomized: bool = False, rho: bytes = None) -> List[bool]:

@@ -28,6 +28,8 @@ struct gs_ctx {
   cudaStream_t stream2 = nullptr;  // second stream of chunked batches (copy / compute overlap), created on first use
   gs::crs_dev* crs = nullptr;  // device
   bool crs_loaded = false;
+  bool xkey_valid = false, ykey_valid = false;  // gs_extract: the last key of each side that matched the loaded CRS
+  gs_fr xkey{}, ykey{};                         // (cleared by gs_crs_load / gs_crs_generate)
   gs_fixed_table<gs::FpOps> tab1;
   gs_fixed_table<gs::Fp2Ops> tab2;
   bool crs_lines_valid = false;   // the stored lines and the fixed-base tables are built by the FIRST call that needs them

@@ -16,7 +16,7 @@ EXPORTED_SYMBOLS = [
     "gs_profile_enable", "gs_profile_read", "gs_diag_fpmul_rate",
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
-    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
     "gs_com1_matmul", "gs_com2_matmul", "gs_fr_matmul",
@@ -75,6 +75,7 @@ def load_library():
         lib.gs_prove_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 8 + [ci, vp, vp]
         lib.gs_rerandomize.argtypes = [vp, ci, sz, sz] + [vp] * 14
         lib.gs_rerandomize_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10 + [ci] + [vp] * 4
+        lib.gs_extract.argtypes = [vp, sz, vp, vp, sz, vp, vp, vp, vp]
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
@@ -285,6 +286,19 @@ class Engine:
         ks = [_buf(x) for x in (a_consts, b_consts, gamma, xcoms, ycoms, pi, theta, x_rand, y_rand, pf_rand)]
         self._chk(self.lib.gs_rerandomize(self.h, ty, m, n, *[k[1] for k in ks], *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
         return outs[0].raw[: m * COM1], outs[1].raw[: n * COM2], outs[2].raw[: cx * COM2], outs[3].raw[: cy * COM1]
+
+    # ---- extraction with the binding key (gs_extract)
+    def extract(self, xcoms: bytes = b"", xkey: bytes = None, ycoms: bytes = b"", ykey: bytes = None):
+        """X_i = xcoms[i].1 - xkey xcoms[i].0 and Y_i = ycoms[i].1 - ykey ycoms[i].0 in one call; xkey = a1, ykey = a2 of
+        crs_generate (Fr bytes).  Returns (G1 bytes, G2 bytes).  A key that does not match the loaded CRS raises GsError."""
+        nx, ny = len(xcoms) // COM1, len(ycoms) // COM2
+        assert len(xcoms) == nx * COM1 and len(ycoms) == ny * COM2
+        assert (not nx or len(xkey) == FR) and (not ny or len(ykey) == FR)
+        ox, oy = ctypes.create_string_buffer(max(1, nx * G1)), ctypes.create_string_buffer(max(1, ny * G2))
+        ks = [_buf(x) if x else (None, ctypes.c_void_p(0)) for x in (xcoms, xkey, ycoms, ykey)]
+        self._chk(self.lib.gs_extract(self.h, nx, ks[0][1], ks[1][1], ny, ks[2][1], ks[3][1], ctypes.cast(ox, ctypes.c_void_p),
+                                      ctypes.cast(oy, ctypes.c_void_p)))
+        return ox.raw[: nx * G1], oy.raw[: ny * G2]
 
     @staticmethod
     def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, gamma_rows=None):

@@ -156,6 +156,16 @@ int gs_rerandomize_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n
                          const gs_fr* pf_rand, int shared_coms, gs_com1* out_xcoms, gs_com2* out_ycoms,
                          gs_com2* out_pi, gs_com1* out_theta);
 
+/* ---- extraction with the binding key (not in the reference) ------------------------------------ */
+/* Opens commitments with the binding key's trapdoor (Groth & Sahai, EUROCRYPT 2008; PAPERS.md).
+ * X_i = xcoms[i].1 - xkey * xcoms[i].0 (G1), Y_i = ycoms[i].1 - ykey * ycoms[i].0 (G2); xkey = a1, ykey = a2 of
+ * gs_crs_generate.  Commitments of scalars give x*g1 / y*g2.  Either side may be empty (n = 0: its pointers may be null).
+ * A key is accepted iff it opens the loaded key's own commitments u[0], u[1] (v[0], v[1]) to the identity; otherwise, and
+ * under a hiding CRS, GS_EARG with nothing written.  GS_EARG as well without a loaded CRS or for a null pointer on a
+ * non-empty side. */
+int gs_extract(gs_ctx* ctx, size_t nx, const gs_com1* xcoms, const gs_fr* xkey, size_t ny, const gs_com2* ycoms,
+               const gs_fr* ykey, gs_g1* out_x, gs_g2* out_y);
+
 /* ---- verification (src/verifier.rs)----------------------------------------------------- */
 /* Verifiable::verify :23-157 for `count` independent (equation, proof) instances of the same
  * type and shape, each laid out contiguously with the given element counts:

@@ -60,6 +60,9 @@ extern "C" {
                                 theta: *const GsCom1, x_rand: *const GsFr, y_rand: *const GsFr, pf_rand: *const GsFr,
                                 shared_coms: i32, out_xcoms: *mut GsCom1, out_ycoms: *mut GsCom2, out_pi: *mut GsCom2,
                                 out_theta: *mut GsCom1) -> i32;
+    // not in the reference: commitments opened with the binding key's trapdoor (xkey = a1, ykey = a2 of gs_crs_generate)
+    pub fn gs_extract(ctx: *mut GsCtx, nx: usize, xcoms: *const GsCom1, xkey: *const GsFr, ny: usize, ycoms: *const GsCom2,
+                      ykey: *const GsFr, out_x: *mut GsG1, out_y: *mut GsG2) -> i32;
     // verifier.rs:23-157
     pub fn gs_verify_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                            gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,

@@ -9,6 +9,7 @@
 //! * dimension errors are the same panics (the C ABI's `GS_EDIM` is re-raised by `ffi::check`).
 #![allow(non_snake_case)]
 pub mod data_structures;
+pub mod extractor;
 pub mod ffi;
 pub mod generator;
 pub mod prover;
