@@ -157,6 +157,128 @@ GS_HD GS_INL void cq_fp2_dot3_k(fp2& r, const fp (&y)[6], const uint32_t* const 
   fp::sub(r.c1, r.c1, P1);
 }
 
+// lo + hi R = sum_t a[t] * B_t unreduced (fp.cuh rowsum_w), B_t streamed from the Q layout: B_t = b0[t], or with SUM the
+// limb-wise sum b0[t] + b1[t] (the carry of each quad is kept for the next one; both canonical, so B_t < 2p fits 12 limbs)
+template <int NT, bool SUM>
+GS_HD GS_INL void cq_mulsum_w(uint32_t (&lo)[12], uint32_t (&hi)[12], const fp (&a)[NT], const uint32_t* const (&b0)[NT],
+                              const uint32_t* const (&b1)[NT]) {
+  uint32_t E[12], O[12], cy[NT];
+#pragma unroll
+  for (int q = 0; q < 3; q++) {
+    q4 bl[NT];
+#pragma unroll
+    for (int t = 0; t < NT; t++) {
+      bl[t] = *(const q4*)(b0[t] + q * CQ_QUAD);
+      if (SUM) {
+        const q4 u = *(const q4*)(b1[t] + q * CQ_QUAD);
+        if (q == 0)
+          bl[t].v[0] = add_cc(bl[t].v[0], u.v[0]);
+        else {
+          add_cc(cy[t], 0xffffffffu);  // CC = carry out of the previous quad
+          bl[t].v[0] = addc_cc(bl[t].v[0], u.v[0]);
+        }
+#pragma unroll
+        for (int i = 1; i < 4; i++) bl[t].v[i] = addc_cc(bl[t].v[i], u.v[i]);
+        cy[t] = addc(0u, 0u);
+      }
+    }
+#pragma unroll
+    for (int ii = 0; ii < 4; ii++) {
+      uint32_t lim[NT];
+#pragma unroll
+      for (int t = 0; t < NT; t++) lim[t] = bl[t].v[ii];
+      if ((ii & 1) == 0) {
+        fp::rowsum_w<NT>(E, O, a, lim, q == 0 && ii == 0);
+        lo[q * 4 + ii] = E[0];
+      } else {
+        fp::rowsum_w<NT>(O, E, a, lim, false);
+        lo[q * 4 + ii] = O[0];
+      }
+    }
+  }
+  fp::window_out(hi, E, O);
+}
+
+// r = sum_{t<NT} Y_t X_t in Fp2 by Karatsuba with ONE Montgomery reduction per output component.  The three sums
+//     P0 = sum Y_t.c0 X_t.c0,   P1 = sum Y_t.c1 X_t.c1,   P2 = sum (Y_t.c0 + Y_t.c1)(X_t.c0 + X_t.c1)
+// are formed as unreduced 24-limb integers, with the component sums NOT reduced, so that exactly
+//     P2 - P0 - P1 = sum (Y_t.c0 X_t.c1 + Y_t.c1 X_t.c0),  in [0, 2 NT p^2)
+// and r.c1 = REDC(P2 - (P0 + P1)), r.c0 = REDC(P0 - P1 + K) with K = p 2^383 (4.92 p^2 > NT p^2 > P1, a multiple of p, so
+// the argument is >= 0 and congruent to P0 - P1).  Both arguments stay below 2 NT p^2 + 4.92 p^2 < p R = 9.84 p^2 for
+// NT <= 4, the bound of fp::redc_w, whose canonical result is therefore the one every other form produces.  The
+// rowsum_w windows need sum_t a[t] < R: at most 2 NT p < R for the component sums.
+// 3 NT Fp products + 2 reductions (NT = 2: 1,176 multiply-adds against the 1,332 of three reduced sums).
+// ld(a, c) fills a[t] with Y_t.c0 (c = 0), Y_t.c1 (c = 1), each canonical, or (c = 2) their plain integer sum
+// Y_t.c0 + Y_t.c1 of exactly those values; X_t.c0, X_t.c1 (canonical) are read from the Q layout.
+template <int NT, class LD>
+GS_HD GS_INL void cq_fp2_dot_w(fp2& r, LD ld, const uint32_t* const (&x0)[NT], const uint32_t* const (&x1)[NT]) {
+  static_assert(NT >= 1 && NT <= 4, "bounds above hold for NT <= 4");
+  uint32_t slo[12], shi[12];
+  {
+    uint32_t lo0[12], hi0[12], lo1[12], hi1[12];
+    {
+      fp a[NT];
+      ld(a, 0);
+      cq_mulsum_w<NT, false>(lo0, hi0, a, x0, x0);
+    }
+    {
+      fp a[NT];
+      ld(a, 1);
+      cq_mulsum_w<NT, false>(lo1, hi1, a, x1, x1);
+    }
+    // S = P0 + P1 (< 2 NT p^2 < 2^768),  D = P0 - P1 + K (the subtraction may wrap mod 2^768; adding K unwraps it)
+    uint32_t dlo[12], dhi[12];
+    slo[0] = add_cc(lo0[0], lo1[0]);
+#pragma unroll
+    for (int i = 1; i < 12; i++) slo[i] = addc_cc(lo0[i], lo1[i]);
+#pragma unroll
+    for (int i = 0; i < 11; i++) shi[i] = addc_cc(hi0[i], hi1[i]);
+    shi[11] = addc(hi0[11], hi1[11]);
+    dlo[0] = sub_cc(lo0[0], lo1[0]);
+#pragma unroll
+    for (int i = 1; i < 12; i++) dlo[i] = subc_cc(lo0[i], lo1[i]);
+#pragma unroll
+    for (int i = 0; i < 11; i++) dhi[i] = subc_cc(hi0[i], hi1[i]);
+    dhi[11] = subc(hi0[11], hi1[11]);
+    // K = p << 383: limbs 11..23 = (p[j] << 31) | (p[j-1] >> 1)
+    dlo[11] = add_cc(dlo[11], FpParams::mod(0) << 31);
+#pragma unroll
+    for (int j = 1; j < 12; j++) dhi[j - 1] = addc_cc(dhi[j - 1], (FpParams::mod(j) << 31) | (FpParams::mod(j - 1) >> 1));
+    dhi[11] = addc(dhi[11], FpParams::mod(11) >> 1);
+    fp::redc_w(r.c0, dlo, dhi);
+  }
+  {
+    uint32_t lo2[12], hi2[12];
+    {
+      fp a[NT];
+      ld(a, 2);
+      cq_mulsum_w<NT, true>(lo2, hi2, a, x0, x1);
+    }
+    lo2[0] = sub_cc(lo2[0], slo[0]);
+#pragma unroll
+    for (int i = 1; i < 12; i++) lo2[i] = subc_cc(lo2[i], slo[i]);
+#pragma unroll
+    for (int i = 0; i < 11; i++) hi2[i] = subc_cc(hi2[i], shi[i]);
+    hi2[11] = subc(hi2[11], shi[11]);
+    fp::redc_w(r.c1, lo2, hi2);
+  }
+}
+
+// register-side operands of cq_fp2_dot_w held in registers: y[2t], y[2t+1] = Y_t.c0, Y_t.c1
+template <int NT>
+struct cq_yreg {
+  const fp (&y)[2 * NT];
+  GS_HD GS_INL void operator()(fp (&a)[NT], int c) const {
+#pragma unroll
+    for (int t = 0; t < NT; t++) {
+      if (c < 2)
+        a[t] = y[2 * t + c];
+      else
+        fp::add_noreduce(a[t], y[2 * t], y[2 * t + 1]);
+    }
+  }
+};
+
 // load coefficient j of the accumulator set `f` into (y0, y1), optionally times xi and/or 2
 GS_HD GS_INL void cq_ld_coef(fp& y0, fp& y1, const uint32_t* f, int j, int lane, bool xi, bool dbl) {
   cq_ld(y0, cq_ptr(f, 2 * j, lane));
@@ -199,10 +321,12 @@ GS_HD GS_INL void cq_line_mul(int k, int lane, const uint32_t* fin, uint32_t* fo
 
 // Same with gamma = 1 (affine line scaled by 1/yP, pairing.cuh g2_affine_step):
 //     fout.a_k = alpha a_k + beta a_{k-2} + a_{k-3}
-// `tile` holds alpha.c0, alpha.c1, beta.c0, beta.c1 (4 Fp): 8 Fp products + 2 reductions per coefficient
-// instead of 12 + 2, and only two register-side operands.
+// `tile` holds alpha.c0, alpha.c1, beta.c0, beta.c1 (4 Fp): a two-term Fp2 dot product per coefficient instead of three,
+// and only two register-side operands.
+// GS_LINE_KARATSUBA selects the form of the dot products here and in cq_sqr: 0 = schoolbook (cq_fp2_dot), 1 = Karatsuba
+// with three reduced sums (cq_fp2_dot2_k), 2 = Karatsuba with one reduction per component (cq_fp2_dot_w).
 #ifndef GS_LINE_KARATSUBA
-#define GS_LINE_KARATSUBA 1
+#define GS_LINE_KARATSUBA 2
 #endif
 GS_HD GS_INL void cq_line_mul_u(int k, int lane, const uint32_t* fin, uint32_t* fout, const uint32_t* tile, bool active) {
   fp y[4];
@@ -212,7 +336,9 @@ GS_HD GS_INL void cq_line_mul_u(int k, int lane, const uint32_t* fin, uint32_t* 
   fp2 r, u;
   const uint32_t* x0[2] = {cq_ptr(tile, 0, lane), cq_ptr(tile, 2, lane)};
   const uint32_t* x1[2] = {cq_ptr(tile, 1, lane), cq_ptr(tile, 3, lane)};
-#if GS_LINE_KARATSUBA
+#if GS_LINE_KARATSUBA == 2
+  cq_fp2_dot_w<2>(r, cq_yreg<2>{y}, x0, x1);
+#elif GS_LINE_KARATSUBA == 1
   cq_fp2_dot2_k(r, y, x0, x1);
 #else
   cq_fp2_dot<2>(r, y, x0, x1);
@@ -225,7 +351,8 @@ GS_HD GS_INL void cq_line_mul_u(int k, int lane, const uint32_t* fin, uint32_t* 
 
 // ------------------------------------------------------------------ squaring
 // fout = fin^2:  b_k = sum_{i<=j, i+j = k mod 6} c_ij a_i a_j,  c_ij = (i<j ? 2 : 1) * (i+j >= 6 ? xi : 1).
-// Even k have 4 terms (2 doubled pairs + 2 squares), odd k have 3 doubled pairs; two passes of <= 2 terms.
+// Even k have 4 terms (2 doubled pairs + 2 squares), odd k have 3 doubled pairs; two passes of <= 2 terms (one pass over
+// all four terms needs more than the 168 registers k_miller4 has).
 GS_HD GS_INL void cq_sqr(int k, int lane, const uint32_t* fin, uint32_t* fout) {
   int ti[4], tj[4], nt = 0;
   for (int i = 0; i < 6; i++) {
@@ -243,7 +370,9 @@ GS_HD GS_INL void cq_sqr(int k, int lane, const uint32_t* fin, uint32_t* fout) {
     cq_ld_coef(y[2], y[3], fin, tj[1], lane, ti[1] + tj[1] >= 6, ti[1] < tj[1]);
     const uint32_t* x0[2] = {cq_ptr(fin, 2 * ti[0], lane), cq_ptr(fin, 2 * ti[1], lane)};
     const uint32_t* x1[2] = {cq_ptr(fin, 2 * ti[0] + 1, lane), cq_ptr(fin, 2 * ti[1] + 1, lane)};
-#if GS_LINE_KARATSUBA
+#if GS_LINE_KARATSUBA == 2
+    cq_fp2_dot_w<2>(r, cq_yreg<2>{y}, x0, x1);
+#elif GS_LINE_KARATSUBA == 1
     cq_fp2_dot2_k(r, y, x0, x1);
 #else
     cq_fp2_dot<2>(r, y, x0, x1);
@@ -256,7 +385,9 @@ GS_HD GS_INL void cq_sqr(int k, int lane, const uint32_t* fin, uint32_t* fout) {
     cq_ld_coef(y[2], y[3], fin, tj[3], lane, ti[3] + tj[3] >= 6, ti[3] < tj[3]);
     const uint32_t* x0[2] = {cq_ptr(fin, 2 * ti[2], lane), cq_ptr(fin, 2 * ti[3], lane)};
     const uint32_t* x1[2] = {cq_ptr(fin, 2 * ti[2] + 1, lane), cq_ptr(fin, 2 * ti[3] + 1, lane)};
-#if GS_LINE_KARATSUBA
+#if GS_LINE_KARATSUBA == 2
+    cq_fp2_dot_w<2>(r2, cq_yreg<2>{y}, x0, x1);
+#elif GS_LINE_KARATSUBA == 1
     cq_fp2_dot2_k(r2, y, x0, x1);
 #else
     cq_fp2_dot<2>(r2, y, x0, x1);
@@ -266,7 +397,11 @@ GS_HD GS_INL void cq_sqr(int k, int lane, const uint32_t* fin, uint32_t* fout) {
     cq_ld_coef(y[0], y[1], fin, tj[2], lane, ti[2] + tj[2] >= 6, ti[2] < tj[2]);
     const uint32_t* x0[1] = {cq_ptr(fin, 2 * ti[2], lane)};
     const uint32_t* x1[1] = {cq_ptr(fin, 2 * ti[2] + 1, lane)};
+#if GS_LINE_KARATSUBA == 2
+    cq_fp2_dot_w<1>(r2, cq_yreg<1>{y}, x0, x1);
+#else
     cq_fp2_dot<1>(r2, y, x0, x1);
+#endif
   }
   cq_ld_coef(r.c0, r.c1, fout, k, lane, false, false);
   fp2::add(r, r, r2);
@@ -289,18 +424,23 @@ GS_HD GS_INL void cq_mul(int k, int lane, const uint32_t* f, const uint32_t* g, 
       x0[t] = cq_ptr(g, 2 * i, lane);
       x1[t] = cq_ptr(g, 2 * i + 1, lane);
     }
+// GS_MUL_KARATSUBA: 0 = schoolbook, 1 = three reduced sums (cq_fp2_dot3_k), 2 = one reduction per component
 #ifndef GS_MUL_KARATSUBA
-#define GS_MUL_KARATSUBA 1
+#define GS_MUL_KARATSUBA 2
 #endif
     if (h == 0) {
-#if GS_MUL_KARATSUBA
+#if GS_MUL_KARATSUBA == 2
+      cq_fp2_dot_w<3>(r, cq_yreg<3>{y}, x0, x1);
+#elif GS_MUL_KARATSUBA == 1
       cq_fp2_dot3_k(r, y, x0, x1);
 #else
       cq_fp2_dot<3>(r, y, x0, x1);
 #endif
       cq_st_coef(fout, k, lane, r);  // parked in the output slot
     } else {
-#if GS_MUL_KARATSUBA
+#if GS_MUL_KARATSUBA == 2
+      cq_fp2_dot_w<3>(r2, cq_yreg<3>{y}, x0, x1);
+#elif GS_MUL_KARATSUBA == 1
       cq_fp2_dot3_k(r2, y, x0, x1);
 #else
       cq_fp2_dot<3>(r2, y, x0, x1);

@@ -332,11 +332,87 @@ struct Mont {
   }
   GS_HD static GS_INL void mulsum_finish(Mont& r, const uint32_t* E, const uint32_t* O) {
     uint32_t t[N];
+    window_out(t, E, O);
+    final_sub(r, t);
+  }
+  // the window after an even number of rows, divided by W: t = (O >> 32) + E
+  GS_HD static GS_INL void window_out(uint32_t* t, const uint32_t* E, const uint32_t* O) {
     t[0] = add_cc(O[1], E[0]);
 #pragma unroll
     for (int i = 1; i < N - 1; i++) t[i] = addc_cc(O[i + 1], E[i]);
     t[N - 1] = addc(0u, E[N - 1]);
+  }
+
+  // ---- the rows of rowsum_l WITHOUT the reduction: P = sum_t a[t] b[t] as an unreduced 2N-limb integer ("wide"), so
+  // that several such sums can be combined before ONE reduction (coop12.cuh cq_fp2_dot_w).  After row i, [0] of the
+  // E argument is limb i of P: it leaves the window (the next row never reads that slot).  After the N rows
+  // window_out(hi, E, O) gives limbs N..2N-1.  The window holds floor(partial sum / W^i) < (sum_t a[t]) W, so it fits
+  // N + 1 limbs (no carry out of O[N-1]) when sum_t a[t] < R; the b[t] may be anything below R.
+  template <int NT>
+  GS_HD static GS_INL void rowsum_w(uint32_t* E, uint32_t* O, const Mont (&a)[NT], const uint32_t (&bl)[NT], bool first) {
+    if (first) {
+#pragma unroll
+      for (int j = 0; j < N; j += 2) {
+        mul_wide(E[j], E[j + 1], a[0].l[j], bl[0]);
+        mul_wide(O[j], O[j + 1], a[0].l[j + 1], bl[0]);
+      }
+    } else {
+      E[0] = add_cc(E[0], O[1]);
+      madc_row_rshift(O, a[0].l + 1, bl[0]);
+      cmad_row(E, a[0].l, bl[0]);
+      O[N - 1] = addc(O[N - 1], 0u);
+    }
+#pragma unroll
+    for (int t = 1; t < NT; t++) {
+      cmad_row(O, a[t].l + 1, bl[t]);
+      cmad_row(E, a[t].l, bl[t]);
+      O[N - 1] = addc(O[N - 1], 0u);
+    }
+  }
+  // ---- one Montgomery reduction of a wide value:  r = (lo + hi R) / R mod p,  for lo + hi R < p R.
+  // The rows of `row` without the a*b part take the window from lo to t = (lo + M p) / R <= p (M < R the Montgomery
+  // quotient; the window stays below R / W^i + p + 1 < 2^(32(N+1))).  hi <= p - 1, so t + hi < 2p and one
+  // conditional subtraction canonicalises it.  N*N + N multiply-adds, like the reduction part of mulsum.
+  GS_HD static GS_INL void redc_w(Mont& r, const uint32_t (&lo)[N], const uint32_t (&hi)[N]) {
+    uint32_t E[N], O[N];
+#pragma unroll
+    for (int i = 0; i < N; i++) {
+      E[i] = lo[i];
+      O[i] = 0u;
+    }
+#pragma unroll
+    for (int i = 0; i < N; i += 2) {
+      redc_row(E, O, i == 0);
+      redc_row(O, E, false);
+    }
+    uint32_t t[N];
+    window_out(t, E, O);
+    t[0] = add_cc(t[0], hi[0]);
+#pragma unroll
+    for (int i = 1; i < N - 1; i++) t[i] = addc_cc(t[i], hi[i]);
+    t[N - 1] = addc(t[N - 1], hi[N - 1]);
     final_sub(r, t);
+  }
+  GS_HD static GS_INL void redc_row(uint32_t* E, uint32_t* O, bool first) {
+    uint32_t m;
+    if (first) {
+      m = mul_lo(E[0], PR::M0);
+      cmad_row_mod<1>(O, m);
+    } else {
+      // as in `row`: E is last row's O, O is last row's E two slots too high (O[1] at position 0); the carry of the
+      // position-0 merge goes into the shifted O chain
+      E[0] = add_cc(E[0], O[1]);
+      m = mul_lo(E[0], PR::M0);
+#pragma unroll
+      for (int j = 0; j < N - 2; j += 2) {
+        O[j] = madc_lo_cc(PR::mod(j + 1), m, O[j + 2]);
+        O[j + 1] = madc_hi_cc(PR::mod(j + 1), m, O[j + 3]);
+      }
+      O[N - 2] = madc_lo_cc(PR::mod(N - 1), m, 0u);
+      O[N - 1] = madc_hi(PR::mod(N - 1), m, 0u);
+    }
+    cmad_row_mod<0>(E, m);
+    O[N - 1] = addc(O[N - 1], 0u);
   }
   // plain limb-wise sum without reduction (inputs < p, result < 2p): an operand for mulsum that counts 2 units
   GS_HD static GS_INL void add_noreduce(Mont& r, const Mont& a, const Mont& b) {
