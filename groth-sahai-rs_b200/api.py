@@ -375,24 +375,41 @@ def verify_batch(equations, proofs, crs: CRS, randomized: bool = False, rho: byt
     reported valid (error <= 2^-62 over `rho`, drawn from the OS CSPRNG when not given); if it rejects, the exact
     per-proof verification below runs and says which proofs failed.  Inputs must be group members (deserialised values
     are), PPE targets members of GT."""
+    ty, m, n, arrays = _batch_arrays(equations, proofs, "verify_batch")
+    if randomized and crs._use().verify_batch_rand(ty, len(equations), m, n, *arrays, rho=rho):
+        return [True] * len(equations)
+    ok = crs._use().verify_batch(ty, len(equations), m, n, *arrays)
+    return [b == 1 for b in ok]
+
+
+def _batch_arrays(equations, proofs, name):
+    """(type, m, n, the eight C-ABI arrays) of a batch of one type and shape; ValueError names `name`."""
     assert len(equations) == len(proofs) and equations
     ty = equations[0].equ_type
     m, n = len(proofs[0].xcoms.coms), len(proofs[0].ycoms.coms)
     for e, p in zip(equations, proofs):     # one type and one shape per batch: a mixed batch would be mis-sliced silently
         if e.equ_type != ty or len(p.xcoms.coms) != m or len(p.ycoms.coms) != n:
-            raise ValueError("verify_batch: every (equation, proof) must have the same type and shape")
+            raise ValueError(f"{name}: every (equation, proof) must have the same type and shape")
         if len(p.equ_proofs) != 1 or p.equ_proofs[0].equ_type != ty:      # verifier.rs:25-26
-            raise ValueError("verify_batch: exactly one EquProof of the equation's type per CProof")
+            raise ValueError(f"{name}: exactly one EquProof of the equation's type per CProof")
         if len(e.a_consts) != n or len(e.b_consts) != m or len(e.gamma) != m or any(len(r) != n for r in e.gamma):
-            raise ValueError("verify_batch: constants / Gamma do not match the number of variables")
+            raise ValueError(f"{name}: constants / Gamma do not match the number of variables")
     cat = lambda f: b"".join(f(e, p) for e, p in zip(equations, proofs))
     arrays = (cat(lambda e, p: b"".join(e.a_consts)), cat(lambda e, p: b"".join(e.b_consts)),
               cat(lambda e, p: _flat(e.gamma)), cat(lambda e, p: e.target), cat(lambda e, p: b"".join(p.xcoms.coms)),
               cat(lambda e, p: b"".join(p.ycoms.coms)), cat(lambda e, p: b"".join(p.equ_proofs[0].pi)),
               cat(lambda e, p: b"".join(p.equ_proofs[0].theta)))
-    if randomized and crs._use().verify_batch_rand(ty, len(equations), m, n, *arrays, rho=rho):
-        return [True] * len(equations)
-    ok = crs._use().verify_batch(ty, len(equations), m, n, *arrays)
+    return ty, m, n, arrays
+
+
+def verify_each_randomized(equations, proofs, crs: CRS, rho: bytes = None) -> List[bool]:
+    """Per-proof verdicts of a batch of one type and shape at close to the randomised cost (opt-in, not in the reference):
+    each proof's four ComT entries are folded with its own random weights into one pairing product and ONE final
+    exponentiation (gs_verify_each_rand).  A bad proof is accepted with probability <= 2^-62 over `rho` (2*count + 1
+    64-bit words, drawn from the OS CSPRNG when not given), each proof on its own, so a batch with some bad proofs still
+    costs one randomised pass.  Inputs must be group members (deserialised values are), PPE targets members of GT."""
+    ty, m, n, arrays = _batch_arrays(equations, proofs, "verify_each_randomized")
+    ok = crs._use().verify_each_rand(ty, len(equations), m, n, *arrays, rho=rho)
     return [b == 1 for b in ok]
 
 

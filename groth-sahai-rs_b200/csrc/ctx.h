@@ -217,9 +217,24 @@ struct walk_ahead {  // G2 walks started early on the second stream (lone statem
   }
 };
 int g2_walk_ahead(gs_ctx* ctx, Scratch& sc, const g2_aff* Y, size_t nprob, int K, const uint8_t* slot_kind, walk_ahead* wa);
+// Single-entry products with one result PER ACCUMULATOR (gs_verify_each_rand): F[A] = the conjugated Miller value of
+// accumulator A (slots [A*S, A*S + S)), neither multiplied over the accumulators nor exponentiated.  The first nf slots of
+// every acc_stride-th accumulator (A = 0, acc_stride, 2 acc_stride, ...) are pairs whose G2 side is one of a few points
+// shared by the whole call, pts[pid[f]], with lines walked once (lines[(pid*68 + step)*2 + {0: lambda, 1: mu}], g2_lines);
+// their Y entries must be the identity so that the per-slot walk skips them.
+struct acc_each {
+  fp12* F = nullptr;
+  int acc_stride = 1;
+  int nf = 0;
+  int pid[4] = {0, 0, 0, 0};
+  const g2_aff* pts = nullptr;
+  const fp2* lines = nullptr;
+};
 int run_pairing_product(gs_ctx* ctx, Scratch& sc, const g1_aff* X, const g2_aff* Y, size_t nprob, int K, fp12* out_comt,
                         uint8_t* ok4, const fp12* target, fp12* out_partial, const uint8_t* slot_kind = nullptr,
-                        const walk_ahead* wa = nullptr, int ne = 4, int S_force = 0);
+                        const walk_ahead* wa = nullptr, int ne = 4, int S_force = 0, const acc_each* each = nullptr);
+// lines[(i*68 + step)*2 + {0: lambda, 1: mu}] of the n G2 points pts[i] (device), walked once each; *lines is owned by `sc`
+int g2_lines(gs_ctx* ctx, Scratch& sc, const g2_aff* pts, int n, fp2** lines);
 int crs_lines_build(gs_ctx* ctx);
 
 // finalexp.cu: f = prod_chunks F[(ch*ne + e)*nprob + p]; g = FE(f); writes out_comt[p*ne+e] and/or ok4[e*nprob + p]

@@ -248,6 +248,55 @@ __global__ void __launch_bounds__(128) k_fixed_tiles(const uint32_t* __restrict_
   }
 }
 
+// Single-entry products with one accumulator (or acc_stride of them) per proof (gs_verify_each_rand): the first nf slots of
+// accumulator A = q * acc_stride pair the proof's folded G1 points with G2 points shared by the whole call (the folded CRS
+// elements), whose lines were walked ONCE (gsi::g2_lines).  thread -> (f, q): 32 consecutive proofs of one f per warp, so
+// the line loads are uniform and, with acc_stride = 1, the 32 lanes of one tile row are written together.
+struct each_pids {
+  int n;
+  int pid[4];
+};
+__global__ void __launch_bounds__(128) k_each_fixed_tiles(const uint32_t* __restrict__ PW, const g2_aff* __restrict__ pts,
+                                                          const fp2* __restrict__ lines, uint32_t* __restrict__ tiles,
+                                                          uint32_t* __restrict__ masks, size_t nq, int acc_stride, int S,
+                                                          each_pids ep) {
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= (size_t)ep.n * nq) return;
+  const size_t q = id % nq;
+  const int f = (int)(id / nq);
+  const int pid = ep.pid[f];
+  if (pts[pid].is_inf()) return;  // pair dropped
+  const size_t A = q * (size_t)acc_stride, k = A * S + f;
+  const int lane = (int)(A & 31);
+  const uint32_t* pw = PW + k * 2 * 12;  // (nprob = np = 1, one G1 coordinate)
+  fp s, wv;
+  uint32_t nz = 0;
+#pragma unroll
+  for (int j = 0; j < 12; j++) {
+    s.l[j] = pw[j];
+    wv.l[j] = pw[12 + j];
+    nz |= wv.l[j];
+  }
+  if (!nz) return;  // identity G1 point: pair dropped
+  const size_t bid = A >> 5;
+  atomicOr(&masks[bid * S + f], 1u << lane);
+  uint32_t* o = tiles + ((bid * S + f) * GS_NUM_LINES) * (size_t)M4_TILE;
+  const fp2* L = lines + (size_t)pid * GS_NUM_LINES * 2;
+#pragma unroll 1
+  for (int idx = 0; idx < GS_NUM_LINES; idx++, o += M4_TILE) {
+    const fp2 lam = L[idx * 2], mu = L[idx * 2 + 1];
+    fp v;
+    fp_mul_n(v, mu.c0, wv);
+    cq_st_stream(cq_ptr(o, 0, lane), v);
+    fp_mul_n(v, mu.c1, wv);
+    cq_st_stream(cq_ptr(o, 1, lane), v);
+    fp_mul_n(v, lam.c0, s);
+    cq_st_stream(cq_ptr(o, 2, lane), v);
+    fp_mul_n(v, lam.c1, s);
+    cq_st_stream(cq_ptr(o, 3, lane), v);
+  }
+}
+
 // ------------------------------------------------------------------ lone statements: walk ahead, evaluate later
 // The walk of a G2 point (lambda, mu per step) does not depend on the G1 side; for a lone statement it is started on
 // a second stream while the statement MSM -- which produces some of the G1 slots -- still runs (verify.cu), and the
@@ -718,6 +767,20 @@ int gsi::g2_walk_ahead(gs_ctx* ctx, Scratch& sc, const g2_aff* Y, size_t nprob, 
   return GS_OK;
 }
 
+// the inversion-free walk of k_g2_walk_jac / k_g2_lines_from_jac over n points (one "problem", slot k = point k)
+int gsi::g2_lines(gs_ctx* ctx, Scratch& sc, const g2_aff* pts, int n, fp2** lines) {
+  std::vector<uint32_t> hwalk(n);
+  for (int i = 0; i < n; i++) hwalk[i] = (uint32_t)i;
+  uint32_t* dwalk;
+  fp2* rec;
+  CUDA_TRY(upload(ctx, sc, &dwalk, hwalk.data(), hwalk.size()));
+  CUDA_TRY(sc.alloc(lines, (size_t)n * GS_NUM_LINES * 2));
+  CUDA_TRY(sc.alloc(&rec, (size_t)n * GS_NUM_LINES * 4));
+  LAUNCH_CFG(k_g2_walk_jac, (size_t)n, 64, 0, pts, rec, (size_t)1, (size_t)1, n, dwalk, n);
+  LAUNCH_CFG(k_g2_lines_from_jac, (size_t)n * 128, 128, 0, pts, rec, *lines, (size_t)1, (size_t)1, n, dwalk);
+  return GS_OK;
+}
+
 // ------------------------------------------------------------------ pairing-product pipeline
 // X, Y: device slot arrays [2][K][nprob].  Produces either ComT values (out_comt, AoS [p][4]) or
 // per-entry verdict bytes ok4[4][nprob] (compared with 1 / target).
@@ -725,12 +788,15 @@ int gsi::g2_walk_ahead(gs_ctx* ctx, Scratch& sc, const g2_aff* Y, size_t nprob, 
 // bytes of HBM; a pass is sized to a whole number of k_miller4 waves (2 groups x 148 SMs x 32 accumulators
 // / 4 entries = 2,368 problems per wave) when the batch is large enough.
 // ne = 1 (gs_verify_batch_rand): SINGLE-entry products prod_k e(X_k, Y_k) over arrays X[K][nprob], Y[K][nprob]; every
-// accumulator takes exactly S = S_force slots (K a multiple of it, S a multiple of 4), un-exponentiated result in out_partial.
+// accumulator takes exactly S = S_force slots (K a multiple of it, S a multiple of 4), un-exponentiated result in out_partial,
+// or, with `each` (gs_verify_each_rand), one un-exponentiated result per accumulator in each->F.
 int gsi::run_pairing_product(gs_ctx* ctx, Scratch& sc, const g1_aff* X, const g2_aff* Y, size_t nprob, int K,
                                fp12* out_comt, uint8_t* ok4, const fp12* target, fp12* out_partial, const uint8_t* slot_kind,
-                               const walk_ahead* wa, int ne, int S_force) {
-  if (ne != 4 && (ne != 1 || nprob != 1 || !out_partial || slot_kind || wa || S_force < 4 || S_force % 4 || K % S_force))
+                               const walk_ahead* wa, int ne, int S_force, const acc_each* each) {
+  if (ne != 4 && (ne != 1 || nprob != 1 || (!out_partial == !each) || slot_kind || wa || S_force < 4 || S_force % 4 || K % S_force))
     FAIL(GS_EARG, "pairing product: bad single-entry configuration");
+  if (each && (ne != 1 || each->nf < 0 || each->nf > 4 || each->nf > S_force || each->acc_stride < 1 || (K / S_force) % each->acc_stride))
+    FAIL(GS_EARG, "pairing product: bad per-accumulator configuration");
   const int na = ne == 4 ? 2 : 1;
   const size_t wave = 2368;
   if (K == 0) {  // a shard that owns no slot: empty product
@@ -789,7 +855,10 @@ int gsi::run_pairing_product(gs_ctx* ctx, Scratch& sc, const g1_aff* X, const g2
   CUDA_TRY(sc.alloc(&PW, (size_t)na * K * 24 * pc));
   CUDA_TRY(sc.alloc(&tiles, nblk_max * S * GS_NUM_LINES * (size_t)M4_TILE));
   CUDA_TRY(sc.alloc(&masks, nblk_max * S));
-  CUDA_TRY(sc.alloc(&F, (size_t)nchunk * ne * nprob));
+  if (each)
+    F = each->F;
+  else
+    CUDA_TRY(sc.alloc(&F, (size_t)nchunk * ne * nprob));
   for (size_t p0 = 0; p0 < nprob; p0 += pc) {
     size_t np = nprob - p0 < pc ? nprob - p0 : pc;
     size_t nblk = ((np * nchunk + 31) / 32) * ne;
@@ -798,6 +867,13 @@ int gsi::run_pairing_product(gs_ctx* ctx, Scratch& sc, const g1_aff* X, const g2
     // (6 points per thread was measured too: 162.6 ms vs 151.0 ms per 65,536 proofs -- the extra local memory costs
     // more than the shared inversion saves)
     if (fs.n) LAUNCH(k_fixed_tiles, (size_t)fs.n * 2 * np, PW, ctx->crs_lines, ctx->crs, tiles, masks, p0, np, K, S, fs);
+    if (each && each->nf) {
+      each_pids ep;
+      ep.n = each->nf;
+      for (int f = 0; f < 4; f++) ep.pid[f] = each->pid[f];
+      const size_t nq = (size_t)nchunk / each->acc_stride;
+      LAUNCH(k_each_fixed_tiles, (size_t)ep.n * nq, PW, each->pts, each->lines, tiles, masks, nq, each->acc_stride, S, ep);
+    }
     if (wa) {
       CUDA_TRY(cudaStreamWaitEvent(ctx->stream, wa->done, 0));
       LAUNCH(k_eval_tiles, (size_t)nwalk * np, PW, Y, wa->lines, tiles, masks, nprob, np, K, S, dwalk, nwalk, ne);
@@ -818,6 +894,7 @@ int gsi::run_pairing_product(gs_ctx* ctx, Scratch& sc, const g1_aff* X, const g2
     LAUNCH_CFG(k_miller4, ((nblk + CQ_GROUPS - 1) / CQ_GROUPS) * CQ_BLOCK_THREADS, CQ_BLOCK_THREADS, CQ_GROUPS * M4_SMEM, tiles, masks,
                F, nprob, p0, np, S, nchunk, nblk, ne);
   }
+  if (each) return GS_OK;
   const fp12* Fr = F;
   if (out_partial) {  // sharded statement: hand back the un-exponentiated Miller products, one per ComT entry
     int rc = gsi::reduce_chunks(ctx, sc, &Fr, nprob, &nchunk, 1, ne);

@@ -778,6 +778,16 @@ __global__ void k_rand_place_pi(const g2_jac* __restrict__ sums, size_t stride, 
   Y1[at + row] = o;
 }
 
+// ---- randomised per-proof verification (gs_verify_each_rand): proof p's c accumulators are A = p*c + j; the final
+// exponentiation multiplies chunk-major values F[j*nprob + p]
+__global__ void k_each_chunk_major(const fp12* __restrict__ M, fp12* __restrict__ F, size_t nprob, int c) {
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (id >= nprob * c) return;
+  const size_t p = id % nprob;
+  const int j = (int)(id / nprob);
+  F[id] = M[p * c + j];
+}
+
 }  // namespace gs
 
 
@@ -1501,6 +1511,216 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
   return GS_OK;
 }
 
+// ------------------------------------------------------------------ randomised per-proof verification: driver
+// The fold of verify_rand_dev stopped one step early: the four ComT entries of proof p are folded with ITS weights
+// (sigma_p, tau_p) and the call's beta, and nothing is multiplied across proofs.  Proof p is accepted iff
+//     FE( prod_k e( sigma_p X_k.0 + tau_p X_k.1 ,  beta Y_k.0 + Y_k.1 ) )  ==  t_p^tau_p   (PPE; 1 for the other types)
+// over the slots (X_k, Y_k) of the exact verifier.  A proof that fails the exact check has a non-zero 2 x 2 matrix E of
+// exponent errors and passes only if sigma beta E00 + sigma E01 + tau beta E10 + tau E11 = 0, a non-zero polynomial of
+// degree 2 in (sigma_p, tau_p, beta): probability <= 2^-62 over 63-bit weights, for every proof on its own (beta being
+// shared does not matter).  Preconditions as for the batch check.
+// Pairs of proof p, contiguous: X1 / Y1 [p*Kp + i], i < nf: the CRS slots (G2 side = one of the three folded CRS points,
+// lines walked once per call, Y1 left the identity), then the Kw walked slots, then identity padding.  Proof p takes the c
+// accumulators p*c .. p*c + c - 1 of S slots each (Kp = c S); c = 1 unless the proofs are few or large.
+static void each_split(size_t nprob, int Kp0, int* S_out, int* c_out) {
+  // as rand_slots_per_acc: waves of 9,472 accumulators x (62 squarings + 68 line steps per slot); at most M4_MAXS = 512
+  // slots per accumulator
+  int best_S = 0, best_c = 1;
+  double best_t = 1e300;
+  for (int c = 1; c <= Kp0; c++) {
+    const int S = ((Kp0 + c - 1) / c + 3) / 4 * 4;
+    if (S > 512) continue;
+    if (S < 8 && c > 1) break;
+    const size_t waves = (nprob * c + 9471) / 9472;
+    const double t = (double)waves * (62.0 * 53.0 + (double)S * 68.0 * 29.0);
+    if (t < best_t) {
+      best_t = t;
+      best_S = S;
+      best_c = c;
+    }
+  }
+  *S_out = best_S;
+  *c_out = best_c;
+}
+
+static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args,
+                                const uint64_t* rho_host, bool shared_x, uint8_t* out_ok_dev) {
+  verify_shape s = make_verify_shape(type, (int)m, (int)n);
+  const std::vector<uint8_t> kind_all = slot_kinds(s);
+  std::vector<int> slot_map(s.K), walk_slot;
+  gsi::acc_each each;
+  for (int k = 0; k < s.K; k++)
+    if (kind_all[k] >= gsi::GS_SLOT_FIXED) {
+      if (each.nf >= 4) FAIL(GS_EDIM, "verify_each_rand: too many CRS slots");
+      each.pid[each.nf] = kind_all[k] - gsi::GS_SLOT_FIXED;
+      slot_map[k] = each.nf++;
+    }
+  const int nf = each.nf;
+  for (int k = 0; k < s.K; k++)
+    if (kind_all[k] < gsi::GS_SLOT_FIXED) {
+      slot_map[k] = nf + (int)walk_slot.size();
+      walk_slot.push_back(k);
+    }
+  const int Kw = (int)walk_slot.size();
+  const jsf33 beta = make_jsf((uint32_t)rho_host[2 * count], (uint32_t)(rho_host[2 * count] >> 32));
+  // Passes as large as the line tiles allow (13,056 B per pair), equal in size.  Unlike verify_rand_dev the whole tile
+  // budget goes to the tiles: a per-proof pass has no bucket sums or product trees beside them, and 65,536 4x4 PPE proofs
+  // (12 pairs each) then run as one pass of 6.9 waves instead of two of 3.5 (4 + 4 waves of k_miller4).
+  int S, c;
+  each_split(count, nf + Kw, &S, &c);
+  if (S == 0) FAIL(GS_EDIM, "verify_each_rand: statement too large");
+  const int Kp = S * c;
+  size_t pass_cap = ctx->tile_budget / 13056 / (size_t)Kp;
+  if (pass_cap > 4 * ctx->verify_batch_max) pass_cap = 4 * ctx->verify_batch_max;
+  if (ctx->verify_batch_max < 23680) pass_cap = ctx->verify_batch_max;  // (lowered by a test: several passes on a small batch)
+  if (pass_cap < 1) FAIL(GS_EDIM, "verify_each_rand: one proof exceeds the tile budget");
+  const size_t npass = (count + pass_cap - 1) / pass_cap;
+  const size_t pass_n = (count + npass - 1) / npass;
+  if (pass_n * (size_t)Kp > ((size_t)1 << 30)) FAIL(GS_EDIM, "verify_each_rand: statement too large for one pass");
+  Scratch top(ctx);
+  g2_aff* Yfix;
+  int *dmap, *dwalk_slot, *dall, *drest;
+  CUDA_TRY(top.alloc(&Yfix, 3));
+  CUDA_TRY(upload(ctx, top, &dmap, slot_map.data(), slot_map.size()));
+  CUDA_TRY(upload(ctx, top, &dwalk_slot, walk_slot.data(), walk_slot.size()));
+  const bool fold_first = !shared_x || count == 1;
+  std::vector<int> all_slots, rest_slots;
+  for (int k = 0; k < s.K; k++) {
+    const bool msm_out = k < s.n || (k == s.sB && !s.groupB) || (type == 3 && k == s.sT);
+    const bool b_slot = s.groupB && k >= s.sB && k < s.sPi;
+    all_slots.push_back(k);
+    if (!msm_out && !b_slot) rest_slots.push_back(k);
+  }
+  CUDA_TRY(upload(ctx, top, &dall, all_slots.data(), all_slots.size()));
+  CUDA_TRY(upload(ctx, top, &drest, rest_slots.data(), rest_slots.size()));
+  // The folded CRS points, their lines and the target powers t_p^tau_p depend on nothing the main stream computes: they
+  // run on the second stream, next to the statement MSM and the folds.
+  if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
+  struct side_stream {  // (as in verify_rand_dev)
+    gs_ctx* ctx;
+    cudaStream_t main_s;
+    cudaEvent_t ev = nullptr;
+    bool pending = false;
+    int fork() {
+      if (!ev && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) return 1;
+      cudaEventRecord(ev, main_s);
+      cudaStreamWaitEvent(ctx->stream2, ev, 0);
+      ctx->stream = ctx->stream2;
+      return 0;
+    }
+    void back() {
+      cudaEventRecord(ev, ctx->stream2);
+      ctx->stream = main_s;
+      pending = true;
+    }
+    void join() {
+      if (pending) cudaStreamWaitEvent(main_s, ev, 0);
+      pending = false;
+    }
+    ~side_stream() {
+      ctx->stream = main_s;
+      join();
+      if (ev) cudaEventDestroy(ev);
+    }
+  } side{ctx, ctx->stream};
+  const bool two = !ctx->profile;  // (per-kernel event times need one stream)
+  fp2* crs_lines = nullptr;
+  if (nf) {
+    if (two && side.fork()) FAIL(GS_ECUDA, "verify_each_rand: event creation failed");
+    int rcl = [&]() -> int {
+      LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, Yfix);
+      return gsi::g2_lines(ctx, top, Yfix, 3, &crs_lines);
+    }();
+    if (two) side.back();
+    if (rcl) return rcl;
+  }
+  each.pts = Yfix;
+  each.acc_stride = c;
+  for (size_t off = 0; off < count; off += pass_n) {
+    const size_t nprob = count - off < pass_n ? count - off : pass_n;
+    Scratch sc(ctx);
+    struct join_on_exit {  // declared after `sc`, destroyed first (see verify_rand_dev)
+      side_stream& s;
+      ~join_on_exit() { s.join(); }
+    } joined{side};
+    const verify_args v = args_at(s, args, off);
+    g1_aff *X, *X1;
+    g2_aff *Y, *Y1;
+    uint64_t* drho;
+    fp12 *M, *want = nullptr;
+    {  // the low 63 bits of every weight (as verify_rand_dev)
+      std::vector<uint64_t> w(rho_host + 2 * off, rho_host + 2 * (off + nprob));
+      for (uint64_t& x : w) x &= 0x7fffffffffffffffull;
+      CUDA_TRY(upload(ctx, sc, &drho, w.data(), w.size()));
+    }
+    if (type == GS_PPE) {  // t_p^tau_p, on the side stream
+      CUDA_TRY(sc.alloc(&want, nprob));
+      if (two && side.fork()) FAIL(GS_ECUDA, "verify_each_rand: event creation failed");
+      int rcg = gsi::gt_pow64(ctx, (const fp12*)v.target, drho + 1, 2, nprob, want);
+      if (two) side.back();
+      if (rcg) return rcg;
+    }
+    const size_t Ktot = nprob * (size_t)Kp;
+    CUDA_TRY(sc.alloc(&X, 2 * (size_t)s.K * nprob));
+    CUDA_TRY(sc.alloc(&Y, 2 * (size_t)s.K * nprob));
+    CUDA_TRY(sc.alloc(&X1, Ktot));
+    CUDA_TRY(sc.alloc(&Y1, Ktot));
+    CUDA_TRY(sc.alloc(&M, nprob * (size_t)c));
+    CUDA_TRY(cudaMemsetAsync(X1, 0, Ktot * sizeof(g1_aff), ctx->stream));  // padding and the CRS pairs' G2 sides: identities
+    CUDA_TRY(cudaMemsetAsync(Y1, 0, Ktot * sizeof(g2_aff), ctx->stream));
+    LAUNCH(k_verify_assemble, nprob * (size_t)s.K, s, v, ctx->crs, X, Y, nprob);
+    if (fold_first) {  // as verify_rand_dev: commitments folded before the statement MSM
+      g1_aff *xfold, *afold;
+      CUDA_TRY(sc.alloc(&xfold, nprob * (size_t)s.nbases));
+      CUDA_TRY(sc.alloc(&afold, nprob * (size_t)(s.groupA ? s.n : 1)));
+      LAUNCH(k_rand_fold_bases, nprob * (size_t)(s.nbases + (s.groupA ? s.n : 0)), s, v, ctx->crs, nprob, drho, xfold, afold,
+             s.groupB ? slot_map[s.sB] : 0, Kp, X1);
+      verify_shape sf = s;
+      sf.na = 1;
+      verify_args vf = v;
+      vf.xfold = xfold;
+      vf.afold = afold;
+      vf.fold_map = dmap;
+      vf.fold_Kw = Kp;
+      vf.fold_X1 = X1;
+      const g1_jac* part;
+      int rcm = statement_msm_partials(ctx, sc, sf, vf, nprob, false, &part);
+      if (rcm) return rcm;
+      LAUNCH(k_vmsm_reduce, nprob * (size_t)sf.n_out_owned() * sf.na, sf, vf, part, (g1_aff*)nullptr, nprob);
+      LAUNCH(k_rand_fold_g1, nprob * rest_slots.size(), X, nprob, s.K, drho, drest, (int)rest_slots.size(), dmap, Kp, X1,
+             (g1_aff*)nullptr);
+    } else {  // one set of commitments under many equations: shared-base tables, every slot folded afterwards
+      const g1_jac* part;
+      int rcm = statement_msm_partials(ctx, sc, s, v, nprob, shared_x, &part);
+      if (rcm) return rcm;
+      LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
+      LAUNCH(k_rand_fold_g1, nprob * all_slots.size(), X, nprob, s.K, drho, dall, (int)all_slots.size(), dmap, Kp, X1,
+             (g1_aff*)nullptr);
+    }
+    LAUNCH(k_rand_fold_g2, nprob * (size_t)Kw, Y, nprob, s.K, beta, dwalk_slot, Kw, Y1 + nf, (size_t)Kp, (size_t)1);
+    side.join();  // the folded CRS points and their lines, this pass's target powers
+    each.F = M;
+    each.lines = crs_lines;
+    int rc = gsi::run_pairing_product(ctx, sc, X1, Y1, 1, (int)Ktot, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1, S, &each);
+    if (rc) return rc;
+    const fp12* Fr = M;
+    int nch = c;
+    if (c > 1) {
+      fp12* F;
+      CUDA_TRY(sc.alloc(&F, nprob * (size_t)c));
+      LAUNCH(k_each_chunk_major, nprob * (size_t)c, M, F, nprob, c);
+      Fr = F;
+      if (nch > 12) {
+        rc = gsi::reduce_chunks(ctx, sc, &Fr, nprob, &nch, 12, 1);
+        if (rc) return rc;
+      }
+    }
+    rc = gsi::launch_final_exp(ctx, Fr, nprob, nch, nullptr, out_ok_dev + off, want, 1);
+    if (rc) return rc;
+  }
+  return GS_OK;
+}
+
 int gs_verify_batch_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                          const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                          const gs_com1* theta, const uint64_t* rho, uint8_t* out_all_ok) {
@@ -1534,6 +1754,39 @@ int gs_verify_batch_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size
   if (int rc = check_lists(ctx, m, n, inputs_set(v) && rho)) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
   return verify_rand_dev(ctx, type, count, m, n, v, rho, false, out_all_ok_dev);
+}
+
+int gs_verify_each_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                        const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                        const gs_com1* theta, const uint64_t* rho, uint8_t* out_ok) {
+  const verify_args h = args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta);
+  if (int rc = check_call(ctx, type, 0, 1, true)) return rc;
+  if (count == 0) return GS_OK;
+  if (!out_ok) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(h) && rho)) return rc;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  Scratch sc(ctx);
+  verify_args d;
+  uint8_t* dok;
+  if (int rc = upload_args(ctx, sc, make_verify_shape(type, (int)m, (int)n), h, 0, count, &d)) return rc;
+  CUDA_TRY(sc.alloc(&dok, count));
+  int rc = verify_each_rand_dev(ctx, type, count, m, n, d, rho, same_rows(xcoms, count, m * sizeof(gs_com1)), dok);
+  if (rc) return rc;
+  CUDA_TRY(cudaMemcpyAsync(out_ok, dok, count, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  return GS_OK;
+}
+
+int gs_verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                            const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                            const gs_com1* theta, const uint64_t* rho, uint8_t* out_ok_dev) {
+  const verify_args v = args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta);
+  if (int rc = check_call(ctx, type, 0, 1, true)) return rc;
+  if (count == 0) return GS_OK;
+  if (!out_ok_dev) return GS_EARG;
+  if (int rc = check_lists(ctx, m, n, inputs_set(v) && rho)) return rc;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  return verify_each_rand_dev(ctx, type, count, m, n, v, rho, false, out_ok_dev);
 }
 
 }  // extern "C"

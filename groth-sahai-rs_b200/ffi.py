@@ -17,6 +17,7 @@ EXPORTED_SYMBOLS = [
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
     "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_verify_each_rand", "gs_verify_each_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
     "gs_com1_matmul", "gs_com2_matmul", "gs_fr_matmul",
@@ -80,6 +81,8 @@ def load_library():
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
         lib.gs_verify_batch_rand_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
+        lib.gs_verify_each_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
+        lib.gs_verify_each_rand_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
         lib.gs_verify_partial.argtypes = [vp, ci, sz, sz, sz] + [vp] * 8 + [ci, ci, vp]
         lib.gs_verify_partial_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 8 + [ci, ci, vp]
         lib.gs_verify_finish.argtypes = [vp, ci, sz, ci, vp, vp, vp]
@@ -358,6 +361,24 @@ class Engine:
         kr = _buf(self._rho(count, rho))
         self._chk(self.lib.gs_verify_batch_rand_dev(self.h, ty, count, m, n, *[ctypes.c_void_p(int(p)) for p in ptrs], kr[1],
                                                     ctypes.c_void_p(int(out_ok_ptr))))
+
+    # ---- randomised per-proof verification (gs_verify_each_rand): one verdict per proof, one final exponentiation each
+    def verify_each_rand(self, ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, rho=None) -> bytes:
+        """count verdict bytes: 1 iff proof p verifies (a bad proof passes with probability <= 2^-62 over rho, each on its
+        own).  Same weights and rho layout as verify_batch_rand; not bit-comparable with verify_batch."""
+        if count and m and n:
+            self._check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta)
+        kr = _buf(self._rho(count, rho))
+        ok = ctypes.create_string_buffer(max(1, count))
+        ks = [_buf(x) for x in (a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta)]
+        self._chk(self.lib.gs_verify_each_rand(self.h, ty, count, m, n, *[k[1] for k in ks], kr[1], ctypes.cast(ok, ctypes.c_void_p)))
+        return ok.raw[:count]
+
+    def verify_each_rand_dev(self, ty, count, m, n, ptrs, out_ok_ptr, rho=None):
+        """All-device variant (rho stays on the host); asynchronous on self.stream, count verdict bytes at out_ok_ptr."""
+        kr = _buf(self._rho(count, rho))
+        self._chk(self.lib.gs_verify_each_rand_dev(self.h, ty, count, m, n, *[ctypes.c_void_p(int(p)) for p in ptrs], kr[1],
+                                                   ctypes.c_void_p(int(out_ok_ptr))))
 
     # ---- one statement sharded by slot over several GPUs (gs_verify_partial / gs_verify_finish)
     def verify_partial(self, ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, rank, world) -> bytes:

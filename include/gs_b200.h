@@ -244,6 +244,27 @@ int gs_verify_batch_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size
                              const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const uint64_t* rho,
                              uint8_t* out_all_ok_dev);
 
+/* Randomised PER-PROOF verification, an opt-in like gs_verify_batch_rand: out_ok[p] = 1 iff proof p verifies, except
+ * with probability <= 2^-62 over `rho` for every bad proof on its own.  The four ComT entries of proof p are folded with
+ * the same weights as gs_verify_batch_rand (sigma_p, tau_p = low 63 bits of rho[2p], rho[2p+1]; beta = rho[2*count],
+ * shared by the call), and nothing is multiplied across proofs: proof p is accepted iff
+ *     FE( prod_k e( sigma_p X_k.0 + tau_p X_k.1 ,  beta Y_k.0 + Y_k.1 ) ) == t_p^tau_p   (PPE; 1 for the other types)
+ * over the slots (X_k, Y_k) of the exact verifier -- one Miller pair per slot and ONE final exponentiation per proof
+ * (csrc/verify.cu, "randomised per-proof verification").  A proof that fails the exact check passes only if a non-zero
+ * polynomial of degree 2 in (sigma_p, tau_p, beta) vanishes.  Preconditions, arrays and return codes as for
+ * gs_verify_batch_rand; count == 0 returns GS_OK and writes nothing; a null rho or output of a non-empty call is
+ * GS_EARG.  An all-zero rho accepts everything (the check is then vacuous).  The verdicts are not bit-comparable with the
+ * reference's.  The _dev variant takes device arrays (rho stays on the host) and writes `count` bytes of device memory,
+ * asynchronously on gs_stream(). */
+int gs_verify_each_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
+                        const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
+                        const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const uint64_t* rho,
+                        uint8_t* out_ok);
+int gs_verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
+                            const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
+                            const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const uint64_t* rho,
+                            uint8_t* out_ok_dev);
+
 /* ---- ComT (src/data_structures.rs) ------------------------------------------------------- */
 /* ComT::pairing :484-491, batched: out[i] = F(xs[i], ys[i]) (4 full pairings each) */
 int gs_comt_pairing(gs_ctx* ctx, size_t count, const gs_com1* xs, const gs_com2* ys, gs_comt* out);

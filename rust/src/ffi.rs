@@ -71,6 +71,10 @@ extern "C" {
     pub fn gs_verify_batch_rand(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                                 gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,
                                 pi: *const GsCom2, theta: *const GsCom1, rho: *const u64, out_all_ok: *mut u8) -> i32;
+    // opt-in, not in the reference: ONE randomised verdict PER PROOF (same rho layout; one final exponentiation each)
+    pub fn gs_verify_each_rand(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
+                               gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,
+                               pi: *const GsCom2, theta: *const GsCom1, rho: *const u64, out_ok: *mut u8) -> i32;
     pub fn gs_verify_partial(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                              gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,
                              pi: *const GsCom2, theta: *const GsCom1, rank: i32, world: i32, out_partial: *mut GsGt) -> i32;

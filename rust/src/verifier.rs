@@ -84,3 +84,29 @@ pub fn verify_batch_ppe<E: Gpu>(equations: &[PPE<E>], proofs: &[CProof<E>], crs:
     }));
     ok.into_iter().map(|x| x == 1).collect()
 }
+
+/// Not in the reference: per-proof verdicts of `count` independent PPE (equation, proof) pairs of one shape at close to
+/// the randomised cost (gs_verify_each_rand): each proof's four ComT entries are folded with its own weights from `rng`
+/// (a cryptographic RNG the prover cannot predict) into one pairing product and ONE final exponentiation.  A bad proof is
+/// accepted with probability <= 2^-62, each proof on its own.
+pub fn verify_each_ppe_rand<E: Gpu>(equations: &[PPE<E>], proofs: &[CProof<E>], crs: &CRS<E>,
+                                    rng: &mut dyn ark_std::rand::RngCore) -> Vec<bool> {
+    assert_eq!(equations.len(), proofs.len());
+    if equations.is_empty() { return vec![]; }
+    let (m, n) = (proofs[0].xcoms.coms.len(), proofs[0].ycoms.coms.len());
+    let (mut a, mut b, mut g, mut t) = (Vec::new(), Vec::new(), Vec::new(), Vec::new());
+    let (mut xc, mut yc, mut pi, mut th) = (Vec::new(), Vec::new(), Vec::new(), Vec::new());
+    for (e, p) in equations.iter().zip(proofs) {
+        assert_eq!((p.xcoms.coms.len(), p.ycoms.coms.len(), p.equ_proofs.len()), (m, n, 1));
+        a.extend(g1s::<E>(&e.a_consts)); b.extend(g2s::<E>(&e.b_consts)); g.extend(fr_matrix::<E>(&e.gamma)); t.push(E::gt(&e.target));
+        xc.extend(com1s(&p.xcoms.coms)); yc.extend(com2s(&p.ycoms.coms));
+        pi.extend(com2s(&p.equ_proofs[0].pi)); th.extend(com1s(&p.equ_proofs[0].theta));
+    }
+    let rho: Vec<u64> = (0..2 * equations.len() + 1).map(|_| rng.next_u64()).collect();
+    let mut ok = vec![0u8; equations.len()];
+    with_crs(&crs.abi(), |c| check(c, unsafe {
+        gs_verify_each_rand(c.raw(), 0, ok.len(), m, n, bytes_of(&a).as_ptr(), bytes_of(&b).as_ptr(), g.as_ptr(),
+                            bytes_of(&t).as_ptr(), xc.as_ptr(), yc.as_ptr(), pi.as_ptr(), th.as_ptr(), rho.as_ptr(), ok.as_mut_ptr())
+    }));
+    ok.into_iter().map(|x| x == 1).collect()
+}
