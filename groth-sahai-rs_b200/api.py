@@ -68,6 +68,24 @@ class ExtractionKey:
 
 
 @dataclass
+class SimulationKey:
+    """The trapdoor of a hiding CRS: t1, t2 of generate_hiding_crs (Fr bytes), with W1 = u[1] + iota_1(g1) = t1 u[0] and
+    W2 = t2 v[0].  Whoever holds it makes accepting proofs of any MSMEG1, MSMEG2, Quad or target-1 PPE statement under
+    that CRS without witnesses (simulate_batch, _Equation.simulate)."""
+    t1: bytes
+    t2: bytes
+
+    def to_bytes(self) -> bytes:
+        return self.t1 + self.t2
+
+    @staticmethod
+    def from_bytes(b: bytes) -> "SimulationKey":
+        if len(b) != 2 * FR:
+            raise ValueError(f"SimulationKey: {len(b)} bytes, expected {2 * FR}")
+        return SimulationKey(b[:FR], b[FR:])
+
+
+@dataclass
 class CRS:
     u: List[bytes]       # 2 x Com1
     v: List[bytes]       # 2 x Com2
@@ -85,10 +103,16 @@ class CRS:
     def generate_crs_with_trapdoor(rng, engine: Engine = None) -> "Tuple[CRS, ExtractionKey]":
         """generate_crs that also returns the binding key's trapdoor (a1, a2) instead of dropping it (not in the reference;
         ExtGen of Groth & Sahai, EUROCRYPT 2008).  Exactly generate_crs's draws: the same rng state gives the same CRS."""
+        crs, (a1, a2, _, _) = CRS._generate(rng, engine)
+        return crs, ExtractionKey(a1, a2)
+
+    @staticmethod
+    def _generate(rng, engine):
+        """The binding key of generator.rs:81-118 and its four Fr draws (a1, a2, t1, t2), drawn in its order."""
         eng = engine or default_engine()
         p1, p2 = rng.g1(), rng.g2()
-        a1, a2, t1, t2 = rng.fr(), rng.fr(), rng.fr(), rng.fr()
-        return CRS.from_bytes(eng.crs_generate(p1, p2, a1, a2, t1, t2), eng, loaded=True), ExtractionKey(a1, a2)
+        s = [rng.fr() for _ in range(4)]
+        return CRS.from_bytes(eng.crs_generate(p1, p2, *s), eng, loaded=True), s
 
     @staticmethod
     def generate_hiding_crs(rng, engine: Engine = None) -> "CRS":
@@ -96,10 +120,16 @@ class CRS:
         offered here because it is what a zero-knowledge simulator needs (SURVEY.md §8f.4).  Same RNG draws as
         generate_crs; the only difference is the last entry of each key: u[1].1 = t1*q1 - g1, v[1].1 = t2*q2 - g2,
         i.e. u[1] - iota_1(g1) and v[1] - iota_2(g2) on the device (gs_com1_sub / gs_com2_sub)."""
-        crs = CRS.generate_crs(rng, engine)
+        return CRS.generate_hiding_crs_with_trapdoor(rng, engine)[0]
+
+    @staticmethod
+    def generate_hiding_crs_with_trapdoor(rng, engine: Engine = None) -> "Tuple[CRS, SimulationKey]":
+        """generate_hiding_crs that also returns its trapdoor (t1, t2), the simulation key of Groth & Sahai (EUROCRYPT
+        2008; not in the reference).  Exactly generate_hiding_crs's draws: the same rng state gives the same CRS."""
+        crs, (_, _, t1, t2) = CRS._generate(rng, engine)
         u1 = Com1.sub(crs.u[1], Com1.linear_map(crs.g1_gen), crs.engine)
         v1 = Com2.sub(crs.v[1], Com2.linear_map(crs.g2_gen), crs.engine)
-        return CRS.from_bytes(crs.u[0] + u1 + crs.v[0] + v1 + crs.g1_gen + crs.g2_gen + crs.gt_gen, crs.engine)
+        return CRS.from_bytes(crs.u[0] + u1 + crs.v[0] + v1 + crs.g1_gen + crs.g2_gen + crs.gt_gen, crs.engine), SimulationKey(t1, t2)
 
     def to_bytes(self) -> bytes:
         return b"".join(self.u) + b"".join(self.v) + self.g1_gen + self.g2_gen + self.gt_gen
@@ -229,6 +259,11 @@ class _Equation:
         (not in the reference; see rerandomize_batch).  RNG order: R' rows, S' rows, then T', row-major."""
         return rerandomize_batch([self], [com_proof], crs, rng)[0]
 
+    def simulate(self, crs: CRS, key: SimulationKey, rng) -> CProof:
+        """An accepting CProof of this equation without witnesses, made with the hiding CRS's trapdoor (not in the
+        reference; see simulate_batch).  RNG order: R rows, S rows, then T, row-major, as commit_and_prove."""
+        return simulate_batch([self], crs, key, rng)[0]
+
     def verify(self, com_proof: CProof, crs: CRS) -> bool:              # verifier.rs:23-157
         assert len(com_proof.equ_proofs) == 1
         ep = com_proof.equ_proofs[0]
@@ -318,6 +353,51 @@ def rerandomize_batch(equations, proofs, crs: CRS, rng, shared_commitments: bool
         cat(lambda p: b"".join(p.ycoms.coms), coms), cat(lambda p: b"".join(p.equ_proofs[0].pi), proofs),
         cat(lambda p: b"".join(p.equ_proofs[0].theta), proofs), cat(_flat, Rs), cat(_flat, Ss), cat(_flat, Ts),
         shared_coms=shared_commitments)
+    xcs, ycs = _split(xc, 192 * m), _split(yc, 384 * n)
+    pis, ths = _split(pi, 384 * cx), _split(th, 192 * cy)
+    out = []
+    for k in range(len(equations)):
+        j = 0 if shared_commitments else k
+        out.append(CProof(Commit1(_split(xcs[j], 192), []), Commit2(_split(ycs[j], 384), []),
+                          [EquProof(_split(pis[k], 384), _split(ths[k], 192), ty, [])]))
+    return out
+
+
+def simulate_batch(equations, crs: CRS, key: SimulationKey, rng, shared_commitments: bool = False) -> List[CProof]:
+    """Zero-knowledge simulation (Groth & Sahai, EUROCRYPT 2008; not in the reference): for every equation a CProof that
+    verifies under the hiding CRS `crs` without any witness, made with its trapdoor `key` in one GPU pass
+    (gs_simulate_batch).  The commitments are of O / 0 and the target is absorbed through t1 / t2, so MSMEG1, MSMEG2 and
+    Quad statements need not be satisfiable; PPE targets must be 1.  Simulated proofs are distributed exactly like real
+    ones.  One type and one shape (m x n, from Gamma) per batch.
+
+    Randomness is drawn per equation in commit_and_prove's order: R (m x cx) rows, then S (n x cy) rows, then T (cy x cx),
+    row-major.  With shared_commitments R and S are drawn once, then T equation by equation, and the returned CProofs share
+    one set of commitments.  The returned Commit*.rand and EquProof.rand are empty, as for rerandomize_batch.  A key that
+    does not belong to `crs` (any key of a binding CRS) or a PPE target other than 1 raises GsError."""
+    assert equations
+    ty = equations[0].equ_type
+    m, n = len(equations[0].gamma), len(equations[0].gamma[0]) if equations[0].gamma else 0
+    for e in equations:
+        if e.equ_type != ty or len(e.gamma) != m or any(len(r) != n for r in e.gamma):
+            raise ValueError("simulate_batch: every equation must have the same type and shape")
+        if len(e.a_consts) != n or len(e.b_consts) != m:
+            raise ValueError("simulate_batch: constants / Gamma do not match the number of variables")
+    cx, cy = equations[0]._cx(), equations[0]._cy()
+    draw = lambda rows, cols: [[rng.fr() for _ in range(cols)] for _ in range(rows)]
+    if shared_commitments:
+        R, S = draw(m, cx), draw(n, cy)
+        Rs, Ss, Ts = [R], [S], [draw(cy, cx) for _ in equations]
+    else:
+        Rs, Ss, Ts = [], [], []
+        for _ in equations:
+            Rs.append(draw(m, cx))
+            Ss.append(draw(n, cy))
+            Ts.append(draw(cy, cx))
+    cat = lambda f, items: b"".join(f(x) for x in items)
+    xc, yc, pi, th = crs._use().simulate_batch(
+        ty, len(equations), m, n, cat(lambda e: b"".join(e.a_consts), equations), cat(lambda e: b"".join(e.b_consts), equations),
+        cat(lambda e: _flat(e.gamma), equations), cat(lambda e: e.target, equations), cat(_flat, Rs), cat(_flat, Ss),
+        cat(_flat, Ts), key.to_bytes(), shared_coms=shared_commitments)
     xcs, ycs = _split(xc, 192 * m), _split(yc, 384 * n)
     pis, ths = _split(pi, 384 * cx), _split(th, 192 * cy)
     out = []

@@ -166,6 +166,7 @@ extern "C" int gs_diag_fpmul_rate(gs_ctx* ctx, double* fpmul_per_sec) {
 
 static int load_crs_device(gs_ctx* ctx, const gs_crs* crs) {
   ctx->xkey_valid = ctx->ykey_valid = false;  // gs_extract checked its cached keys against the previous CRS
+  ctx->tkey_valid = false;                      // gs_simulate likewise
   crs_dev h;
   memset(&h, 0, sizeof(h));
   for (int k = 0; k < 2; k++)

@@ -30,6 +30,8 @@ struct gs_ctx {
   bool crs_loaded = false;
   bool xkey_valid = false, ykey_valid = false;  // gs_extract: the last key of each side that matched the loaded CRS
   gs_fr xkey{}, ykey{};                         // (cleared by gs_crs_load / gs_crs_generate)
+  bool tkey_valid = false;  // gs_simulate: the last simulation key (t1, t2) that matched the loaded CRS (cleared likewise)
+  gs_fr tkey[2]{};
   gs_fixed_table<gs::FpOps> tab1;
   gs_fixed_table<gs::Fp2Ops> tab2;
   bool crs_lines_valid = false;   // the stored lines and the fixed-base tables are built by the FIRST call that needs them
@@ -182,6 +184,20 @@ static inline size_t elem_size_T(int type) {
   return type == 0 ? sizeof(gs::fp12) : type == 1 ? sizeof(gs::g1_aff) : type == 2 ? sizeof(gs::g2_aff) : sizeof(gs::fr);
 }
 
+namespace gs {
+// prover.cu: the Fr algebra of the prover, batched over blockIdx.y = proof instance (`*_bs` = elements between instances, 0: shared);
+// `lanes` = 1 (one thread per output) or 32 (one warp per output, fr_lanes)
+__global__ void k_fr_matmul(fr* __restrict__ out, const fr* __restrict__ A, size_t a_rs, size_t a_cs, const fr* __restrict__ B,
+                            size_t b_rs, size_t b_cs, size_t r, size_t k, size_t c, size_t a_bs, size_t b_bs, int lanes);
+__global__ void k_coef_pi(fr* __restrict__ out, const fr* __restrict__ RG, const fr* __restrict__ S, const fr* __restrict__ T, int cx,
+                          int cy, size_t n, size_t s_bs, int lanes);
+__global__ void k_concat_scalars(fr* __restrict__ sv, const fr* __restrict__ R, const fr* __restrict__ RG, int cx, size_t m, size_t n,
+                                 size_t r_bs);
+__global__ void k_fr_dot(fr* __restrict__ out, const fr* __restrict__ sv, const fr* __restrict__ w0, size_t m, const fr* __restrict__ w1,
+                         size_t n, int rows, size_t w1_bs, int lanes);
+static inline int fr_lanes(size_t k, size_t outputs) { return (k >= 128 && outputs * 32 <= ((size_t)1 << 24)) ? 32 : 1; }
+}  // namespace gs
+
 // ---- functions that cross translation units (namespace gsi = "internal") ----
 namespace gsi {
 using namespace gs;
@@ -282,5 +298,40 @@ int rerand_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_
                    const fr* coef, const fr* e, const Aff<F>* dold, Aff<F>* dout);
 template <class F>
 int com_matmul_impl(gs_ctx* ctx, size_t r, size_t k, size_t c, const gs_fr* lhs, const void* mat, void* out);
+
+// theta (G1, `theta()`) and pi (G2, `pi()`) of a batch of proofs are independent: in the latency regime (`two_streams`: few
+// products) theta runs on the second stream next to pi.  Returns theta's error code, else pi's.
+template <class Theta, class Pi>
+int theta_pi_fork(gs_ctx* ctx, bool two_streams, const char* what, Theta&& theta, Pi&& pi) {
+  cudaStream_t main_stream = ctx->stream;
+  cudaEvent_t fork = nullptr, join = nullptr;
+  if (two_streams) {
+    if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
+    CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
+    if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
+      cudaEventDestroy(fork);
+      FAIL(GS_ECUDA, std::string(what) + ": event creation failed");
+    }
+    cudaEventRecord(fork, main_stream);
+    cudaStreamWaitEvent(ctx->stream2, fork, 0);
+    ctx->stream = ctx->stream2;
+  }
+  int rc_th = theta();
+  if (two_streams) {
+    cudaEventRecord(join, ctx->stream2);
+    ctx->stream = main_stream;
+  }
+  int rc_pi = pi();
+  if (two_streams) {
+    cudaStreamWaitEvent(main_stream, join, 0);  // also orders the scratch frees (main stream) after theta's kernels
+    cudaEventDestroy(fork);
+    cudaEventDestroy(join);
+  }
+  return rc_th ? rc_th : rc_pi;
+}
+
+// extract.cu: *all_identity = (coms[i].1 - key coms[i].0 is the identity for every i < n), n DEVICE commitments (k_extract)
+template <class F>
+int extract_all_identity(gs_ctx* ctx, const Aff<F>* coms, size_t n, const gs_fr* key, bool* all_identity);
 
 }  // namespace gsi

@@ -68,20 +68,33 @@ static extract_digits digits_of(const gs_fr* key) {
   return make_extract_digits<F>(c);
 }
 
+// *all_identity = (coms[i].1 - key coms[i].0 is the identity for every i < n), n device commitments
+template <class F>
+int extract_all_identity(gs_ctx* ctx, const Aff<F>* coms, size_t n, const gs_fr* key, bool* all_identity) {
+  Scratch sc(ctx);
+  Aff<F>* dout;
+  CUDA_TRY(sc.alloc(&dout, n));
+  LAUNCH_CFG((k_extract<F>), n, GS_EXT_NT, 0, coms, dout, n, digits_of<F>(key));
+  std::vector<Aff<F>> h(n);
+  CUDA_TRY(cudaMemcpyAsync(h.data(), dout, n * sizeof(Aff<F>), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  *all_identity = true;
+  for (const Aff<F>& p : h) *all_identity = *all_identity && p.is_inf();
+  return GS_OK;
+}
+template int extract_all_identity<FpOps>(gs_ctx*, const g1_aff*, size_t, const gs_fr*, bool*);
+template int extract_all_identity<Fp2Ops>(gs_ctx*, const g2_aff*, size_t, const gs_fr*, bool*);
+
 // The key matches the loaded CRS iff extracting the two key commitments u[0], u[1] (v[0], v[1]) gives the identity
 // twice.  Under the hiding key u[1] - iota_1(g1) extracts to -g1, so that key fails as well.  A validated key is
 // cached until the next gs_crs_load / gs_crs_generate.
 template <class F>
-static int key_check(gs_ctx* ctx, const gs_fr* key, const extract_digits& dg) {
+static int key_check(gs_ctx* ctx, const gs_fr* key) {
   if (ext_side<F>::valid(ctx) && memcmp(&ext_side<F>::cached(ctx), key, sizeof(gs_fr)) == 0) return GS_OK;
-  Scratch sc(ctx);
-  Aff<F>* dout;
-  CUDA_TRY(sc.alloc(&dout, 2));
-  LAUNCH_CFG((k_extract<F>), 2, GS_EXT_NT, 0, ext_side<F>::key(ctx->crs), dout, (size_t)2, dg);
-  Aff<F> h[2];
-  CUDA_TRY(cudaMemcpyAsync(h, dout, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  if (!h[0].is_inf() || !h[1].is_inf()) FAIL(GS_EARG, ext_side<F>::bad_key);
+  bool ok;
+  int rc = extract_all_identity<F>(ctx, ext_side<F>::key(ctx->crs), 2, key, &ok);
+  if (rc) return rc;
+  if (!ok) FAIL(GS_EARG, ext_side<F>::bad_key);
   ext_side<F>::cached(ctx) = *key;
   ext_side<F>::valid(ctx) = true;
   return GS_OK;
@@ -163,11 +176,11 @@ int gs_extract(gs_ctx* ctx, size_t nx, const gs_com1* xcoms, const gs_fr* xkey, 
   int rc;
   if (nx) {
     dx = digits_of<FpOps>(xkey);
-    if ((rc = key_check<FpOps>(ctx, xkey, dx))) return rc;
+    if ((rc = key_check<FpOps>(ctx, xkey))) return rc;
   }
   if (ny) {
     dy = digits_of<Fp2Ops>(ykey);
-    if ((rc = key_check<Fp2Ops>(ctx, ykey, dy))) return rc;
+    if ((rc = key_check<Fp2Ops>(ctx, ykey))) return rc;
   }
   if (nx && (rc = extract_side<FpOps>(ctx, nx, (const g1_aff*)xcoms, dx, (g1_aff*)out_x))) return rc;
   if (ny && (rc = extract_side<Fp2Ops>(ctx, ny, (const g2_aff*)ycoms, dy, (g2_aff*)out_y))) return rc;

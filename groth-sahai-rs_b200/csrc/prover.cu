@@ -111,7 +111,6 @@ __device__ GS_INL void fr_warp_sum(fr& acc) {
     fr::add(acc, acc, o);
   }
 }
-static inline int fr_lanes(size_t k, size_t outputs) { return (k >= 128 && outputs * 32 <= ((size_t)1 << 24)) ? 32 : 1; }
 
 // out (r x c) = A (r x k) * B (k x c), row-major; optional transposes via strides.
 // Every prover kernel is batched over blockIdx.y = proof instance; `*_bs` = elements between instances (0: shared).
@@ -339,35 +338,15 @@ static int prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, c
       const int l_d = fr_lanes(m + n, (size_t)cy * nb);
       LAUNCH_B(k_fr_dot, (size_t)cy * l_d, nb, e_th, sv_th, (const fr*)dA, n, (const fr*)dX, m, cy, shared_vars ? (size_t)0 : m, l_d);
     }
-    // pi (G2) and theta (G1) are independent: in the latency regime (few proofs) theta runs on the second stream next to pi
-    const bool two_streams = nb * (m + n) * 2 < 32768;
-    cudaStream_t main_stream = ctx->stream;
-    cudaEvent_t fork = nullptr, join = nullptr;
-    if (two_streams) {
-      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-      if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
-        cudaEventDestroy(fork);
-        FAIL(GS_ECUDA, "prove: event creation failed");
-      }
-      cudaEventRecord(fork, main_stream);
-      cudaStreamWaitEvent(ctx->stream2, fork, 0);
-      ctx->stream = ctx->stream2;
-    }
     // theta_i = sum_j S[j][i] iota(A_j) + sum_k SG[i][k] iota(X_k) + sum_l T[i][l] u_l          (l < cx)
-    int rc_th = proof_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, dA, n, dX, m, shared_vars, cx, dT, (size_t)cx, e_th, dth);
-    if (two_streams) {
-      cudaEventRecord(join, ctx->stream2);
-      ctx->stream = main_stream;
-    }
-    int rc_pi = proof_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, dB, m, dY, n, shared_vars, cy, coef_pi, (size_t)cy, e_pi, dpi);
-    if (two_streams) {
-      cudaStreamWaitEvent(main_stream, join, 0);  // also orders the scratch frees (main stream) after theta's kernels
-      cudaEventDestroy(fork);
-      cudaEventDestroy(join);
-    }
-    if (rc_th) return rc_th;
-    if (rc_pi) return rc_pi;
+    // theta on the second stream next to pi in the latency regime (few proofs)
+    int rc = theta_pi_fork(
+        ctx, nb * (m + n) * 2 < 32768, "prove",
+        [&] { return proof_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, dA, n, dX, m, shared_vars, cx, dT, (size_t)cx, e_th, dth); },
+        [&] {
+          return proof_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, dB, m, dY, n, shared_vars, cy, coef_pi, (size_t)cy, e_pi, dpi);
+        });
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(out_pi + off * cx, dpi, nb * 2 * cx * sizeof(g2_aff), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaMemcpyAsync(out_theta + off * cy, dth, nb * 2 * cy * sizeof(g1_aff), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
@@ -481,33 +460,11 @@ static int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_
     CUDA_TRY(sc.alloc(&dpo, nb * 2 * cx));
     CUDA_TRY(sc.alloc(&dto, nb * 2 * cy));
     // theta' on the second stream next to pi' in the latency regime, as in prove_impl
-    const bool two_streams = nb * (m + n) * 2 < 32768;
-    cudaStream_t main_stream = ctx->stream;
-    cudaEvent_t fork = nullptr, join = nullptr;
-    if (two_streams) {
-      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-      if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
-        cudaEventDestroy(fork);
-        FAIL(GS_ECUDA, "rerandomize: event creation failed");
-      }
-      cudaEventRecord(fork, main_stream);
-      cudaStreamWaitEvent(ctx->stream2, fork, 0);
-      ctx->stream = ctx->stream2;
-    }
-    int rc_th = rerand_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, SG, dA, n, dXc, m, shared, cx, dT, e_th, dTh, dto);
-    if (two_streams) {
-      cudaEventRecord(join, ctx->stream2);
-      ctx->stream = main_stream;
-    }
-    int rc_pi = rerand_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, RG, dB, m, dYc, n, shared, cy, coef_pi, e_pi, dPi, dpo);
-    if (two_streams) {
-      cudaStreamWaitEvent(main_stream, join, 0);  // also orders the scratch frees (main stream) after theta's kernels
-      cudaEventDestroy(fork);
-      cudaEventDestroy(join);
-    }
-    if (rc_th) return rc_th;
-    if (rc_pi) return rc_pi;
+    int rc = theta_pi_fork(
+        ctx, nb * (m + n) * 2 < 32768, "rerandomize",
+        [&] { return rerand_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, SG, dA, n, dXc, m, shared, cx, dT, e_th, dTh, dto); },
+        [&] { return rerand_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, RG, dB, m, dYc, n, shared, cy, coef_pi, e_pi, dPi, dpo); });
+    if (rc) return rc;
     if (do_coms) {
       CUDA_TRY(cudaMemcpyAsync(out_xcoms + voff * m, dXo, nv * m * 2 * sizeof(g1_aff), cudaMemcpyDeviceToHost, ctx->stream));
       CUDA_TRY(cudaMemcpyAsync(out_ycoms + voff * n, dYo, nv * n * 2 * sizeof(g2_aff), cudaMemcpyDeviceToHost, ctx->stream));

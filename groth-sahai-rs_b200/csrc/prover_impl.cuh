@@ -723,8 +723,9 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
     // few terms (a lone statement): split every scalar multiplication over PARTS threads to shorten the serial chain;
     // big batches are throughput-bound and keep one thread per term (measured on C4: the split costs ~5 % there)
     // many equations over one witness set: the variable terms come from shared-base window tables (break-even ~20 uses
-    // of a base; required here: 64) and every thread takes a whole scalar
-    const bool var_tables = vars_shared && nvars > 0 && count * rows >= 64;
+    // of a base; required here: 64) and every thread takes a whole scalar.  A simulated proof (simulate.cu) has no
+    // variable terms (nvars = 0) and takes this branch for the shared scalar vector of its constant terms alone.
+    const bool var_tables = vars_shared && count * rows >= 64;
     // ONE big statement: bucket MSM (pippenger.cuh) from ctx->pip_min terms up -- W * N additions per row instead of a
     // windowed scalar multiplication per term
     if (count == 1 && !var_tables && nt >= ctx->pip_min) {
@@ -757,6 +758,7 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
       cudaStream_t main_stream = ctx->stream;
       ctx->stream = ctx->stream2;
       int rct = [&]() -> int {
+        if (nvars == 0) return GS_OK;
         int rcb = shared_base_tables<F>(ctx, (const Aff<F>*)dvars, nvars, ptab, J);
         if (rcb) return rcb;
         LAUNCH_B((k_msm_var_terms_tab<F>), nvars * rows, count, terms, sv, ptab, nconst, nvars, rows);

@@ -16,7 +16,7 @@ EXPORTED_SYMBOLS = [
     "gs_profile_enable", "gs_profile_read", "gs_diag_fpmul_rate",
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
-    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_simulate", "gs_simulate_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_each_rand", "gs_verify_each_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
@@ -77,6 +77,8 @@ def load_library():
         lib.gs_rerandomize.argtypes = [vp, ci, sz, sz] + [vp] * 14
         lib.gs_rerandomize_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10 + [ci] + [vp] * 4
         lib.gs_extract.argtypes = [vp, sz, vp, vp, sz, vp, vp, vp, vp]
+        lib.gs_simulate.argtypes = [vp, ci, sz, sz] + [vp] * 12
+        lib.gs_simulate_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 7 + [ci] + [vp] * 5
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
@@ -302,6 +304,38 @@ class Engine:
         self._chk(self.lib.gs_extract(self.h, nx, ks[0][1], ks[1][1], ny, ks[2][1], ks[3][1], ctypes.cast(ox, ctypes.c_void_p),
                                       ctypes.cast(oy, ctypes.c_void_p)))
         return ox.raw[: nx * G1], oy.raw[: ny * G2]
+
+    # ---- zero-knowledge simulation with the hiding key (gs_simulate_batch)
+    def simulate_batch(self, ty, count, m, n, a_consts, b_consts, gamma, target, x_rand, y_rand, pf_rand, tkey, shared_coms=False):
+        """`count` simulated proofs in one pass with the hiding key's trapdoor tkey = t1 || t2 (Fr bytes): commitments of
+        O / 0 under R = x_rand, S = y_rand and proofs under T = pf_rand that verify against `target` (PPE: only target 1).
+        Returns (xcoms, ycoms, pi, theta) bytes, proof-major; with shared_coms R, S and the commitments are one set."""
+        cx, cy = _cx(ty), _cy(ty)
+        reps = 1 if shared_coms else count
+        if count and m and n:
+            assert len(a_consts) == count * n * _a_size(ty) and len(b_consts) == count * m * _b_size(ty)
+            assert len(gamma) == count * m * n * FR and len(target) == count * _t_size(ty) and len(pf_rand) == count * cx * cy * FR
+            assert len(x_rand) == reps * m * cx * FR and len(y_rand) == reps * n * cy * FR and len(tkey) == 2 * FR
+        outs = [ctypes.create_string_buffer(max(1, k)) for k in
+                (reps * m * COM1, reps * n * COM2, count * cx * COM2, count * cy * COM1)]
+        ks = [_buf(x) for x in (a_consts, b_consts, gamma, target, x_rand, y_rand, pf_rand)]
+        kt = _buf(tkey)
+        self._chk(self.lib.gs_simulate_batch(self.h, ty, count, m, n, *[k[1] for k in ks], 1 if shared_coms else 0, kt[1],
+                                             *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
+        return (outs[0].raw[: reps * m * COM1], outs[1].raw[: reps * n * COM2], outs[2].raw[: count * cx * COM2],
+                outs[3].raw[: count * cy * COM1])
+
+    def simulate(self, ty, m, n, a_consts, b_consts, gamma, target, x_rand, y_rand, pf_rand, tkey):
+        """One simulated proof (gs_simulate); returns (xcoms, ycoms, pi, theta) bytes."""
+        cx, cy = _cx(ty), _cy(ty)
+        if m and n:
+            assert len(a_consts) == n * _a_size(ty) and len(b_consts) == m * _b_size(ty) and len(gamma) == m * n * FR
+            assert len(target) == _t_size(ty) and len(tkey) == 2 * FR
+            assert len(x_rand) == m * cx * FR and len(y_rand) == n * cy * FR and len(pf_rand) == cx * cy * FR
+        outs = [ctypes.create_string_buffer(max(1, k)) for k in (m * COM1, n * COM2, cx * COM2, cy * COM1)]
+        ks = [_buf(x) for x in (a_consts, b_consts, gamma, target, x_rand, y_rand, pf_rand, tkey)]
+        self._chk(self.lib.gs_simulate(self.h, ty, m, n, *[k[1] for k in ks], *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
+        return outs[0].raw[: m * COM1], outs[1].raw[: n * COM2], outs[2].raw[: cx * COM2], outs[3].raw[: cy * COM1]
 
     @staticmethod
     def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, gamma_rows=None):

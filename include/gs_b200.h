@@ -166,6 +166,29 @@ int gs_rerandomize_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n
 int gs_extract(gs_ctx* ctx, size_t nx, const gs_com1* xcoms, const gs_fr* xkey, size_t ny, const gs_com2* ycoms,
                const gs_fr* ykey, gs_g1* out_x, gs_g2* out_y);
 
+/* ---- zero-knowledge simulation with the hiding key (not in the reference) ------------------------ */
+/* Makes accepting proofs WITHOUT witnesses with the hiding key's trapdoor (Groth & Sahai, EUROCRYPT 2008; PAPERS.md).
+ * Whoever holds tkey = (t1, t2) of a hiding CRS can make proofs that verify under that CRS for ANY MSMEG1, MSMEG2 or Quad
+ * statement and any PPE statement with target 1, true or not; they are distributed exactly like real proofs.  Under the
+ * hiding key W1 = u[1] + iota_1(g1) = t1 u[0] and W2 = t2 v[0].  With R = x_rand (m x cx), S = y_rand (n x cy) and
+ * T = pf_rand (cy x cx), drawn as for commit + prove:
+ *   c = R u_x                         d = S v_y                     (commitments of O / 0)
+ *   pi    = R^T iota_y(B) + (R^T Gamma S - T^T) v_y  [- t1 iota_2(T2)   MSMEG2]
+ *   theta = S^T iota_x(A) + T u_x                    [- t2 iota_1(T1)   MSMEG1;   - t t2 W1   Quad]
+ * i.e. the prover with every witness O / 0 and the target absorbed through the trapdoor.  Arrays as gs_rerandomize_batch
+ * (target[count] as gs_verify_batch); with shared_coms != 0, x_rand, y_rand, out_xcoms and out_ycoms are ONE set for every
+ * equation.  Return codes as gs_prove_batch, and GS_EARG, with nothing written, when tkey is not the loaded CRS's
+ * simulation key (every binding CRS fails), for a PPE target other than 1, without a loaded CRS, or for a null pointer.
+ * count == 0 returns GS_OK.  gs_simulate is the batch of one. */
+int gs_simulate(gs_ctx* ctx, int type, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                const gs_fr* gamma, const void* target, const gs_fr* x_rand, const gs_fr* y_rand,
+                const gs_fr* pf_rand, const gs_fr* tkey /* [2] = t1, t2 */, gs_com1* out_xcoms,
+                gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta);
+int gs_simulate_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
+                      const void* b_consts, const gs_fr* gamma, const void* target, const gs_fr* x_rand,
+                      const gs_fr* y_rand, const gs_fr* pf_rand, int shared_coms, const gs_fr* tkey,
+                      gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta);
+
 /* ---- verification (src/verifier.rs)----------------------------------------------------- */
 /* Verifiable::verify :23-157 for `count` independent (equation, proof) instances of the same
  * type and shape, each laid out contiguously with the given element counts:

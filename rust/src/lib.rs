@@ -13,6 +13,7 @@ pub mod extractor;
 pub mod ffi;
 pub mod generator;
 pub mod prover;
+pub mod simulator;
 pub mod statement;
 pub mod verifier;
 

@@ -11,9 +11,9 @@ use std::fmt::Debug;
 pub trait Commit: Eq + Debug { fn append(&mut self, other: &mut Self); }
 
 #[derive(Clone, Debug, CanonicalSerialize, CanonicalDeserialize)]
-pub struct Commit1<E: Gpu> { pub coms: Vec<Com1<E>>, pub(super) rand: Matrix<E::ScalarField> }
+pub struct Commit1<E: Gpu> { pub coms: Vec<Com1<E>>, pub(crate) rand: Matrix<E::ScalarField> }
 #[derive(Clone, Debug, CanonicalSerialize, CanonicalDeserialize)]
-pub struct Commit2<E: Gpu> { pub coms: Vec<Com2<E>>, pub(super) rand: Matrix<E::ScalarField> }
+pub struct Commit2<E: Gpu> { pub coms: Vec<Com2<E>>, pub(crate) rand: Matrix<E::ScalarField> }
 
 macro_rules! commit_impl {
     ($t:ident) => {

@@ -16,7 +16,7 @@ pub trait Provable<E: Gpu, A1, A2, AT> {
 }
 
 #[derive(Clone, Debug, PartialEq, Eq, CanonicalSerialize, CanonicalDeserialize)]
-pub struct EquProof<E: Gpu> { pub pi: Vec<Com2<E>>, pub theta: Vec<Com1<E>>, pub equ_type: EquType, rand: Matrix<E::ScalarField> }
+pub struct EquProof<E: Gpu> { pub pi: Vec<Com2<E>>, pub theta: Vec<Com1<E>>, pub equ_type: EquType, pub(crate) rand: Matrix<E::ScalarField> }
 
 #[derive(Clone, Debug, PartialEq, Eq)]
 pub struct CProof<E: Gpu> { pub xcoms: Commit1<E>, pub ycoms: Commit2<E>, pub equ_proofs: Vec<EquProof<E>> }
