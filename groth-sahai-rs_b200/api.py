@@ -408,6 +408,126 @@ def simulate_batch(equations, crs: CRS, key: SimulationKey, rng, shared_commitme
     return out
 
 
+# ---------------------------------------------------------------- zero knowledge for PPE targets (not in the reference)
+@dataclass
+class ZkPPE:
+    """A PPE  sum_j e(A_j, Y_j) + sum_i e(X_i, B_i) + sum_ij gamma_ij e(X_i, Y_j) = sum_k e(P_k, Q_k)  whose target is given
+    as K >= 1 public pairs (P_k in G1, Q_k in G2), proved zero-knowledge through the augmented statement of Groth & Sahai
+    (EUROCRYPT 2008): a PPE' with target 1 over (X | Z) with constants (B | -Q), and K equations Z_k - delta P_k = O whose
+    delta has the fixed commitment W2 (include/gs_b200.h, gs_zk_ppe_prove_batch).  Real proofs (prove) and simulated ones
+    (simulate, with the hiding CRS's trapdoor) are distributed identically under a hiding CRS."""
+    a_consts: List[bytes]                   # n x G1
+    b_consts: List[bytes]                   # m x G2
+    gamma: List[List[bytes]]                # m x n Fr
+    target_pairs: List[Tuple[bytes, bytes]]  # K x (G1, G2)
+
+    def shape(self): return len(self.b_consts), len(self.a_consts), len(self.target_pairs)
+
+    def prove(self, xvars, yvars, crs: CRS, rng) -> "ZkPPEProof":
+        return zk_prove_batch([self], [xvars], [yvars], crs, rng)[0]
+
+    def simulate(self, crs: CRS, key: SimulationKey, rng) -> "ZkPPEProof":
+        return zk_simulate_batch([self], crs, key, rng)[0]
+
+    def verify(self, proof: "ZkPPEProof", crs: CRS) -> bool:
+        return zk_verify_batch([self], [proof], crs)[0]
+
+
+@dataclass
+class ZkPPEProof:
+    xcoms: Commit1          # m + K: X_1..X_m, then Z_1..Z_K
+    ycoms: Commit2          # n
+    ppe: EquProof           # the proof of PPE' (target 1)
+    lin: List[EquProof]     # K MSMEG1 proofs of Z_k - delta P_k = O
+
+
+def _zk_statement_arrays(statements, name):
+    """(m, n, K, the five statement arrays of the C ABI) of a non-empty batch of one shape; ValueError names `name`."""
+    m, n, K = statements[0].shape()
+    for s in statements:
+        if s.shape() != (m, n, K) or len(s.gamma) != m or any(len(r) != n for r in s.gamma):
+            raise ValueError(f"{name}: every statement must have the same shape (m, n, K) and an m x n Gamma")
+    cat = lambda f: b"".join(f(s) for s in statements)
+    return m, n, K, (cat(lambda s: b"".join(s.a_consts)), cat(lambda s: b"".join(s.b_consts)), cat(lambda s: _flat(s.gamma)),
+                     cat(lambda s: b"".join(p for p, _ in s.target_pairs)), cat(lambda s: b"".join(q for _, q in s.target_pairs)))
+
+
+def _zk_draws(count, m, n, K, rng):
+    """per statement: R rows ((m + K) x 2), S rows (n x 2), T (2 x 2, row-major), then T_1..T_K (1 x 2 each)"""
+    draw = lambda rows, cols: [[rng.fr() for _ in range(cols)] for _ in range(rows)]
+    out = []
+    for _ in range(count):
+        R, S, T = draw(m + K, 2), draw(n, 2), draw(2, 2)
+        out.append((R, S, T, [draw(1, 2) for _ in range(K)]))
+    return out
+
+
+def _zk_proofs(out, draws, m, n, K, keep_rand):
+    xc, yc, pi, th, lpi, lth = out
+    res = []
+    for i, (R, S, T, Ts) in enumerate(draws):
+        lp, lt = _split(lpi[i * K * 768:(i + 1) * K * 768], 768), _split(lth[i * K * 192:(i + 1) * K * 192], 192)
+        res.append(ZkPPEProof(Commit1(_split(xc[i * (m + K) * 192:(i + 1) * (m + K) * 192], 192), R if keep_rand else []),
+                              Commit2(_split(yc[i * n * 384:(i + 1) * n * 384], 384), S if keep_rand else []),
+                              EquProof(_split(pi[i * 768:(i + 1) * 768], 384), _split(th[i * 384:(i + 1) * 384], 192), 0,
+                                       T if keep_rand else []),
+                              [EquProof(_split(p, 384), [t], 1, r if keep_rand else []) for p, t, r in zip(lp, lt, Ts)]))
+    return res
+
+
+def zk_prove_batch(statements, xvars, yvars, crs: CRS, rng) -> List[ZkPPEProof]:
+    """Zero-knowledge proofs of many ZkPPE statements of one shape (m, n, K) in one GPU pass (gs_zk_ppe_prove_batch);
+    xvars[i] (m x G1) and yvars[i] (n x G2) satisfy statement i.  Randomness is drawn statement by statement: R rows
+    ((m + K) x 2), S rows (n x 2), T (2 x 2, row-major), then T_1..T_K (1 x 2 each) -- the same stream as zk_simulate_batch."""
+    if not statements:
+        return []
+    m, n, K, arrays = _zk_statement_arrays(statements, "zk_prove_batch")
+    if len(xvars) != len(statements) or len(yvars) != len(statements) or any(len(x) != m for x in xvars) or \
+            any(len(y) != n for y in yvars):
+        raise ValueError("zk_prove_batch: one list of m x-variables and n y-variables per statement")
+    draws = _zk_draws(len(statements), m, n, K, rng)
+    cat = lambda f: b"".join(f(d) for d in draws)
+    out = crs._use().zk_ppe_prove_batch(
+        len(statements), m, n, K, *arrays, b"".join(b"".join(x) for x in xvars), b"".join(b"".join(y) for y in yvars),
+        cat(lambda d: _flat(d[0])), cat(lambda d: _flat(d[1])), cat(lambda d: _flat(d[2])), cat(lambda d: b"".join(_flat(t) for t in d[3])))
+    return _zk_proofs(out, draws, m, n, K, True)
+
+
+def zk_simulate_batch(statements, crs: CRS, key: SimulationKey, rng) -> List[ZkPPEProof]:
+    """ZkPPEProofs that verify under the hiding CRS `crs` for ANY target pairs, made without witnesses with its trapdoor
+    `key` in one GPU pass (gs_zk_ppe_simulate_batch).  Draws as zk_prove_batch.  The returned Commit*.rand and
+    EquProof.rand are empty, as for simulate_batch.  A key that does not belong to `crs` raises GsError."""
+    if not statements:
+        return []
+    m, n, K, arrays = _zk_statement_arrays(statements, "zk_simulate_batch")
+    draws = _zk_draws(len(statements), m, n, K, rng)
+    cat = lambda f: b"".join(f(d) for d in draws)
+    out = crs._use().zk_ppe_simulate_batch(
+        len(statements), m, n, K, *arrays, cat(lambda d: _flat(d[0])), cat(lambda d: _flat(d[1])), cat(lambda d: _flat(d[2])),
+        cat(lambda d: b"".join(_flat(t) for t in d[3])), key.to_bytes())
+    return _zk_proofs(out, draws, m, n, K, False)
+
+
+def zk_verify_batch(statements, proofs, crs: CRS) -> List[bool]:
+    """Verdicts of many (ZkPPE, ZkPPEProof) pairs of one shape in one GPU pass (gs_zk_ppe_verify_batch): a statement is
+    accepted iff PPE' and every Z_k - delta P_k = O verify, with delta's commitment W2 taken from `crs`."""
+    if len(proofs) != len(statements):
+        raise ValueError("zk_verify_batch: one proof per statement")
+    if not statements:
+        return []
+    m, n, K, arrays = _zk_statement_arrays(statements, "zk_verify_batch")
+    for p in proofs:
+        if len(p.xcoms.coms) != m + K or len(p.ycoms.coms) != n or len(p.lin) != K or len(p.ppe.pi) != 2 or \
+                len(p.ppe.theta) != 2 or any(len(e.pi) != 2 or len(e.theta) != 1 for e in p.lin):
+            raise ValueError("zk_verify_batch: a proof does not match the statements' shape (m, n, K)")
+    cat = lambda f: b"".join(f(p) for p in proofs)
+    ok = crs._use().zk_ppe_verify_batch(
+        len(statements), m, n, K, *arrays, cat(lambda p: b"".join(p.xcoms.coms)), cat(lambda p: b"".join(p.ycoms.coms)),
+        cat(lambda p: b"".join(p.ppe.pi)), cat(lambda p: b"".join(p.ppe.theta)),
+        cat(lambda p: b"".join(b"".join(e.pi) for e in p.lin)), cat(lambda p: b"".join(b"".join(e.theta) for e in p.lin)))
+    return [b == 1 for b in ok]
+
+
 # ---------------------------------------------------------------- extraction with the binding key (not in the reference)
 # X = c.1 - a1 c.0 for a commitment under a binding CRS (u[0] = (p1, a1 p1), u[1] = t1 u[0]); scalar commitments give x p1
 # (x itself cannot be recovered), the G2 side likewise with a2 (gs_extract).  The key is checked against the engine's

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 OUT = os.path.join(HERE, "libgs_b200.so")
-SOURCES = ["core.cu", "pairing.cu", "finalexp.cu", "verify.cu", "prover.cu", "prover_g1.cu", "prover_g2.cu", "groupops.cu", "serial.cu", "extract.cu", "simulate.cu"]
+SOURCES = ["core.cu", "pairing.cu", "finalexp.cu", "verify.cu", "prover.cu", "prover_g1.cu", "prover_g2.cu", "groupops.cu", "serial.cu", "extract.cu", "simulate.cu", "zk.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

@@ -330,6 +330,24 @@ int theta_pi_fork(gs_ctx* ctx, bool two_streams, const char* what, Theta&& theta
   return rc_th ? rc_th : rc_pi;
 }
 
+// prover.cu: `count` proofs of one type and shape (gs_prove_batch, host arrays)
+int prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+               const gs_fr* gamma, const void* xvars, const void* yvars, const gs_fr* x_rand, const gs_fr* y_rand,
+               const gs_fr* pf_rand, bool shared_vars, gs_com2* out_pi, gs_com1* out_theta);
+// simulate.cu: `count` simulated proofs (gs_simulate_batch, host arrays), and the check of tkey against the loaded CRS
+// that gs_simulate_batch runs first (cached in ctx->tkey).  with_coms = false: the commitments of O / 0 are neither made nor
+// written (a caller that has them already); out_xcoms / out_ycoms may then be null
+int simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                  const gs_fr* gamma, const void* target, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
+                  const gs_fr* tkey, gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta,
+                  bool with_coms = true);
+int sim_key_check(gs_ctx* ctx, const gs_fr* tkey);
+// verify.cu: gs_verify_batch_dev (device arrays, verdicts out_ok_dev[count]); `shared_y`: every problem has the same
+// y-commitments, whose lines are then walked once
+int verify_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+               const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+               const gs_com1* theta, bool shared_y, uint8_t* out_ok_dev);
+
 // extract.cu: *all_identity = (coms[i].1 - key coms[i].0 is the identity for every i < n), n DEVICE commitments (k_extract)
 template <class F>
 int extract_all_identity(gs_ctx* ctx, const Aff<F>* coms, size_t n, const gs_fr* key, bool* all_identity);

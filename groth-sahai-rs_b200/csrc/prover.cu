@@ -274,12 +274,14 @@ int gs_batch_commit_scalar_b2(gs_ctx* ctx, size_t n, const gs_fr* ys, const gs_f
   return batch_commit_impl<Fp2Ops>(ctx, n, 2, 0, buf.data(), 1, buf.data() + n, 1, 2 * n, nullptr, out);
 }
 
+}  // extern "C"
+
 // `count` independent Provable::prove calls of one type and shape, every kernel batched over blockIdx.y.
 // Per-proof arrays are contiguous ([count][...]); with shared_vars the witnesses and their commitment randomness
 // are one set.  gs_prove is the batch of one.
-static int prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                      const gs_fr* gamma, const void* xvars, const void* yvars, const gs_fr* x_rand, const gs_fr* y_rand,
-                      const gs_fr* pf_rand, bool shared_vars, gs_com2* out_pi, gs_com1* out_theta) {
+int gsi::prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                    const gs_fr* gamma, const void* xvars, const void* yvars, const gs_fr* x_rand, const gs_fr* y_rand,
+                    const gs_fr* pf_rand, bool shared_vars, gs_com2* out_pi, gs_com1* out_theta) {
   if (!ctx) return GS_EARG;
   if (type < 0 || type > 3) FAIL(GS_EARG, "prove: bad equation type");
   if (!ctx->crs_loaded) FAIL(GS_EARG, "prove: no CRS loaded");
@@ -353,6 +355,8 @@ static int prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, c
   }
   return GS_OK;
 }
+
+extern "C" {
 
 int gs_prove(gs_ctx* ctx, int type, size_t m, size_t n, const void* a_consts, const void* b_consts, const gs_fr* gamma,
              const void* xvars, const void* yvars, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand,

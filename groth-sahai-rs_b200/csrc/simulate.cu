@@ -31,9 +31,11 @@ int trapdoor_matches(gs_ctx* ctx, const Aff<F>* key0, const Aff<F>* w, const gs_
   return extract_all_identity<F>(ctx, pairs, 2, t, ok);
 }
 
+}  // namespace
+
 // tkey = (t1, t2) is the loaded CRS's simulation key iff W1 = t1 u[0] and W2 = t2 v[0].  Under a binding key
 // W1 = t1 u[0] + iota_1(g1), so no key passes.  A validated key is cached until the next gs_crs_load / gs_crs_generate.
-int sim_key_check(gs_ctx* ctx, const gs_fr* tkey) {
+int gsi::sim_key_check(gs_ctx* ctx, const gs_fr* tkey) {
   if (ctx->tkey_valid && memcmp(ctx->tkey, tkey, sizeof(ctx->tkey)) == 0) return GS_OK;
   bool ok1, ok2;
   int rc = trapdoor_matches<FpOps>(ctx, &ctx->crs->u[0][0], &ctx->crs->w1[0], &tkey[0], &ok1);
@@ -45,6 +47,8 @@ int sim_key_check(gs_ctx* ctx, const gs_fr* tkey) {
   ctx->tkey_valid = true;
   return GS_OK;
 }
+
+namespace {
 
 // c_i = R[i] key for N commitments of O / 0 (host arrays): R[i][0] key_0 + R[i][1] key_1 (ns = 2) or r_i key_0 (ns = 1,
 // the second scalar stream is a zero with stride 0 on W)
@@ -67,16 +71,19 @@ cudaError_t upload_with_column(gs_ctx* ctx, Scratch& sc, uint8_t** dst, const vo
   return e;
 }
 
-int simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                  const gs_fr* gamma, const void* target, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
-                  const gs_fr* tkey, gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta) {
+}  // namespace
+
+int gsi::simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                       const gs_fr* gamma, const void* target, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
+                       const gs_fr* tkey, gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta,
+                       bool with_coms) {
   if (!ctx) return GS_EARG;
   if (type < 0 || type > 3) FAIL(GS_EARG, "simulate: bad equation type");
   if (!ctx->crs_loaded) FAIL(GS_EARG, "simulate: no CRS loaded");
   if (count == 0) return GS_OK;
   if (m == 0 || n == 0) FAIL(GS_EDIM, "simulate: empty variable list");
   if (m > 1 << 22 || n > 1 << 22) FAIL(GS_EDIM, "simulate: too many variables");
-  if (!a_consts || !b_consts || !gamma || !target || !x_rand || !y_rand || !pf_rand || !tkey || !out_xcoms || !out_ycoms ||
+  if (!a_consts || !b_consts || !gamma || !target || !x_rand || !y_rand || !pf_rand || !tkey || (with_coms && (!out_xcoms || !out_ycoms)) ||
       !out_pi || !out_theta)
     return GS_EARG;
   if (type == GS_PPE) {
@@ -94,8 +101,8 @@ int simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const
   const size_t szA = elem_size_A(type), szB = elem_size_B(type), szT = elem_size_T(type);
   const size_t nv = shared ? 1 : count;
   // the commitments first: a big batch (re)builds the fixed-base tables that the proof elements read
-  if ((rc = commit_zero<FpOps>(ctx, nv * m, cx, x_rand, out_xcoms))) return rc;
-  if ((rc = commit_zero<Fp2Ops>(ctx, nv * n, cy, y_rand, out_ycoms))) return rc;
+  if (with_coms && (rc = commit_zero<FpOps>(ctx, nv * m, cx, x_rand, out_xcoms))) return rc;
+  if (with_coms && (rc = commit_zero<Fp2Ops>(ctx, nv * n, cy, y_rand, out_ycoms))) return rc;
   // the extra constant column: theta's for MSMEG1 / Quad, pi's for MSMEG2, with the scalar -t2 / -t1 in every proof
   const size_t xa = (type == GS_MSMEG1 || type == GS_QUAD) ? 1 : 0, yb = type == GS_MSMEG2 ? 1 : 0;
   const size_t MAXB = 32768;  // gridDim.y limit is 65,535
@@ -175,8 +182,6 @@ int simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const
   }
   return GS_OK;
 }
-
-}  // namespace
 
 extern "C" {
 

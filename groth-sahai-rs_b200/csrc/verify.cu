@@ -1044,6 +1044,17 @@ int gs_verify_batch_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n,
                      nullptr, false);
 }
 
+}  // extern "C"
+
+int gsi::verify_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                    const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                    const gs_com1* theta, bool shared_y, uint8_t* out_ok_dev) {
+  return verify_impl(ctx, type, count, m, n, args_of(a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta), 0, 1, out_ok_dev,
+                     nullptr, false, shared_y);
+}
+
+extern "C" {
+
 int gs_verify_partial_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts,
                           const void* b_consts, const gs_fr* gamma, const void* target, const gs_com1* xcoms,
                           const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, int rank, int world,

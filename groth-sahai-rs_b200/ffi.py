@@ -16,7 +16,8 @@ EXPORTED_SYMBOLS = [
     "gs_profile_enable", "gs_profile_read", "gs_diag_fpmul_rate",
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
-    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_simulate", "gs_simulate_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_simulate", "gs_simulate_batch",
+    "gs_zk_ppe_prove_batch", "gs_zk_ppe_simulate_batch", "gs_zk_ppe_verify_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_each_rand", "gs_verify_each_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
@@ -79,6 +80,9 @@ def load_library():
         lib.gs_extract.argtypes = [vp, sz, vp, vp, sz, vp, vp, vp, vp]
         lib.gs_simulate.argtypes = [vp, ci, sz, sz] + [vp] * 12
         lib.gs_simulate_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 7 + [ci] + [vp] * 5
+        lib.gs_zk_ppe_prove_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 17
+        lib.gs_zk_ppe_simulate_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 16
+        lib.gs_zk_ppe_verify_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 12
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
@@ -336,6 +340,56 @@ class Engine:
         ks = [_buf(x) for x in (a_consts, b_consts, gamma, target, x_rand, y_rand, pf_rand, tkey)]
         self._chk(self.lib.gs_simulate(self.h, ty, m, n, *[k[1] for k in ks], *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
         return outs[0].raw[: m * COM1], outs[1].raw[: n * COM2], outs[2].raw[: cx * COM2], outs[3].raw[: cy * COM1]
+
+    # ---- zero knowledge for PPE targets given as pairs (gs_zk_ppe_*_batch)
+    @staticmethod
+    def _zk_sizes(count, m, n, K, named):
+        """The C side reads count * (shape) bytes from every buffer: a short one would be read past its end."""
+        want = {"a_consts": n * G1, "b_consts": m * G2, "gamma": m * n * FR, "tp": K * G1, "tq": K * G2, "xvars": m * G1,
+                "yvars": n * G2, "x_rand": (m + K) * 2 * FR, "y_rand": n * 2 * FR, "pf_rand": 4 * FR, "lin_rand": K * 2 * FR,
+                "xcoms": (m + K) * COM1, "ycoms": n * COM2, "pi": 2 * COM2, "theta": 2 * COM1, "lin_pi": K * 2 * COM2,
+                "lin_theta": K * COM1, "tkey": 2 * FR}
+        for nm, buf in named.items():
+            w = want[nm] * (1 if nm == "tkey" else count)
+            if len(buf) != w:
+                raise GsError(1, f"zk_ppe: {nm} is {len(buf)} bytes, expected {w} for count {count}, m {m}, n {n}, K {K}")
+
+    def _zk_proofs(self, fn, count, m, n, K, named):
+        """call gs_zk_ppe_prove_batch / _simulate_batch; (xcoms, ycoms, pi, theta, lin_pi, lin_theta) bytes"""
+        if count and m and n and K:
+            self._zk_sizes(count, m, n, K, named)
+        sizes = [count * k for k in ((m + K) * COM1, n * COM2, 2 * COM2, 2 * COM1, K * 2 * COM2, K * COM1)]
+        outs = [ctypes.create_string_buffer(max(1, k)) for k in sizes]
+        ks = [_buf(x) for x in named.values()]
+        self._chk(fn(self.h, count, m, n, K, *[k[1] for k in ks], *[ctypes.cast(o, ctypes.c_void_p) for o in outs]))
+        return tuple(o.raw[:k] for o, k in zip(outs, sizes))
+
+    def zk_ppe_prove_batch(self, count, m, n, K, a_consts, b_consts, gamma, tp, tq, xvars, yvars, x_rand, y_rand, pf_rand,
+                           lin_rand):
+        """`count` zero-knowledge proofs of PPEs whose targets are the products of K pairings e(tp_k, tq_k)
+        (gs_zk_ppe_prove_batch).  Returns (xcoms, ycoms, pi, theta, lin_pi, lin_theta) bytes, proof-major."""
+        return self._zk_proofs(self.lib.gs_zk_ppe_prove_batch, count, m, n, K, dict(
+            a_consts=a_consts, b_consts=b_consts, gamma=gamma, tp=tp, tq=tq, xvars=xvars, yvars=yvars, x_rand=x_rand,
+            y_rand=y_rand, pf_rand=pf_rand, lin_rand=lin_rand))
+
+    def zk_ppe_simulate_batch(self, count, m, n, K, a_consts, b_consts, gamma, tp, tq, x_rand, y_rand, pf_rand, lin_rand, tkey):
+        """The outputs of zk_ppe_prove_batch without witnesses, made with the hiding key tkey = t1 || t2
+        (gs_zk_ppe_simulate_batch); they verify for any target pairs."""
+        return self._zk_proofs(self.lib.gs_zk_ppe_simulate_batch, count, m, n, K, dict(
+            a_consts=a_consts, b_consts=b_consts, gamma=gamma, tp=tp, tq=tq, x_rand=x_rand, y_rand=y_rand, pf_rand=pf_rand,
+            lin_rand=lin_rand, tkey=tkey))
+
+    def zk_ppe_verify_batch(self, count, m, n, K, a_consts, b_consts, gamma, tp, tq, xcoms, ycoms, pi, theta, lin_pi,
+                            lin_theta) -> bytes:
+        """out_ok bytes of gs_zk_ppe_verify_batch: 1 iff PPE' and every L_k of the statement verify."""
+        named = dict(a_consts=a_consts, b_consts=b_consts, gamma=gamma, tp=tp, tq=tq, xcoms=xcoms, ycoms=ycoms, pi=pi,
+                     theta=theta, lin_pi=lin_pi, lin_theta=lin_theta)
+        if count and m and n and K:
+            self._zk_sizes(count, m, n, K, named)
+        ok = ctypes.create_string_buffer(max(1, count))
+        ks = [_buf(x) for x in named.values()]
+        self._chk(self.lib.gs_zk_ppe_verify_batch(self.h, count, m, n, K, *[k[1] for k in ks], ctypes.cast(ok, ctypes.c_void_p)))
+        return ok.raw[:count]
 
     @staticmethod
     def _check_verify_sizes(ty, count, m, n, a_consts, b_consts, gamma, target, xcoms, ycoms, pi, theta, gamma_rows=None):

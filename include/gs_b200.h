@@ -189,6 +189,47 @@ int gs_simulate_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, c
                       const gs_fr* y_rand, const gs_fr* pf_rand, int shared_coms, const gs_fr* tkey,
                       gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta);
 
+/* ---- zero knowledge for PPE targets (not in the reference) ---------------------------------------- */
+/* gs_simulate_batch takes PPE statements with target 1 only.  A PPE with a target given as K >= 1 public pairs,
+ *     sum_j e(A_j, Y_j) + sum_i e(X_i, B_i) + sum_ij gamma_ij e(X_i, Y_j) = sum_k e(P_k, Q_k),
+ * is proved zero-knowledge as the augmented statement of Groth & Sahai (EUROCRYPT 2008; PAPERS.md):
+ *   PPE'  target 1, x-variables (X_1..X_m, Z_1..Z_K), b' = (B_1..B_m, -Q_1..-Q_K), a' = A, Gamma' = Gamma + K zero rows;
+ *   L_k   (k = 1..K) the MSMEG1 equation Z_k - delta P_k = O: x-variable Z_k, scalar y-variable delta, a = [-P_k],
+ *         b = [1], Gamma = [[0]], target O.  The x-commitment of L_k is c_{m+k} of PPE'.
+ * delta's commitment is FIXED: W2 = 1 W2 + 0 v[0], which the verifier takes from the loaded CRS, never from the proof.
+ * Under a binding CRS it binds delta = 1, so Z_k = P_k and PPE' is the original equation.  Under a hiding CRS
+ * W2 = t2 v[0] is also the commitment of 0 with randomness t2: the simulator proves L_k with Z_k = O, delta = 0.
+ *   prove    witness (X, Y, Z = P, delta = 1): c = commit(X | P) under R, d = commit(Y) under S (gs_batch_commit_g1 / _g2),
+ *            PPE' proved under T (gs_prove_batch), L_k proved with xvars [P_k], yvars [1], x_rand = row m+k of R,
+ *            y_rand [0] and T_k (gs_prove_batch of MSMEG1).
+ *   simulate c = R u, d = S v (commitments of O), PPE' simulated with target 1 (gs_simulate_batch), L_k simulated as
+ *            MSMEG1 with target O, x_rand = row m+k of R, y_rand [t2] and T_k.
+ *   verify   accepted iff PPE' verifies on (c, d, pi, theta) and every L_k on ([c_{m+k}], [W2], lin_pi_k, lin_theta_k).
+ * Real and simulated proofs are honest proofs of the same augmented statement, identically distributed under a hiding
+ * CRS.  Arrays are proof-major (count statements of one shape m, n, K):
+ *   a_consts[count][n] (G1), b_consts[count][m] (G2), gamma[count][m][n], tp[count][K] (G1), tq[count][K] (G2),
+ *   xvars[count][m], yvars[count][n], x_rand[count][m+K][2], y_rand[count][n][2], pf_rand[count][2][2],
+ *   lin_rand[count][K][1][2]; out_xcoms[count][m+K], out_ycoms[count][n], out_pi[count][2], out_theta[count][2],
+ *   out_lin_pi[count][K][2], out_lin_theta[count][K][1] (verify reads the same names without out_).
+ * The simulator takes no witnesses and the hiding key tkey = (t1, t2), checked as for gs_simulate_batch.
+ * GS_EDIM for m, n or K = 0 (a target-1 PPE needs no augmented statement: gs_prove / gs_simulate) or m + K, n over 2^20;
+ * GS_EARG, with nothing written, for a null pointer, no loaded CRS, or a tkey that is not the loaded CRS's simulation key
+ * (every binding CRS fails).  count == 0 returns GS_OK.  out_ok[i] = 1 iff statement i verifies. */
+int gs_zk_ppe_prove_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                          const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
+                          const gs_g1* xvars, const gs_g2* yvars, const gs_fr* x_rand, const gs_fr* y_rand,
+                          const gs_fr* pf_rand, const gs_fr* lin_rand, gs_com1* out_xcoms, gs_com2* out_ycoms,
+                          gs_com2* out_pi, gs_com1* out_theta, gs_com2* out_lin_pi, gs_com1* out_lin_theta);
+int gs_zk_ppe_simulate_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                             const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
+                             const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, const gs_fr* lin_rand,
+                             const gs_fr* tkey /* [2] = t1, t2 */, gs_com1* out_xcoms, gs_com2* out_ycoms,
+                             gs_com2* out_pi, gs_com1* out_theta, gs_com2* out_lin_pi, gs_com1* out_lin_theta);
+int gs_zk_ppe_verify_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                           const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
+                           const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                           const gs_com2* lin_pi, const gs_com1* lin_theta, uint8_t* out_ok);
+
 /* ---- verification (src/verifier.rs)----------------------------------------------------- */
 /* Verifiable::verify :23-157 for `count` independent (equation, proof) instances of the same
  * type and shape, each laid out contiguously with the given element counts:

@@ -71,6 +71,21 @@ extern "C" {
                              gamma: *const GsFr, target: *const u8, x_rand: *const GsFr, y_rand: *const GsFr,
                              pf_rand: *const GsFr, shared_coms: i32, tkey: *const GsFr, out_xcoms: *mut GsCom1,
                              out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1) -> i32;
+    // not in the reference: zero knowledge for PPE targets given as pairs (tp[count][K] in G1, tq[count][K] in G2)
+    pub fn gs_zk_ppe_prove_batch(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
+                                 gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, xvars: *const GsG1, yvars: *const GsG2,
+                                 x_rand: *const GsFr, y_rand: *const GsFr, pf_rand: *const GsFr, lin_rand: *const GsFr,
+                                 out_xcoms: *mut GsCom1, out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1,
+                                 out_lin_pi: *mut GsCom2, out_lin_theta: *mut GsCom1) -> i32;
+    pub fn gs_zk_ppe_simulate_batch(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
+                                    gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, x_rand: *const GsFr, y_rand: *const GsFr,
+                                    pf_rand: *const GsFr, lin_rand: *const GsFr, tkey: *const GsFr, out_xcoms: *mut GsCom1,
+                                    out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1, out_lin_pi: *mut GsCom2,
+                                    out_lin_theta: *mut GsCom1) -> i32;
+    pub fn gs_zk_ppe_verify_batch(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
+                                  gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, xcoms: *const GsCom1, ycoms: *const GsCom2,
+                                  pi: *const GsCom2, theta: *const GsCom1, lin_pi: *const GsCom2, lin_theta: *const GsCom1,
+                                  out_ok: *mut u8) -> i32;
     // verifier.rs:23-157
     pub fn gs_verify_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                            gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,

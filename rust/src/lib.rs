@@ -16,6 +16,7 @@ pub mod prover;
 pub mod simulator;
 pub mod statement;
 pub mod verifier;
+pub mod zk;
 
 pub use crate::generator::{AbstractCrs, CRS};
 pub use crate::statement::*;
