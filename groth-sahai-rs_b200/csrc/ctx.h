@@ -170,6 +170,59 @@ struct PassStreams {
   }
 };
 
+// Side work on the context's second stream next to the main stream (ctx->stream at construction).  fork(): the second
+// stream waits for everything queued on the main stream so far and becomes ctx->stream; back(): ctx->stream is the main
+// stream again, the side work stays pending; join(): the main stream waits for the side work (back() first if still
+// forked).  The destructor joins, so on every exit the main stream -- where Scratch releases its buffers -- is ordered after
+// the side work.  A failed event creation, record or wait is GS_ECUDA; both events are destroyed on every path.  With
+// `two` = false everything stays on the main stream and the calls do nothing.
+struct SideStream {
+  gs_ctx* ctx;
+  cudaStream_t main_s;
+  bool two, forked = false, pending = false;
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  explicit SideStream(gs_ctx* c, bool two_streams = true) : ctx(c), main_s(c->stream), two(two_streams) {}
+  SideStream(const SideStream&) = delete;
+  SideStream& operator=(const SideStream&) = delete;
+  int fork() {
+    if (!two) return GS_OK;
+    if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
+    if (!ev_fork) CUDA_TRY(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
+    if (!ev_join) CUDA_TRY(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventRecord(ev_fork, main_s));
+    CUDA_TRY(cudaStreamWaitEvent(ctx->stream2, ev_fork, 0));
+    ctx->stream = ctx->stream2;
+    forked = true;
+    return GS_OK;
+  }
+  int back() {
+    if (!forked) return GS_OK;
+    forked = false;
+    ctx->stream = main_s;
+    CUDA_TRY(cudaEventRecord(ev_join, ctx->stream2));
+    pending = true;
+    return GS_OK;
+  }
+  int join() {
+    if (int rc = back()) return rc;
+    if (!pending) return GS_OK;
+    pending = false;
+    CUDA_TRY(cudaStreamWaitEvent(main_s, ev_join, 0));
+    return GS_OK;
+  }
+  ~SideStream() {
+    join();
+    if (ev_fork) cudaEventDestroy(ev_fork);
+    if (ev_join) cudaEventDestroy(ev_join);
+  }
+};
+// joins `side` when it goes out of scope: declared after a Scratch whose buffers the side work uses, it orders the main
+// stream after that work on every exit (error returns included) before the Scratch releases them
+struct SideJoin {
+  SideStream& side;
+  ~SideJoin() { side.join(); }
+};
+
 template <class T>
 static inline cudaError_t upload(gs_ctx* ctx, Scratch& s, T** dst, const void* src, size_t count) {
   cudaError_t e = s.alloc(dst, count);
@@ -300,34 +353,17 @@ template <class F>
 int com_matmul_impl(gs_ctx* ctx, size_t r, size_t k, size_t c, const gs_fr* lhs, const void* mat, void* out);
 
 // theta (G1, `theta()`) and pi (G2, `pi()`) of a batch of proofs are independent: in the latency regime (`two_streams`: few
-// products) theta runs on the second stream next to pi.  Returns theta's error code, else pi's.
+// products) theta runs on the second stream next to pi.  The join also orders the scratch frees (main stream) after
+// theta's kernels.
 template <class Theta, class Pi>
-int theta_pi_fork(gs_ctx* ctx, bool two_streams, const char* what, Theta&& theta, Pi&& pi) {
-  cudaStream_t main_stream = ctx->stream;
-  cudaEvent_t fork = nullptr, join = nullptr;
-  if (two_streams) {
-    if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-    CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-    if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
-      cudaEventDestroy(fork);
-      FAIL(GS_ECUDA, std::string(what) + ": event creation failed");
-    }
-    cudaEventRecord(fork, main_stream);
-    cudaStreamWaitEvent(ctx->stream2, fork, 0);
-    ctx->stream = ctx->stream2;
-  }
-  int rc_th = theta();
-  if (two_streams) {
-    cudaEventRecord(join, ctx->stream2);
-    ctx->stream = main_stream;
-  }
-  int rc_pi = pi();
-  if (two_streams) {
-    cudaStreamWaitEvent(main_stream, join, 0);  // also orders the scratch frees (main stream) after theta's kernels
-    cudaEventDestroy(fork);
-    cudaEventDestroy(join);
-  }
-  return rc_th ? rc_th : rc_pi;
+int theta_pi_fork(gs_ctx* ctx, bool two_streams, Theta&& theta, Pi&& pi) {
+  SideStream side(ctx, two_streams);
+  int rc = side.fork();
+  if (!rc) rc = theta();
+  if (!rc) rc = side.back();
+  if (!rc) rc = pi();
+  if (!rc) rc = side.join();
+  return rc;
 }
 
 // prover.cu: `count` proofs of one type and shape (gs_prove_batch, host arrays)

@@ -343,7 +343,7 @@ int gsi::prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, con
     // theta_i = sum_j S[j][i] iota(A_j) + sum_k SG[i][k] iota(X_k) + sum_l T[i][l] u_l          (l < cx)
     // theta on the second stream next to pi in the latency regime (few proofs)
     int rc = theta_pi_fork(
-        ctx, nb * (m + n) * 2 < 32768, "prove",
+        ctx, nb * (m + n) * 2 < 32768,
         [&] { return proof_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, dA, n, dX, m, shared_vars, cx, dT, (size_t)cx, e_th, dth); },
         [&] {
           return proof_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, dB, m, dY, n, shared_vars, cy, coef_pi, (size_t)cy, e_pi, dpi);
@@ -465,7 +465,7 @@ static int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_
     CUDA_TRY(sc.alloc(&dto, nb * 2 * cy));
     // theta' on the second stream next to pi' in the latency regime, as in prove_impl
     int rc = theta_pi_fork(
-        ctx, nb * (m + n) * 2 < 32768, "rerandomize",
+        ctx, nb * (m + n) * 2 < 32768,
         [&] { return rerand_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, SG, dA, n, dXc, m, shared, cx, dT, e_th, dTh, dto); },
         [&] { return rerand_element<Fp2Ops>(ctx, sc, nb, cx, s.groupB, sv_pi, RG, dB, m, dYc, n, shared, cy, coef_pi, e_pi, dPi, dpo); });
     if (rc) return rc;

@@ -749,42 +749,28 @@ int proof_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_t
       Aff<F>* ptab;
       Jac<F>* J;
       CUDA_TRY(shared_base_alloc<F>(sc, nvars, &ptab, &J));
-      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-      cudaEvent_t fork, join;
-      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-      CUDA_TRY(cudaEventCreateWithFlags(&join, cudaEventDisableTiming));
-      CUDA_TRY(cudaEventRecord(fork, ctx->stream));
-      CUDA_TRY(cudaStreamWaitEvent(ctx->stream2, fork, 0));
-      cudaStream_t main_stream = ctx->stream;
-      ctx->stream = ctx->stream2;
-      int rct = [&]() -> int {
-        if (nvars == 0) return GS_OK;
+      SideStream side(ctx);
+      if (int rc = side.fork()) return rc;
+      if (nvars > 0) {
         int rcb = shared_base_tables<F>(ctx, (const Aff<F>*)dvars, nvars, ptab, J);
         if (rcb) return rcb;
         LAUNCH_B((k_msm_var_terms_tab<F>), nvars * rows, count, terms, sv, ptab, nconst, nvars, rows);
-        return GS_OK;
-      }();
-      cudaEventRecord(join, ctx->stream2);
-      ctx->stream = main_stream;
-      int rcc = [&]() -> int {
-        if (nconst * PipSplit<F>::PARTS >= 64 && count >= 16) {
-          // shared witnesses = shared commitment randomness: the constants of ALL equations are multiplied by the same
-          // scalar vector, so the bucket lists are built once and every equation sums its points along them
-          // (pippenger.cuh, "ONE scalar vector").  The sum lands in term slot 0, the other constant slots are identities.
-          for (int row = 0; row < rows; row++)
-            CUDA_TRY(cudaMemset2DAsync(terms + (size_t)row * nt, nt * rows * sizeof(Jac<F>), 0, nconst * sizeof(Jac<F>), count,
-                                       ctx->stream));
-          return shared_scalar_sums<F>(ctx, sc, sv, nt, rows, (const Aff<F>*)dconst, nconst, count, terms, nt);
-        }
+      }
+      if (int rc = side.back()) return rc;
+      if (nconst * PipSplit<F>::PARTS >= 64 && count >= 16) {
+        // shared witnesses = shared commitment randomness: the constants of ALL equations are multiplied by the same
+        // scalar vector, so the bucket lists are built once and every equation sums its points along them
+        // (pippenger.cuh, "ONE scalar vector").  The sum lands in term slot 0, the other constant slots are identities.
+        for (int row = 0; row < rows; row++)
+          CUDA_TRY(cudaMemset2DAsync(terms + (size_t)row * nt, nt * rows * sizeof(Jac<F>), 0, nconst * sizeof(Jac<F>), count,
+                                     ctx->stream));
+        int rcs = shared_scalar_sums<F>(ctx, sc, sv, nt, rows, (const Aff<F>*)dconst, nconst, count, terms, nt);
+        if (rcs) return rcs;
+      } else {
         LAUNCH_B((k_msm_terms<F>), nconst * rows, count, terms, sv, (const Aff<F>*)dconst, nconst, (const Aff<F>*)dvars, (size_t)0, rows,
                  (size_t)0, 1, nt);
-        return GS_OK;
-      }();
-      cudaStreamWaitEvent(ctx->stream, join, 0);
-      cudaEventDestroy(fork);
-      cudaEventDestroy(join);
-      if (rct) return rct;
-      if (rcc) return rcc;
+      }
+      if (int rc = side.join()) return rc;
     }
     int rc = reduce_rows<F>(ctx, terms, ntp, ntp, rows, count);
     if (rc) return rc;
@@ -860,37 +846,20 @@ int rerand_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_
       Aff<F>* ptab;
       Jac<F>* J;
       CUDA_TRY(shared_base_alloc<F>(sc, 2 * ncom, &ptab, &J));
-      if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-      cudaEvent_t fork, join;
-      CUDA_TRY(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-      if (cudaEventCreateWithFlags(&join, cudaEventDisableTiming) != cudaSuccess) {
-        cudaEventDestroy(fork);
-        FAIL(GS_ECUDA, "rerandomize: event creation failed");
-      }
-      cudaEventRecord(fork, ctx->stream);
-      cudaStreamWaitEvent(ctx->stream2, fork, 0);
-      cudaStream_t main_stream = ctx->stream;
-      ctx->stream = ctx->stream2;
-      int rct = [&]() -> int {
-        int rcb = shared_base_tables<F>(ctx, dcom, 2 * ncom, ptab, J);
-        if (rcb) return rcb;
-        LAUNCH_B((k_rerand_com_terms_tab<F>), (size_t)rows * 2 * ncom, count, terms, sv, svs, nconst, ptab, n0, ncom, rows);
-        return GS_OK;
-      }();
-      cudaEventRecord(join, ctx->stream2);
-      ctx->stream = main_stream;
-      int rcc = [&]() -> int {
-        if (n0 == 0) return GS_OK;
-        if (const_sums) return shared_scalar_sums<F>(ctx, sc, sv, svs, rows, B, n0, count, terms + ntp, 2 * ntp);
+      SideStream side(ctx);
+      if (int rc = side.fork()) return rc;
+      int rcb = shared_base_tables<F>(ctx, dcom, 2 * ncom, ptab, J);
+      if (rcb) return rcb;
+      LAUNCH_B((k_rerand_com_terms_tab<F>), (size_t)rows * 2 * ncom, count, terms, sv, svs, nconst, ptab, n0, ncom, rows);
+      if (int rc = side.back()) return rc;
+      if (n0 > 0 && const_sums) {
+        int rcs = shared_scalar_sums<F>(ctx, sc, sv, svs, rows, B, n0, count, terms + ntp, 2 * ntp);
+        if (rcs) return rcs;
+      } else if (n0 > 0) {
         LAUNCH_B((k_rerand_terms<F>), (size_t)rows * n0, count, terms, sv, svs, nconst, B, n0, dcom, ncom, (size_t)0, rows,
                  (size_t)0, n0, 1);
-        return GS_OK;
-      }();
-      cudaStreamWaitEvent(ctx->stream, join, 0);
-      cudaEventDestroy(fork);
-      cudaEventDestroy(join);
-      if (rct) return rct;
-      if (rcc) return rcc;
+      }
+      if (int rc = side.join()) return rc;
     }
     int rc = reduce_rows<F>(ctx, terms, ntp, ntp, rows * 2, count);
     if (rc) return rc;

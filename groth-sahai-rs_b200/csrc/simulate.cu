@@ -167,7 +167,7 @@ int gsi::simulate_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, 
     CUDA_TRY(sc.alloc(&dth, nb * 2 * cy));
     // proof_element without variable terms; theta on the second stream next to pi in the latency regime, as in prove_impl
     rc = theta_pi_fork(
-        ctx, nb * (m + n) * 2 < 32768, "simulate",
+        ctx, nb * (m + n) * 2 < 32768,
         [&] {
           return proof_element<FpOps>(ctx, sc, nb, cy, s.groupA, sv_th, dA, n + xa, nullptr, 0, shared, cx, dT, (size_t)cx, e_th, dth);
         },

@@ -1262,16 +1262,128 @@ int gs_verify_finish(gs_ctx* ctx, int type, size_t count, int nparts, const gs_g
   return GS_OK;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------ randomised verification: the stages both drivers share
+// Time of a Miller product over `nacc` accumulators of S slots: every accumulator pays 62 squarings (~53 M each as
+// executed) next to ~29 M x 68 steps per slot, and the accumulators fill waves of 2 x 148 x 32 lanes
+static double acc_cost(size_t nacc, int S) {
+  const size_t waves = (nacc + 9471) / 9472;
+  return (double)waves * (62.0 * 53.0 + (double)S * 68.0 * 29.0);
+}
+
+// The slots of a randomised check: `walk`, whose G2 side is walked proof by proof; `fix`, the CRS slots (G2 side v_1, v_2
+// or W2: pid 0, 1, 2); `summed`, summed over the proofs (the bucket sums of the batch check), in neither list.
+// k_rand_fold_g1 folds the `all` slots when the statement MSM keeps both coordinates, the `rest` when the commitments are
+// folded first.  `map` (where each slot's fold goes) is the driver's encoding; rand_upload makes the device copies.
+struct rand_slots {
+  std::vector<int> walk, fix, pid, summed, all, rest, map;
+  int *dmap = nullptr, *dwalk = nullptr, *dall = nullptr, *drest = nullptr;
+};
+template <class Summed>
+static rand_slots rand_classify(const verify_shape& s, Summed summed) {
+  const std::vector<uint8_t> kind = slot_kinds(s);
+  rand_slots sl;
+  sl.map.assign(s.K, 0);
+  for (int k = 0; k < s.K; k++) {
+    if (summed(k)) {
+      sl.summed.push_back(k);
+      continue;
+    }
+    if (kind[k] >= gsi::GS_SLOT_FIXED) {
+      sl.fix.push_back(k);
+      sl.pid.push_back(kind[k] - gsi::GS_SLOT_FIXED);
+    } else {
+      sl.walk.push_back(k);
+    }
+    // slots whose G1 side k_verify_assemble writes (everything but the MSM outputs); with the commitments folded first the
+    // (c_i, iota_2(B_i)) slots need no fold either
+    const bool msm_out = k < s.n || (k == s.sB && !s.groupB) || (s.type == 3 && k == s.sT);
+    const bool b_slot = s.groupB && k >= s.sB && k < s.sPi;
+    sl.all.push_back(k);
+    if (!msm_out && !b_slot) sl.rest.push_back(k);
+  }
+  return sl;
+}
+static int rand_upload(gs_ctx* ctx, Scratch& top, rand_slots& sl) {
+  CUDA_TRY(upload(ctx, top, &sl.dmap, sl.map.data(), sl.map.size()));
+  CUDA_TRY(upload(ctx, top, &sl.dwalk, sl.walk.data(), sl.walk.size()));
+  CUDA_TRY(upload(ctx, top, &sl.dall, sl.all.data(), sl.all.size()));
+  CUDA_TRY(upload(ctx, top, &sl.drest, sl.rest.data(), sl.rest.size()));
+  return GS_OK;
+}
+
+// beta, the weight of the G2 sides: rho[2 count] in joint sparse form
+static jsf33 rand_beta(const uint64_t* rho, size_t count) {
+  return make_jsf((uint32_t)rho[2 * count], (uint32_t)(rho[2 * count] >> 32));
+}
+// the weights (sigma_p, tau_p) of proofs [off, off + nprob) on the device, their low 63 bits: below |x|, so a weight is
+// its own first sub-scalar on both groups (bucket sums)
+static int rand_weights(gs_ctx* ctx, Scratch& sc, const uint64_t* rho, size_t off, size_t nprob, uint64_t** drho) {
+  std::vector<uint64_t> w(rho + 2 * off, rho + 2 * (off + nprob));
+  for (uint64_t& x : w) x &= 0x7fffffffffffffffull;
+  CUDA_TRY(upload(ctx, sc, drho, w.data(), w.size()));
+  return GS_OK;
+}
+
+// Proofs per pass: passes of at most `cap` proofs (at most 4 verify_batch_max), equal in size, so that the per-pass
+// fixed costs (bucket-sum chains, product trees, partial last waves) are paid as rarely as possible; 0 if `cap` is 0
+static size_t rand_pass_size(const gs_ctx* ctx, size_t count, size_t cap) {
+  if (cap > 4 * ctx->verify_batch_max) cap = 4 * ctx->verify_batch_max;
+  if (ctx->verify_batch_max < 23680) cap = ctx->verify_batch_max;  // (lowered by a test: several passes on a small batch)
+  if (cap == 0) return 0;
+  const size_t npass = (count + cap - 1) / cap;
+  return (count + npass - 1) / npass;
+}
+
+// From the assembled slots X / Y [2][K][nprob] to the pairs of the folded problem: the G1 side sigma_p X_k.0 + tau_p X_k.1
+// of slot k of proof p goes to X1[p * stride + map[k]] (map[k] < 0: Xfix, the CRS slots of the batch check), the G2 side
+// beta Y_k.0 + Y_k.1 of the i-th walked slot to Y1[p * stride + i].  `shared`: one set of commitments under many equations.
+static int rand_fold(gs_ctx* ctx, Scratch& sc, verify_shape& s, const verify_args& v, size_t nprob, bool shared, const rand_slots& sl,
+                     const uint64_t* drho, const jsf33& beta, g1_aff* X, const g2_aff* Y, int stride, g1_aff* X1, g2_aff* Y1,
+                     g1_aff* Xfix) {
+  if (!shared) {
+    // the commitments are folded BEFORE the statement MSM, which then sums single points: half the scalar products;
+    // its outputs are folded slots already, the (c_i, iota_2(B_i)) slots are the folded bases themselves
+    g1_aff *xfold, *afold;
+    CUDA_TRY(sc.alloc(&xfold, nprob * (size_t)s.nbases));
+    CUDA_TRY(sc.alloc(&afold, nprob * (size_t)(s.groupA ? s.n : 1)));
+    LAUNCH(k_rand_fold_bases, nprob * (size_t)(s.nbases + (s.groupA ? s.n : 0)), s, v, ctx->crs, nprob, drho, xfold, afold,
+           s.groupB ? sl.map[s.sB] : 0, stride, X1);
+    verify_shape sf = s;
+    sf.na = 1;
+    verify_args vf = v;
+    vf.xfold = xfold;
+    vf.afold = afold;
+    vf.fold_map = sl.dmap;
+    vf.fold_Kw = stride;
+    vf.fold_X1 = X1;
+    vf.fold_Xfix = Xfix;
+    const g1_jac* part;
+    int rcm = statement_msm_partials(ctx, sc, sf, vf, nprob, false, &part);
+    if (rcm) return rcm;
+    LAUNCH(k_vmsm_reduce, nprob * (size_t)sf.n_out_owned() * sf.na, sf, vf, part, (g1_aff*)nullptr, nprob);
+    LAUNCH(k_rand_fold_g1, nprob * sl.rest.size(), X, nprob, s.K, drho, sl.drest, (int)sl.rest.size(), sl.dmap, stride, X1, Xfix);
+  } else {
+    // the statement MSM keeps its shared-base tables (both coordinates), every slot is folded afterwards
+    const g1_jac* part;
+    int rcm = statement_msm_partials(ctx, sc, s, v, nprob, true, &part);
+    if (rcm) return rcm;
+    LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
+    LAUNCH(k_rand_fold_g1, nprob * sl.all.size(), X, nprob, s.K, drho, sl.dall, (int)sl.all.size(), sl.dmap, stride, X1, Xfix);
+  }
+  const int Kw = (int)sl.walk.size();
+  LAUNCH(k_rand_fold_g2, nprob * (size_t)Kw, Y, nprob, s.K, beta, sl.dwalk, Kw, Y1, (size_t)stride, (size_t)1);
+  return GS_OK;
+}
+
 // ------------------------------------------------------------------ randomised batch verification: driver
-// slots per Miller accumulator: every accumulator pays 62 squarings (~53 M each as executed) next to ~29 M x 68 steps per slot,
-// and the accumulators fill waves of 2 x 148 x 32 lanes; pick the multiple of 4 that minimises waves x (time per accumulator)
+// slots per Miller accumulator: the multiple of 4 that minimises acc_cost
 static int rand_slots_per_acc(size_t npairs) {
   int best = 8;
   double best_t = 1e300;
   for (int S = 8; S <= 128; S += 4) {
-    const size_t nacc = (npairs + S - 1) / S;
-    const size_t waves = (nacc + 9471) / 9472;
-    const double t = (double)waves * (62.0 * 53.0 + (double)S * 68.0 * 29.0);
+    const double t = acc_cost((npairs + S - 1) / S, S);
     if (t < best_t) {
       best_t = t;
       best = S;
@@ -1283,136 +1395,69 @@ static int rand_slots_per_acc(size_t npairs) {
 static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args, const uint64_t* rho_host,
                            bool shared_x, uint8_t* out_ok_dev) {
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
-  const std::vector<uint8_t> kind_all = slot_kinds(s);
-  // per-proof pairs (G2 side walked) and CRS slots (G1 sides summed over the proofs)
-  std::vector<int> slot_map(s.K), walk_slot, pi_slots, theta_slots;
-  fix_pids fpids;
-  int nfix = 0;
   // a big batch sums its pi and theta slots over the proofs with the bucket method (small ones pair them proof by proof:
   // the bucket kernels are dependent chains that do not shrink with the batch)
   const bool use_pip = count >= ctx->rand_pip_min && ctx->verify_batch_max >= 23680;
-  for (int k = 0; k < s.K; k++) {
-    if (use_pip && k >= s.sPi && k < s.sT) {
-      (k < s.sTh ? pi_slots : theta_slots).push_back(k);
-      slot_map[k] = 0;  // (never looked up: neither an MSM output nor in a fold list)
-      continue;
-    }
-    if (kind_all[k] >= gsi::GS_SLOT_FIXED) {
-      if (nfix >= 8) FAIL(GS_EDIM, "verify_rand: too many CRS slots");
-      fpids.pid[nfix] = kind_all[k] - gsi::GS_SLOT_FIXED;
-      slot_map[k] = -(nfix + 1);
-      nfix++;
-    } else {
-      slot_map[k] = (int)walk_slot.size();
-      walk_slot.push_back(k);
-    }
+  rand_slots sl = rand_classify(s, [&](int k) { return use_pip && k >= s.sPi && k < s.sT; });
+  const int Kw = (int)sl.walk.size(), nfix = (int)sl.fix.size();
+  if (nfix > 8) FAIL(GS_EDIM, "verify_rand: too many CRS slots");
+  // per-proof pairs (G2 side walked) at map 0, 1, ..., CRS slots (G1 sides summed over the proofs) at -1, -2, ...
+  fix_pids fpids;
+  for (int i = 0; i < nfix; i++) {
+    sl.map[sl.fix[i]] = -(i + 1);
+    fpids.pid[i] = sl.pid[i];
   }
-  const int Kw = (int)walk_slot.size();
-  const jsf33 beta = make_jsf((uint32_t)rho_host[2 * count], (uint32_t)(rho_host[2 * count] >> 32));
-  // Passes as large as the line tiles allow (13 KB per pair; half the budget, the slot arrays and tables need room too) and
-  // equal in size: the per-pass fixed costs (bucket-sum chains, product trees, partial last waves) are paid as rarely as
-  // possible -- 65,536 4x4 PPE proofs are ONE pass.
-  size_t pass_cap = ctx->tile_budget / 2 / 13056 / (size_t)(Kw ? Kw : 1);
-  if (pass_cap > 4 * ctx->verify_batch_max) pass_cap = 4 * ctx->verify_batch_max;
-  if (ctx->verify_batch_max < 23680) pass_cap = ctx->verify_batch_max;  // (lowered by a test: several passes on a small batch)
-  if (pass_cap < 1) pass_cap = 1;
-  const size_t npass = (count + pass_cap - 1) / pass_cap;
-  const size_t pass_n = (count + npass - 1) / npass;
+  for (int i = 0; i < Kw; i++) sl.map[sl.walk[i]] = i;
+  std::vector<int> pi_slots, theta_slots;
+  for (int k : sl.summed) (k < s.sTh ? pi_slots : theta_slots).push_back(k);
+  const jsf33 beta = rand_beta(rho_host, count);
+  // Passes as large as the line tiles allow (13 KB per pair; half the budget, the slot arrays and tables need room too):
+  // 65,536 4x4 PPE proofs are ONE pass.
+  size_t pass_n = rand_pass_size(ctx, count, ctx->tile_budget / 2 / 13056 / (size_t)(Kw ? Kw : 1));
+  if (pass_n == 0) pass_n = 1;
+  const size_t npass = (count + pass_n - 1) / pass_n;
   if ((size_t)pass_n * Kw + nfix > ((size_t)1 << 30)) FAIL(GS_EDIM, "verify_rand: statement too large for one pass");
   Scratch top(ctx);
   fp12 *Mall, *Tall;
   g2_aff* Yfix;
-  int *dmap, *dwalk_slot;
+  int* dpi_slots;
   uint8_t* ok1;
   CUDA_TRY(top.alloc(&Mall, npass));
   CUDA_TRY(top.alloc(&Tall, npass + 1));
   CUDA_TRY(top.alloc(&Yfix, 3));
   CUDA_TRY(top.alloc(&ok1, 4));
-  CUDA_TRY(upload(ctx, top, &dmap, slot_map.data(), slot_map.size()));
-  CUDA_TRY(upload(ctx, top, &dwalk_slot, walk_slot.data(), walk_slot.size()));
-  // slots whose G1 side k_verify_assemble writes (everything but the MSM outputs); with the commitments folded first the
-  // (c_i, iota_2(B_i)) slots need no fold either
-  const bool fold_first = !shared_x || count == 1;
-  std::vector<int> all_slots, rest_slots;
-  for (int k = 0; k < s.K; k++) {
-    const bool msm_out = k < s.n || (k == s.sB && !s.groupB) || (type == 3 && k == s.sT);
-    const bool b_slot = s.groupB && k >= s.sB && k < s.sPi;
-    const bool summed = use_pip && k >= s.sPi && k < s.sT;
-    if (!summed) all_slots.push_back(k);
-    if (!msm_out && !b_slot && !summed) rest_slots.push_back(k);
-  }
-  int *dall, *drest, *dpi_slots;
+  if (int rc = rand_upload(ctx, top, sl)) return rc;
   CUDA_TRY(upload(ctx, top, &dpi_slots, pi_slots.data(), pi_slots.size()));
-  CUDA_TRY(upload(ctx, top, &dall, all_slots.data(), all_slots.size()));
-  CUDA_TRY(upload(ctx, top, &drest, rest_slots.data(), rest_slots.size()));
+  const bool shared = shared_x && count > 1;
   // The folded CRS points and the target powers prod_p t_p^tau_p depend on nothing the main stream computes: they run on
   // the second stream (latency-bound kernels: a 66-step scalar multiplication in 3 threads, a product tree), next to the
-  // statement MSM and the line walk.  `side` is waited for before their results are used and before their buffers die.
-  if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-  struct side_stream {
-    gs_ctx* ctx;
-    cudaStream_t main_s;
-    cudaEvent_t ev = nullptr;
-    bool pending = false;
-    int fork() {  // second stream ordered after everything queued on the main stream so far; ctx->stream := second stream
-      if (!ev && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) return 1;
-      cudaEventRecord(ev, main_s);
-      cudaStreamWaitEvent(ctx->stream2, ev, 0);
-      ctx->stream = ctx->stream2;
-      return 0;
-    }
-    void back() {  // ctx->stream := main stream; the side work is pending until join()
-      cudaEventRecord(ev, ctx->stream2);
-      ctx->stream = main_s;
-      pending = true;
-    }
-    void join() {
-      if (pending) cudaStreamWaitEvent(main_s, ev, 0);
-      pending = false;
-    }
-    ~side_stream() {
-      ctx->stream = main_s;
-      join();
-      if (ev) cudaEventDestroy(ev);
-    }
-  } side{ctx, ctx->stream};
-  const bool two = !ctx->profile;  // (per-kernel event times need one stream)
-  if (two && side.fork()) FAIL(GS_ECUDA, "verify_rand: event creation failed");
+  // statement MSM and the line walk.  (Per-kernel event times need one stream.)
+  SideStream side(ctx, !ctx->profile);
+  if (int rc = side.fork()) return rc;
   LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, Yfix);
-  if (two) side.back();
+  if (int rc = side.back()) return rc;
   size_t pass = 0;
   for (size_t off = 0; off < count; off += pass_n, pass++) {
     const size_t nprob = count - off < pass_n ? count - off : pass_n;
     Scratch sc(ctx);
-    struct join_on_exit {  // declared after `sc`, destroyed first: on EVERY exit of the pass (error returns included) the
-      side_stream& s;      // main stream is ordered after the side work before `sc` releases buffers that work still uses
-      ~join_on_exit() { s.join(); }
-    } joined{side};
+    SideJoin joined{side};
     const verify_args v = args_at(s, args, off);
     g1_aff *X, *X1, *Xfix;
     g2_aff *Y, *Y1;
     uint64_t* drho;
-    {  // the low 63 bits of every weight: below |x|, so a weight is its own first sub-scalar on both groups (bucket sums)
-      std::vector<uint64_t> w(rho_host + 2 * off, rho_host + 2 * (off + nprob));
-      for (uint64_t& x : w) x &= 0x7fffffffffffffffull;
-      CUDA_TRY(upload(ctx, sc, &drho, w.data(), w.size()));
-    }
+    if (int rc = rand_weights(ctx, sc, rho_host, off, nprob, &drho)) return rc;
     if (type == GS_PPE) {  // prod_p t_p^tau_p, on the side stream
-      if (two && side.fork()) FAIL(GS_ECUDA, "verify_rand: event creation failed");
-      int rcg = [&]() -> int {
-        fp12* P;
-        CUDA_TRY(sc.alloc(&P, nprob));
-        int rc = gsi::gt_pow64(ctx, (const fp12*)v.target, drho + 1, 2, nprob, P);
-        if (rc) return rc;
-        const fp12* Pr = P;
-        int nch = (int)nprob;
-        rc = gsi::reduce_chunks(ctx, sc, &Pr, 1, &nch, 1, 1);
-        if (rc) return rc;
-        CUDA_TRY(cudaMemcpyAsync(Tall + pass, Pr, sizeof(fp12), cudaMemcpyDeviceToDevice, ctx->stream));
-        return GS_OK;
-      }();
-      if (two) side.back();
-      if (rcg) return rcg;
+      if (int rc = side.fork()) return rc;
+      fp12* P;
+      CUDA_TRY(sc.alloc(&P, nprob));
+      int rc = gsi::gt_pow64(ctx, (const fp12*)v.target, drho + 1, 2, nprob, P);
+      if (rc) return rc;
+      const fp12* Pr = P;
+      int nch = (int)nprob;
+      rc = gsi::reduce_chunks(ctx, sc, &Pr, 1, &nch, 1, 1);
+      if (rc) return rc;
+      CUDA_TRY(cudaMemcpyAsync(Tall + pass, Pr, sizeof(fp12), cudaMemcpyDeviceToDevice, ctx->stream));
+      if ((rc = side.back())) return rc;
     }
     CUDA_TRY(sc.alloc(&X, 2 * (size_t)s.K * nprob));
     CUDA_TRY(sc.alloc(&Y, 2 * (size_t)s.K * nprob));
@@ -1430,71 +1475,36 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
     if (nextra) {
       // bucket sums of the pi / theta slots: they need the assembled slots only, and their kernels are short dependent
       // chains -- on the second stream, next to the statement MSM and the folds
-      if (two && side.fork()) FAIL(GS_ECUDA, "verify_rand: event creation failed");
-      int rcx = [&]() -> int {
-        fr* sv;
-        CUDA_TRY(sc.alloc(&sv, 2 * nprob));
-        LAUNCH(k_rho_to_fr, 2 * nprob, drho, nprob, sv);
-        size_t at = nprob * Kw + nfix;
-        for (size_t t = 0; t < theta_slots.size(); t++, at++) {
-          const int k = theta_slots[t];
-          g1_jac* sum;
+      if (int rc = side.fork()) return rc;
+      fr* sv;
+      CUDA_TRY(sc.alloc(&sv, 2 * nprob));
+      LAUNCH(k_rho_to_fr, 2 * nprob, drho, nprob, sv);
+      size_t at = nprob * Kw + nfix;
+      for (size_t t = 0; t < theta_slots.size(); t++, at++) {
+        const int k = theta_slots[t];  // (theta slot sTh + j pairs with the CRS point j)
+        g1_jac* sum;
+        size_t stride;
+        int rcp = gsi::pippenger_rows<FpOps>(ctx, sc, sv, 1, X + ((size_t)0 * s.K + k) * nprob, nprob, X + ((size_t)1 * s.K + k) * nprob,
+                                              nprob, &sum, &stride, 0, 63);
+        if (rcp) return rcp;
+        LAUNCH_CFG(k_rand_place_theta, 1, 32, 0, sum, Yfix, k - s.sTh, at, X1, Y1);
+      }
+      if (!pi_slots.empty()) {
+        g2_aff* Ypi;
+        CUDA_TRY(sc.alloc(&Ypi, pi_slots.size() * nprob));
+        LAUNCH(k_rand_fold_g2, nprob * pi_slots.size(), Y, nprob, s.K, beta, dpi_slots, (int)pi_slots.size(), Ypi, (size_t)1, nprob);
+        for (size_t t = 0; t < pi_slots.size(); t++, at += 2) {
+          g2_jac* sums;
           size_t stride;
-          int rcp = gsi::pippenger_rows<FpOps>(ctx, sc, sv, 1, X + ((size_t)0 * s.K + k) * nprob, nprob, X + ((size_t)1 * s.K + k) * nprob,
-                                                nprob, &sum, &stride, 0, 63);
+          int rcp = gsi::pippenger_rows<Fp2Ops>(ctx, sc, sv, 2, Ypi + t * nprob, nprob, (const g2_aff*)nullptr, 0, &sums, &stride, 0, 63);
           if (rcp) return rcp;
-          LAUNCH_CFG(k_rand_place_theta, 1, 32, 0, sum, Yfix, (int)(kind_all[k] - gsi::GS_SLOT_FIXED), at, X1, Y1);
+          LAUNCH_CFG(k_rand_place_pi, 32, 32, 0, sums, stride, ctx->crs, pi_slots[t] - s.sPi, at, X1, Y1);
         }
-        if (!pi_slots.empty()) {
-          g2_aff* Ypi;
-          CUDA_TRY(sc.alloc(&Ypi, pi_slots.size() * nprob));
-          LAUNCH(k_rand_fold_g2, nprob * pi_slots.size(), Y, nprob, s.K, beta, dpi_slots, (int)pi_slots.size(), Ypi, (size_t)1, nprob);
-          for (size_t t = 0; t < pi_slots.size(); t++, at += 2) {
-            g2_jac* sums;
-            size_t stride;
-            int rcp = gsi::pippenger_rows<Fp2Ops>(ctx, sc, sv, 2, Ypi + t * nprob, nprob, (const g2_aff*)nullptr, 0, &sums, &stride, 0, 63);
-            if (rcp) return rcp;
-            LAUNCH_CFG(k_rand_place_pi, 32, 32, 0, sums, stride, ctx->crs, pi_slots[t] - s.sPi, at, X1, Y1);
-          }
-        }
-        return GS_OK;
-      }();
-      if (two) side.back();
-      if (rcx) return rcx;
+      }
+      if (int rc = side.back()) return rc;
     }
-    if (fold_first) {
-      // the commitments are folded BEFORE the statement MSM, which then sums single points: half the scalar products;
-      // its outputs are folded slots already, the (c_i, iota_2(B_i)) slots are the folded bases themselves
-      g1_aff *xfold, *afold;
-      CUDA_TRY(sc.alloc(&xfold, nprob * (size_t)s.nbases));
-      CUDA_TRY(sc.alloc(&afold, nprob * (size_t)(s.groupA ? s.n : 1)));
-      LAUNCH(k_rand_fold_bases, nprob * (size_t)(s.nbases + (s.groupA ? s.n : 0)), s, v, ctx->crs, nprob, drho, xfold, afold,
-             s.groupB ? slot_map[s.sB] : 0, Kw, X1);
-      verify_shape sf = s;
-      sf.na = 1;
-      verify_args vf = v;
-      vf.xfold = xfold;
-      vf.afold = afold;
-      vf.fold_map = dmap;
-      vf.fold_Kw = Kw;
-      vf.fold_X1 = X1;
-      vf.fold_Xfix = Xfix;
-      const g1_jac* part;
-      int rcm = statement_msm_partials(ctx, sc, sf, vf, nprob, false, &part);
-      if (rcm) return rcm;
-      LAUNCH(k_vmsm_reduce, nprob * (size_t)sf.n_out_owned() * sf.na, sf, vf, part, (g1_aff*)nullptr, nprob);
-      LAUNCH(k_rand_fold_g1, nprob * rest_slots.size(), X, nprob, s.K, drho, drest, (int)rest_slots.size(), dmap, Kw, X1, Xfix);
-    } else {
-      // one set of commitments under many equations: the statement MSM keeps its shared-base tables (both coordinates),
-      // every slot is folded afterwards
-      const g1_jac* part;
-      int rcm = statement_msm_partials(ctx, sc, s, v, nprob, shared_x, &part);
-      if (rcm) return rcm;
-      LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
-      LAUNCH(k_rand_fold_g1, nprob * all_slots.size(), X, nprob, s.K, drho, dall, (int)all_slots.size(), dmap, Kw, X1, Xfix);
-    }
-    LAUNCH(k_rand_fold_g2, nprob * (size_t)Kw, Y, nprob, s.K, beta, dwalk_slot, Kw, Y1, (size_t)Kw, (size_t)1);
-    side.join();  // the folded CRS points (and, long finished, this pass's target powers)
+    if (int rc = rand_fold(ctx, sc, s, v, nprob, shared, sl, drho, beta, X, Y, Kw, X1, Y1, Xfix)) return rc;
+    if (int rc = side.join()) return rc;  // the folded CRS points (and, long finished, this pass's target powers)
     if (nfix) {
       const int L = 32;
       const size_t nstrips = (nprob + L - 1) / L;
@@ -1534,16 +1544,14 @@ static int verify_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t
 // lines walked once per call, Y1 left the identity), then the Kw walked slots, then identity padding.  Proof p takes the c
 // accumulators p*c .. p*c + c - 1 of S slots each (Kp = c S); c = 1 unless the proofs are few or large.
 static void each_split(size_t nprob, int Kp0, int* S_out, int* c_out) {
-  // as rand_slots_per_acc: waves of 9,472 accumulators x (62 squarings + 68 line steps per slot); at most M4_MAXS = 512
-  // slots per accumulator
+  // at most M4_MAXS = 512 slots per accumulator
   int best_S = 0, best_c = 1;
   double best_t = 1e300;
   for (int c = 1; c <= Kp0; c++) {
     const int S = ((Kp0 + c - 1) / c + 3) / 4 * 4;
     if (S > 512) continue;
     if (S < 8 && c > 1) break;
-    const size_t waves = (nprob * c + 9471) / 9472;
-    const double t = (double)waves * (62.0 * 53.0 + (double)S * 68.0 * 29.0);
+    const double t = acc_cost(nprob * c, S);
     if (t < best_t) {
       best_t = t;
       best_S = S;
@@ -1557,23 +1565,17 @@ static void each_split(size_t nprob, int Kp0, int* S_out, int* c_out) {
 static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args,
                                 const uint64_t* rho_host, bool shared_x, uint8_t* out_ok_dev) {
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
-  const std::vector<uint8_t> kind_all = slot_kinds(s);
-  std::vector<int> slot_map(s.K), walk_slot;
+  rand_slots sl = rand_classify(s, [](int) { return false; });
+  const int Kw = (int)sl.walk.size(), nf = (int)sl.fix.size();
+  if (nf > 4) FAIL(GS_EDIM, "verify_each_rand: too many CRS slots");
   gsi::acc_each each;
-  for (int k = 0; k < s.K; k++)
-    if (kind_all[k] >= gsi::GS_SLOT_FIXED) {
-      if (each.nf >= 4) FAIL(GS_EDIM, "verify_each_rand: too many CRS slots");
-      each.pid[each.nf] = kind_all[k] - gsi::GS_SLOT_FIXED;
-      slot_map[k] = each.nf++;
-    }
-  const int nf = each.nf;
-  for (int k = 0; k < s.K; k++)
-    if (kind_all[k] < gsi::GS_SLOT_FIXED) {
-      slot_map[k] = nf + (int)walk_slot.size();
-      walk_slot.push_back(k);
-    }
-  const int Kw = (int)walk_slot.size();
-  const jsf33 beta = make_jsf((uint32_t)rho_host[2 * count], (uint32_t)(rho_host[2 * count] >> 32));
+  each.nf = nf;
+  for (int i = 0; i < nf; i++) {
+    sl.map[sl.fix[i]] = i;
+    each.pid[i] = sl.pid[i];
+  }
+  for (int i = 0; i < Kw; i++) sl.map[sl.walk[i]] = nf + i;
+  const jsf33 beta = rand_beta(rho_host, count);
   // Passes as large as the line tiles allow (13,056 B per pair), equal in size.  Unlike verify_rand_dev the whole tile
   // budget goes to the tiles: a per-proof pass has no bucket sums or product trees beside them, and 65,536 4x4 PPE proofs
   // (12 pairs each) then run as one pass of 6.9 waves instead of two of 3.5 (4 + 4 waves of k_miller4).
@@ -1581,95 +1583,41 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
   each_split(count, nf + Kw, &S, &c);
   if (S == 0) FAIL(GS_EDIM, "verify_each_rand: statement too large");
   const int Kp = S * c;
-  size_t pass_cap = ctx->tile_budget / 13056 / (size_t)Kp;
-  if (pass_cap > 4 * ctx->verify_batch_max) pass_cap = 4 * ctx->verify_batch_max;
-  if (ctx->verify_batch_max < 23680) pass_cap = ctx->verify_batch_max;  // (lowered by a test: several passes on a small batch)
-  if (pass_cap < 1) FAIL(GS_EDIM, "verify_each_rand: one proof exceeds the tile budget");
-  const size_t npass = (count + pass_cap - 1) / pass_cap;
-  const size_t pass_n = (count + npass - 1) / npass;
+  const size_t pass_n = rand_pass_size(ctx, count, ctx->tile_budget / 13056 / (size_t)Kp);
+  if (pass_n == 0) FAIL(GS_EDIM, "verify_each_rand: one proof exceeds the tile budget");
   if (pass_n * (size_t)Kp > ((size_t)1 << 30)) FAIL(GS_EDIM, "verify_each_rand: statement too large for one pass");
   Scratch top(ctx);
   g2_aff* Yfix;
-  int *dmap, *dwalk_slot, *dall, *drest;
   CUDA_TRY(top.alloc(&Yfix, 3));
-  CUDA_TRY(upload(ctx, top, &dmap, slot_map.data(), slot_map.size()));
-  CUDA_TRY(upload(ctx, top, &dwalk_slot, walk_slot.data(), walk_slot.size()));
-  const bool fold_first = !shared_x || count == 1;
-  std::vector<int> all_slots, rest_slots;
-  for (int k = 0; k < s.K; k++) {
-    const bool msm_out = k < s.n || (k == s.sB && !s.groupB) || (type == 3 && k == s.sT);
-    const bool b_slot = s.groupB && k >= s.sB && k < s.sPi;
-    all_slots.push_back(k);
-    if (!msm_out && !b_slot) rest_slots.push_back(k);
-  }
-  CUDA_TRY(upload(ctx, top, &dall, all_slots.data(), all_slots.size()));
-  CUDA_TRY(upload(ctx, top, &drest, rest_slots.data(), rest_slots.size()));
+  if (int rc = rand_upload(ctx, top, sl)) return rc;
+  const bool shared = shared_x && count > 1;
   // The folded CRS points, their lines and the target powers t_p^tau_p depend on nothing the main stream computes: they
   // run on the second stream, next to the statement MSM and the folds.
-  if (!ctx->stream2) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking));
-  struct side_stream {  // (as in verify_rand_dev)
-    gs_ctx* ctx;
-    cudaStream_t main_s;
-    cudaEvent_t ev = nullptr;
-    bool pending = false;
-    int fork() {
-      if (!ev && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) return 1;
-      cudaEventRecord(ev, main_s);
-      cudaStreamWaitEvent(ctx->stream2, ev, 0);
-      ctx->stream = ctx->stream2;
-      return 0;
-    }
-    void back() {
-      cudaEventRecord(ev, ctx->stream2);
-      ctx->stream = main_s;
-      pending = true;
-    }
-    void join() {
-      if (pending) cudaStreamWaitEvent(main_s, ev, 0);
-      pending = false;
-    }
-    ~side_stream() {
-      ctx->stream = main_s;
-      join();
-      if (ev) cudaEventDestroy(ev);
-    }
-  } side{ctx, ctx->stream};
-  const bool two = !ctx->profile;  // (per-kernel event times need one stream)
+  SideStream side(ctx, !ctx->profile);
   fp2* crs_lines = nullptr;
   if (nf) {
-    if (two && side.fork()) FAIL(GS_ECUDA, "verify_each_rand: event creation failed");
-    int rcl = [&]() -> int {
-      LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, Yfix);
-      return gsi::g2_lines(ctx, top, Yfix, 3, &crs_lines);
-    }();
-    if (two) side.back();
-    if (rcl) return rcl;
+    if (int rc = side.fork()) return rc;
+    LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, Yfix);
+    if (int rc = gsi::g2_lines(ctx, top, Yfix, 3, &crs_lines)) return rc;
+    if (int rc = side.back()) return rc;
   }
   each.pts = Yfix;
   each.acc_stride = c;
   for (size_t off = 0; off < count; off += pass_n) {
     const size_t nprob = count - off < pass_n ? count - off : pass_n;
     Scratch sc(ctx);
-    struct join_on_exit {  // declared after `sc`, destroyed first (see verify_rand_dev)
-      side_stream& s;
-      ~join_on_exit() { s.join(); }
-    } joined{side};
+    SideJoin joined{side};
     const verify_args v = args_at(s, args, off);
     g1_aff *X, *X1;
     g2_aff *Y, *Y1;
     uint64_t* drho;
     fp12 *M, *want = nullptr;
-    {  // the low 63 bits of every weight (as verify_rand_dev)
-      std::vector<uint64_t> w(rho_host + 2 * off, rho_host + 2 * (off + nprob));
-      for (uint64_t& x : w) x &= 0x7fffffffffffffffull;
-      CUDA_TRY(upload(ctx, sc, &drho, w.data(), w.size()));
-    }
+    if (int rc = rand_weights(ctx, sc, rho_host, off, nprob, &drho)) return rc;
     if (type == GS_PPE) {  // t_p^tau_p, on the side stream
       CUDA_TRY(sc.alloc(&want, nprob));
-      if (two && side.fork()) FAIL(GS_ECUDA, "verify_each_rand: event creation failed");
-      int rcg = gsi::gt_pow64(ctx, (const fp12*)v.target, drho + 1, 2, nprob, want);
-      if (two) side.back();
-      if (rcg) return rcg;
+      if (int rc = side.fork()) return rc;
+      if (int rc = gsi::gt_pow64(ctx, (const fp12*)v.target, drho + 1, 2, nprob, want)) return rc;
+      if (int rc = side.back()) return rc;
     }
     const size_t Ktot = nprob * (size_t)Kp;
     CUDA_TRY(sc.alloc(&X, 2 * (size_t)s.K * nprob));
@@ -1680,36 +1628,8 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
     CUDA_TRY(cudaMemsetAsync(X1, 0, Ktot * sizeof(g1_aff), ctx->stream));  // padding and the CRS pairs' G2 sides: identities
     CUDA_TRY(cudaMemsetAsync(Y1, 0, Ktot * sizeof(g2_aff), ctx->stream));
     LAUNCH(k_verify_assemble, nprob * (size_t)s.K, s, v, ctx->crs, X, Y, nprob);
-    if (fold_first) {  // as verify_rand_dev: commitments folded before the statement MSM
-      g1_aff *xfold, *afold;
-      CUDA_TRY(sc.alloc(&xfold, nprob * (size_t)s.nbases));
-      CUDA_TRY(sc.alloc(&afold, nprob * (size_t)(s.groupA ? s.n : 1)));
-      LAUNCH(k_rand_fold_bases, nprob * (size_t)(s.nbases + (s.groupA ? s.n : 0)), s, v, ctx->crs, nprob, drho, xfold, afold,
-             s.groupB ? slot_map[s.sB] : 0, Kp, X1);
-      verify_shape sf = s;
-      sf.na = 1;
-      verify_args vf = v;
-      vf.xfold = xfold;
-      vf.afold = afold;
-      vf.fold_map = dmap;
-      vf.fold_Kw = Kp;
-      vf.fold_X1 = X1;
-      const g1_jac* part;
-      int rcm = statement_msm_partials(ctx, sc, sf, vf, nprob, false, &part);
-      if (rcm) return rcm;
-      LAUNCH(k_vmsm_reduce, nprob * (size_t)sf.n_out_owned() * sf.na, sf, vf, part, (g1_aff*)nullptr, nprob);
-      LAUNCH(k_rand_fold_g1, nprob * rest_slots.size(), X, nprob, s.K, drho, drest, (int)rest_slots.size(), dmap, Kp, X1,
-             (g1_aff*)nullptr);
-    } else {  // one set of commitments under many equations: shared-base tables, every slot folded afterwards
-      const g1_jac* part;
-      int rcm = statement_msm_partials(ctx, sc, s, v, nprob, shared_x, &part);
-      if (rcm) return rcm;
-      LAUNCH(k_vmsm_reduce, nprob * (size_t)s.n_out_owned() * s.na, s, v, part, X, nprob);
-      LAUNCH(k_rand_fold_g1, nprob * all_slots.size(), X, nprob, s.K, drho, dall, (int)all_slots.size(), dmap, Kp, X1,
-             (g1_aff*)nullptr);
-    }
-    LAUNCH(k_rand_fold_g2, nprob * (size_t)Kw, Y, nprob, s.K, beta, dwalk_slot, Kw, Y1 + nf, (size_t)Kp, (size_t)1);
-    side.join();  // the folded CRS points and their lines, this pass's target powers
+    if (int rc = rand_fold(ctx, sc, s, v, nprob, shared, sl, drho, beta, X, Y, Kp, X1, Y1 + nf, nullptr)) return rc;
+    if (int rc = side.join()) return rc;  // the folded CRS points and their lines, this pass's target powers
     each.F = M;
     each.lines = crs_lines;
     int rc = gsi::run_pairing_product(ctx, sc, X1, Y1, 1, (int)Ktot, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1, S, &each);
@@ -1732,6 +1652,25 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
   return GS_OK;
 }
 
+// gs_verify_batch_rand / gs_verify_each_rand past their checks: the host arrays uploaded, the driver, `nout` verdict bytes
+// copied back
+static int rand_host(gs_ctx* ctx, decltype(&verify_rand_dev) driver, int type, size_t count, size_t m, size_t n, const verify_args& h,
+                     const uint64_t* rho, uint8_t* out, size_t nout) {
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  Scratch sc(ctx);
+  verify_args d;
+  uint8_t* dok;
+  if (int rc = upload_args(ctx, sc, make_verify_shape(type, (int)m, (int)n), h, 0, count, &d)) return rc;
+  CUDA_TRY(sc.alloc(&dok, nout));
+  int rc = driver(ctx, type, count, m, n, d, rho, same_rows(h.xcoms, count, m * sizeof(gs_com1)), dok);
+  if (rc) return rc;
+  CUDA_TRY(cudaMemcpyAsync(out, dok, nout, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  return GS_OK;
+}
+
+extern "C" {
+
 int gs_verify_batch_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                          const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                          const gs_com1* theta, const uint64_t* rho, uint8_t* out_all_ok) {
@@ -1743,17 +1682,7 @@ int gs_verify_batch_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n
     return GS_OK;
   }
   if (int rc = check_lists(ctx, m, n, inputs_set(h) && rho)) return rc;
-  CUDA_TRY(cudaSetDevice(ctx->device));
-  Scratch sc(ctx);
-  verify_args d;
-  uint8_t* dok;
-  if (int rc = upload_args(ctx, sc, make_verify_shape(type, (int)m, (int)n), h, 0, count, &d)) return rc;
-  CUDA_TRY(sc.alloc(&dok, 4));
-  int rc = verify_rand_dev(ctx, type, count, m, n, d, rho, same_rows(xcoms, count, m * sizeof(gs_com1)), dok);
-  if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(out_all_ok, dok, 1, cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  return GS_OK;
+  return rand_host(ctx, verify_rand_dev, type, count, m, n, h, rho, out_all_ok, 1);
 }
 
 int gs_verify_batch_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
@@ -1775,17 +1704,7 @@ int gs_verify_each_rand(gs_ctx* ctx, int type, size_t count, size_t m, size_t n,
   if (count == 0) return GS_OK;
   if (!out_ok) return GS_EARG;
   if (int rc = check_lists(ctx, m, n, inputs_set(h) && rho)) return rc;
-  CUDA_TRY(cudaSetDevice(ctx->device));
-  Scratch sc(ctx);
-  verify_args d;
-  uint8_t* dok;
-  if (int rc = upload_args(ctx, sc, make_verify_shape(type, (int)m, (int)n), h, 0, count, &d)) return rc;
-  CUDA_TRY(sc.alloc(&dok, count));
-  int rc = verify_each_rand_dev(ctx, type, count, m, n, d, rho, same_rows(xcoms, count, m * sizeof(gs_com1)), dok);
-  if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(out_ok, dok, count, cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  return GS_OK;
+  return rand_host(ctx, verify_each_rand_dev, type, count, m, n, h, rho, out_ok, count);
 }
 
 int gs_verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
