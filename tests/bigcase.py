@@ -63,6 +63,7 @@ class Case:
             for row in gam:
                 row[1] = row[2] = row[0]
             gam[0][3], gam[m - 1][3] = 1, R - 1
+        self.xs, self.ys, self.a, self.b, self.gam = xs, ys, a, b, gam     # the discrete logs (tests/entry_ref.py)
         self.A, self.B = _enc_side1(crs, ty, a), _enc_side2(crs, ty, b)
         self.X, self.Y = _enc_side1(crs, ty, xs), _enc_side2(crs, ty, ys)
         self.G = frmat_b(gam)
@@ -94,6 +95,7 @@ class Statement:
         b = [fr_list(rng, m) for _ in range(E)]
         gam = [[fr_list(rng, n) for _ in range(m)] for _ in range(E)]
         flat = lambda rows: [x for r in rows for x in r]
+        self.xs, self.ys, self.a, self.b, self.gam = xs, ys, a, b, gam
         self.X, self.Y = _enc_side1(crs, ty, xs), _enc_side2(crs, ty, ys)
         self.A, self.B = _enc_side1(crs, ty, flat(a)), _enc_side2(crs, ty, flat(b))     # [E][n], [E][m]
         self.G = b"".join(frmat_b(g) for g in gam)

@@ -56,7 +56,7 @@ class ZkCase:
         self.B, self.Y = b"".join(g2s[:E * m]), b"".join(g2s[E * m:E * (m + n)])
         self.Q, self.negQ = g2s[E * (m + n):E * (m + n + K)], g2s[E * (m + n + K):]
         self.G = b"".join(frmat_b(g) for g in gam)
-        self.gam = gam
+        self.gam, self.xs, self.ys = gam, xs, ys
         self.xr, self.yr = fr_list(rng, E * (m + K) * 2), fr_list(rng, E * n * 2)
         self.Tr, self.Lr = fr_list(rng, E * 4), fr_list(rng, E * K * 2)
 
