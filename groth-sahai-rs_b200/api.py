@@ -508,6 +508,21 @@ def zk_simulate_batch(statements, crs: CRS, key: SimulationKey, rng) -> List[ZkP
     return _zk_proofs(out, draws, m, n, K, False)
 
 
+def _zk_verify_arrays(statements, proofs, name):
+    """(m, n, K, the eleven arrays of gs_zk_ppe_verify_batch) of a non-empty batch with one proof per statement, shapes
+    checked"""
+    m, n, K, arrays = _zk_statement_arrays(statements, name)
+    for p in proofs:
+        if len(p.xcoms.coms) != m + K or len(p.ycoms.coms) != n or len(p.lin) != K or len(p.ppe.pi) != 2 or \
+                len(p.ppe.theta) != 2 or any(len(e.pi) != 2 or len(e.theta) != 1 for e in p.lin):
+            raise ValueError(f"{name}: a proof does not match the statements' shape (m, n, K)")
+    cat = lambda f: b"".join(f(p) for p in proofs)
+    return m, n, K, (*arrays, cat(lambda p: b"".join(p.xcoms.coms)), cat(lambda p: b"".join(p.ycoms.coms)),
+                     cat(lambda p: b"".join(p.ppe.pi)), cat(lambda p: b"".join(p.ppe.theta)),
+                     cat(lambda p: b"".join(b"".join(e.pi) for e in p.lin)),
+                     cat(lambda p: b"".join(b"".join(e.theta) for e in p.lin)))
+
+
 def zk_verify_batch(statements, proofs, crs: CRS) -> List[bool]:
     """Verdicts of many (ZkPPE, ZkPPEProof) pairs of one shape in one GPU pass (gs_zk_ppe_verify_batch): a statement is
     accepted iff PPE' and every Z_k - delta P_k = O verify, with delta's commitment W2 taken from `crs`."""
@@ -515,16 +530,23 @@ def zk_verify_batch(statements, proofs, crs: CRS) -> List[bool]:
         raise ValueError("zk_verify_batch: one proof per statement")
     if not statements:
         return []
-    m, n, K, arrays = _zk_statement_arrays(statements, "zk_verify_batch")
-    for p in proofs:
-        if len(p.xcoms.coms) != m + K or len(p.ycoms.coms) != n or len(p.lin) != K or len(p.ppe.pi) != 2 or \
-                len(p.ppe.theta) != 2 or any(len(e.pi) != 2 or len(e.theta) != 1 for e in p.lin):
-            raise ValueError("zk_verify_batch: a proof does not match the statements' shape (m, n, K)")
-    cat = lambda f: b"".join(f(p) for p in proofs)
-    ok = crs._use().zk_ppe_verify_batch(
-        len(statements), m, n, K, *arrays, cat(lambda p: b"".join(p.xcoms.coms)), cat(lambda p: b"".join(p.ycoms.coms)),
-        cat(lambda p: b"".join(p.ppe.pi)), cat(lambda p: b"".join(p.ppe.theta)),
-        cat(lambda p: b"".join(b"".join(e.pi) for e in p.lin)), cat(lambda p: b"".join(b"".join(e.theta) for e in p.lin)))
+    m, n, K, arrays = _zk_verify_arrays(statements, proofs, "zk_verify_batch")
+    ok = crs._use().zk_ppe_verify_batch(len(statements), m, n, K, *arrays)
+    return [b == 1 for b in ok]
+
+
+def zk_verify_each_randomized(statements, proofs, crs: CRS, rho: bytes = None) -> List[bool]:
+    """Per-statement verdicts of many (ZkPPE, ZkPPEProof) pairs of one shape at close to the cost of one equation (opt-in):
+    PPE' and the K equations Z_k - delta P_k = O are folded, each with random weights of its own, into one pairing product
+    and ONE final exponentiation per statement (gs_zk_ppe_verify_each_rand).  A bad statement is accepted with probability
+    <= 2^-62 over `rho` (2*count*(1 + K) + 1 64-bit words, drawn from the OS CSPRNG when not given), each statement on its
+    own.  Inputs must be group members (deserialised values are)."""
+    if len(proofs) != len(statements):
+        raise ValueError("zk_verify_each_randomized: one proof per statement")
+    if not statements:
+        return []
+    m, n, K, arrays = _zk_verify_arrays(statements, proofs, "zk_verify_each_randomized")
+    ok = crs._use().zk_ppe_verify_each_rand(len(statements), m, n, K, *arrays, rho=rho)
     return [b == 1 for b in ok]
 
 

@@ -383,6 +383,15 @@ int sim_key_check(gs_ctx* ctx, const gs_fr* tkey);
 int verify_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                const gs_fr* gamma, const void* target, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
                const gs_com1* theta, bool shared_y, uint8_t* out_ok_dev);
+// verify.cu: gs_zk_ppe_verify_each_rand past its checks and uploads, device arrays of `count` statements: PPE' (m = the m + K
+// x-variables, n) and the count * K equations L_k (MSMEG1, 1 x 1, y-commitment W2); out_ok_dev[i] = the randomised verdict
+// of statement i with weights rho_ppe[2i], rho_ppe[2i + 1] (PPE'), rho_lin[2(iK + k)], rho_lin[2(iK + k) + 1] (L_k) and
+// beta from *rho_beta (host words)
+int zk_each_rand_dev(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts, const gs_g2* b_consts,
+                     const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                     const gs_g1* lin_a, const gs_fr* lin_b, const gs_fr* lin_gamma, const gs_g1* lin_target, const gs_com1* lin_xcoms,
+                     const gs_com2* lin_ycoms, const gs_com2* lin_pi, const gs_com1* lin_theta, const uint64_t* rho_ppe,
+                     const uint64_t* rho_lin, const uint64_t* rho_beta, uint8_t* out_ok_dev);
 
 // extract.cu: *all_identity = (coms[i].1 - key coms[i].0 is the identity for every i < n), n DEVICE commitments (k_extract)
 template <class F>

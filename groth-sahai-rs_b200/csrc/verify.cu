@@ -1,5 +1,7 @@
 // Verifiable::verify for the four equation types (src/verifier.rs:23-157): slot assembly, the G1-side
 // statement MSM (re-association of verifier.rs:39-42, SURVEY.md §8a), then the pairing-product pipeline.
+#include <algorithm>
+
 #include "batchinv.cuh"
 #include "ctx.h"
 #include "endo.cuh"
@@ -788,6 +790,39 @@ __global__ void k_each_chunk_major(const fp12* __restrict__ M, fp12* __restrict_
   F[id] = M[p * c + j];
 }
 
+// ---- randomised per-statement verification of zk PPEs (gs_zk_ppe_verify_each_rand): statement i's pairs are
+// X1 / Y1 [i*Kp + .].  thread -> (i, r): the G1 side of the statement's CRS pair r (0: v_1, 2: W2) gets the folds of its
+// K L_k's slots with that CRS point (XfixL[f*nprob*K + i*K + k], lin_pid.pid[f]); pair 0 already holds PPE' theta_0's.
+// The threads also copy the L_k's Kl walked pairs (X1L / Y1L [(i*K + k)*Kl + j], j = r/2, r/2 + 2, ...) to pairs
+// at_lin + k*Kl + j.  All 128 threads reach the block-wide inversion.
+__global__ void __launch_bounds__(128) k_zk_rand_place(size_t nprob, int K, int Kp, int at_lin, const g1_aff* __restrict__ X1L,
+                                                       const g2_aff* __restrict__ Y1L, int Kl, const g1_aff* __restrict__ XfixL,
+                                                       fix_pids lin_pid, int nfl, g1_aff* __restrict__ X1, g2_aff* __restrict__ Y1) {
+  __shared__ fp sm[2 * 128];
+  const size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const bool active = id < nprob * 2;
+  const size_t i = active ? id % nprob : 0;
+  const int r = active ? 2 * (int)(id / nprob) : 0;
+  g1_jac acc;
+  acc.set_inf();
+  if (active) {
+    const size_t nl = nprob * K;
+    if (r == 0) acc.from_affine(X1[i * Kp]);
+    for (int k = 0; k < K; k++) {
+      const size_t q = i * K + k;
+      for (int f = 0; f < nfl; f++)
+        if (lin_pid.pid[f] == r) g1_jac::add_mixed(acc, acc, XfixL[f * nl + q]);
+      for (int j = r / 2; j < Kl; j += 2) {
+        X1[i * Kp + at_lin + k * Kl + j] = X1L[q * Kl + j];
+        Y1[i * Kp + at_lin + k * Kl + j] = Y1L[q * Kl + j];
+      }
+    }
+  }
+  g1_aff out;
+  block_to_affine<128>(out, acc, sm);
+  if (active) X1[i * Kp + r] = out;
+}
+
 }  // namespace gs
 
 
@@ -1562,6 +1597,40 @@ static void each_split(size_t nprob, int Kp0, int* S_out, int* c_out) {
   *c_out = best_c;
 }
 
+// The folded CRS points of beta (Yfix, 3 of them, owned by `top`) and their lines, on the side stream
+static int each_crs_points(gs_ctx* ctx, Scratch& top, SideStream& side, const jsf33& beta, g2_aff** Yfix, fp2** lines) {
+  CUDA_TRY(top.alloc(Yfix, 3));
+  if (int rc = side.fork()) return rc;
+  LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, *Yfix);
+  if (int rc = gsi::g2_lines(ctx, top, *Yfix, 3, lines)) return rc;
+  return side.back();
+}
+
+// The Miller products of a pass of nprob proofs (c accumulators of S pairs each, `each`), their final exponentiations and
+// the verdicts out_ok_dev[p] = (FE(product of proof p) == want[p]) (want null: 1)
+static int each_finish(gs_ctx* ctx, Scratch& sc, const g1_aff* X1, const g2_aff* Y1, size_t nprob, int S, int c, gsi::acc_each& each,
+                       const fp12* want, uint8_t* out_ok_dev) {
+  fp12* M;
+  CUDA_TRY(sc.alloc(&M, nprob * (size_t)c));
+  each.F = M;
+  int rc = gsi::run_pairing_product(ctx, sc, X1, Y1, 1, (int)(nprob * (size_t)S * c), nullptr, nullptr, nullptr, nullptr, nullptr,
+                                    nullptr, 1, S, &each);
+  if (rc) return rc;
+  const fp12* Fr = M;
+  int nch = c;
+  if (c > 1) {
+    fp12* F;
+    CUDA_TRY(sc.alloc(&F, nprob * (size_t)c));
+    LAUNCH(k_each_chunk_major, nprob * (size_t)c, M, F, nprob, c);
+    Fr = F;
+    if (nch > 12) {
+      rc = gsi::reduce_chunks(ctx, sc, &Fr, nprob, &nch, 12, 1);
+      if (rc) return rc;
+    }
+  }
+  return gsi::launch_final_exp(ctx, Fr, nprob, nch, nullptr, out_ok_dev, want, 1);
+}
+
 static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const verify_args& args,
                                 const uint64_t* rho_host, bool shared_x, uint8_t* out_ok_dev) {
   verify_shape s = make_verify_shape(type, (int)m, (int)n);
@@ -1587,21 +1656,17 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
   if (pass_n == 0) FAIL(GS_EDIM, "verify_each_rand: one proof exceeds the tile budget");
   if (pass_n * (size_t)Kp > ((size_t)1 << 30)) FAIL(GS_EDIM, "verify_each_rand: statement too large for one pass");
   Scratch top(ctx);
-  g2_aff* Yfix;
-  CUDA_TRY(top.alloc(&Yfix, 3));
   if (int rc = rand_upload(ctx, top, sl)) return rc;
   const bool shared = shared_x && count > 1;
   // The folded CRS points, their lines and the target powers t_p^tau_p depend on nothing the main stream computes: they
   // run on the second stream, next to the statement MSM and the folds.
   SideStream side(ctx, !ctx->profile);
+  g2_aff* Yfix = nullptr;
   fp2* crs_lines = nullptr;
-  if (nf) {
-    if (int rc = side.fork()) return rc;
-    LAUNCH_CFG(k_rand_fold_crs, 3, 32, 0, ctx->crs, beta, Yfix);
-    if (int rc = gsi::g2_lines(ctx, top, Yfix, 3, &crs_lines)) return rc;
-    if (int rc = side.back()) return rc;
-  }
+  if (nf)
+    if (int rc = each_crs_points(ctx, top, side, beta, &Yfix, &crs_lines)) return rc;
   each.pts = Yfix;
+  each.lines = crs_lines;
   each.acc_stride = c;
   for (size_t off = 0; off < count; off += pass_n) {
     const size_t nprob = count - off < pass_n ? count - off : pass_n;
@@ -1611,7 +1676,7 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
     g1_aff *X, *X1;
     g2_aff *Y, *Y1;
     uint64_t* drho;
-    fp12 *M, *want = nullptr;
+    fp12* want = nullptr;
     if (int rc = rand_weights(ctx, sc, rho_host, off, nprob, &drho)) return rc;
     if (type == GS_PPE) {  // t_p^tau_p, on the side stream
       CUDA_TRY(sc.alloc(&want, nprob));
@@ -1624,30 +1689,106 @@ static int verify_each_rand_dev(gs_ctx* ctx, int type, size_t count, size_t m, s
     CUDA_TRY(sc.alloc(&Y, 2 * (size_t)s.K * nprob));
     CUDA_TRY(sc.alloc(&X1, Ktot));
     CUDA_TRY(sc.alloc(&Y1, Ktot));
-    CUDA_TRY(sc.alloc(&M, nprob * (size_t)c));
     CUDA_TRY(cudaMemsetAsync(X1, 0, Ktot * sizeof(g1_aff), ctx->stream));  // padding and the CRS pairs' G2 sides: identities
     CUDA_TRY(cudaMemsetAsync(Y1, 0, Ktot * sizeof(g2_aff), ctx->stream));
     LAUNCH(k_verify_assemble, nprob * (size_t)s.K, s, v, ctx->crs, X, Y, nprob);
     if (int rc = rand_fold(ctx, sc, s, v, nprob, shared, sl, drho, beta, X, Y, Kp, X1, Y1 + nf, nullptr)) return rc;
     if (int rc = side.join()) return rc;  // the folded CRS points and their lines, this pass's target powers
-    each.F = M;
-    each.lines = crs_lines;
-    int rc = gsi::run_pairing_product(ctx, sc, X1, Y1, 1, (int)Ktot, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 1, S, &each);
-    if (rc) return rc;
-    const fp12* Fr = M;
-    int nch = c;
-    if (c > 1) {
-      fp12* F;
-      CUDA_TRY(sc.alloc(&F, nprob * (size_t)c));
-      LAUNCH(k_each_chunk_major, nprob * (size_t)c, M, F, nprob, c);
-      Fr = F;
-      if (nch > 12) {
-        rc = gsi::reduce_chunks(ctx, sc, &Fr, nprob, &nch, 12, 1);
-        if (rc) return rc;
-      }
-    }
-    rc = gsi::launch_final_exp(ctx, Fr, nprob, nch, nullptr, out_ok_dev + off, want, 1);
-    if (rc) return rc;
+    if (int rc = each_finish(ctx, sc, X1, Y1, nprob, S, c, each, want, out_ok_dev + off)) return rc;
+  }
+  return GS_OK;
+}
+
+// ------------------------------------------------------------------ randomised per-statement verification of zk PPEs
+// (gs_zk_ppe_verify_each_rand).  Statement i is PPE' (target 1) and its K equations L_k (target O, iota_T(O) = 1).  Every
+// equation e has weights of its own, (sigma_e, tau_e), the call one beta; each equation's slots are folded as
+// verify_each_rand_dev folds them, and all folded pairs of the statement go into ONE Miller product:
+//     accept i  iff  FE( prod_e prod_k e( sigma_e X_k.0 + tau_e X_k.1 ,  beta Y_k.0 + Y_k.1 ) ) == 1.
+// A statement the exact verifier rejects has some equation with a non-zero error matrix E^(e) and passes only if
+// sum_e (sigma_e beta E00 + sigma_e E01 + tau_e beta E10 + tau_e E11) = 0: a non-zero polynomial of degree 2, probability
+// <= 2^-62 over 63-bit weights.  The weights must be independent per equation: with shared ones, errors +D on PPE' theta_0
+// and -D on L_k's theta (both paired with v_1) cancel.
+// By bilinearity every slot of the statement whose G2 side is the same CRS point becomes ONE pair (the G1 sides summed):
+// statement i's pairs are [i*Kp + .] = (v_1: PPE' theta_0 + the L_k's theta), (v_2: PPE' theta_1), (W2: the L_k's d, b c
+// and target slots), then PPE''s walked slots, then the two walked pi slots of every L_k, then identity padding.  At
+// m = n = 4, K = 1 that is 3 + 13 = 16 pairs, one accumulator.  L_k's d-slot, which slot_kinds marks walked, is W2 here.
+int gsi::zk_each_rand_dev(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts, const gs_g2* b_consts,
+                          const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                          const gs_g1* lin_a, const gs_fr* lin_b, const gs_fr* lin_gamma, const gs_g1* lin_target,
+                          const gs_com1* lin_xcoms, const gs_com2* lin_ycoms, const gs_com2* lin_pi, const gs_com1* lin_theta,
+                          const uint64_t* rho_ppe, const uint64_t* rho_lin, const uint64_t* rho_beta, uint8_t* out_ok_dev) {
+  verify_shape sp = make_verify_shape(GS_PPE, (int)m, (int)n), sl = make_verify_shape(GS_MSMEG1, 1, 1);
+  const verify_args ap = args_of(a_consts, b_consts, gamma, nullptr, xcoms, ycoms, pi, theta);
+  const verify_args al = args_of(lin_a, lin_b, lin_gamma, lin_target, lin_xcoms, lin_ycoms, lin_pi, lin_theta);
+  constexpr int nf = 3;  // the CRS pairs, pid 0, 1, 2
+  // PPE': theta_j (CRS pid j) folds straight into pair j, the walked slots into pairs nf, nf + 1, ...
+  rand_slots slp = rand_classify(sp, [](int) { return false; });
+  const int KwP = (int)slp.walk.size();
+  for (size_t f = 0; f < slp.fix.size(); f++) slp.map[slp.fix[f]] = slp.pid[f];
+  for (int i = 0; i < KwP; i++) slp.map[slp.walk[i]] = nf + i;
+  // L_k: the d-slot joins the W2 slots; all CRS slots to XfixL (-1, -2, ...), the walked pi slots to pairs 0, 1 of its own
+  rand_slots sll = rand_classify(sl, [](int) { return false; });
+  sll.walk.erase(std::find(sll.walk.begin(), sll.walk.end(), 0));
+  sll.fix.push_back(0);
+  sll.pid.push_back(2);
+  const int Kl = (int)sll.walk.size(), nfl = (int)sll.fix.size();
+  fix_pids lin_pid;
+  for (int f = 0; f < nfl; f++) {
+    sll.map[sll.fix[f]] = -(f + 1);
+    lin_pid.pid[f] = sll.pid[f];
+  }
+  for (int i = 0; i < Kl; i++) sll.map[sll.walk[i]] = i;
+  gsi::acc_each each;
+  each.nf = nf;
+  for (int f = 0; f < nf; f++) each.pid[f] = f;
+  const jsf33 beta = rand_beta(rho_beta, 0);
+  const size_t at_lin = nf + (size_t)KwP, Kpair = at_lin + K * (size_t)Kl;
+  int S, c;
+  each_split(count, (int)Kpair, &S, &c);
+  if (S == 0) FAIL(GS_EDIM, "zk_ppe_verify_each_rand: statement too large");
+  const int Kp = S * c;
+  const size_t pass_n = rand_pass_size(ctx, count, ctx->tile_budget / 13056 / (size_t)Kp);
+  if (pass_n == 0) FAIL(GS_EDIM, "zk_ppe_verify_each_rand: one statement exceeds the tile budget");
+  if (pass_n * (size_t)Kp > ((size_t)1 << 30)) FAIL(GS_EDIM, "zk_ppe_verify_each_rand: statement too large for one pass");
+  Scratch top(ctx);
+  if (int rc = rand_upload(ctx, top, slp)) return rc;
+  if (int rc = rand_upload(ctx, top, sll)) return rc;
+  SideStream side(ctx, !ctx->profile);
+  g2_aff* Yfix;
+  fp2* crs_lines;
+  if (int rc = each_crs_points(ctx, top, side, beta, &Yfix, &crs_lines)) return rc;
+  each.pts = Yfix;
+  each.lines = crs_lines;
+  each.acc_stride = c;
+  for (size_t off = 0; off < count; off += pass_n) {
+    const size_t nprob = count - off < pass_n ? count - off : pass_n, nl = nprob * K;
+    Scratch sc(ctx);
+    SideJoin joined{side};
+    const verify_args vp = args_at(sp, ap, off), vl = args_at(sl, al, off * K);
+    g1_aff *XP, *XL, *X1, *X1L, *XfixL;
+    g2_aff *YP, *YL, *Y1, *Y1L;
+    uint64_t *drp, *drl;
+    if (int rc = rand_weights(ctx, sc, rho_ppe, off, nprob, &drp)) return rc;
+    if (int rc = rand_weights(ctx, sc, rho_lin, off * K, nl, &drl)) return rc;
+    const size_t Ktot = nprob * (size_t)Kp;
+    CUDA_TRY(sc.alloc(&XP, 2 * (size_t)sp.K * nprob));
+    CUDA_TRY(sc.alloc(&YP, 2 * (size_t)sp.K * nprob));
+    CUDA_TRY(sc.alloc(&XL, 2 * (size_t)sl.K * nl));
+    CUDA_TRY(sc.alloc(&YL, 2 * (size_t)sl.K * nl));
+    CUDA_TRY(sc.alloc(&X1, Ktot));
+    CUDA_TRY(sc.alloc(&Y1, Ktot));
+    CUDA_TRY(sc.alloc(&X1L, nl * Kl));
+    CUDA_TRY(sc.alloc(&Y1L, nl * Kl));
+    CUDA_TRY(sc.alloc(&XfixL, nl * nfl));
+    CUDA_TRY(cudaMemsetAsync(X1, 0, Ktot * sizeof(g1_aff), ctx->stream));  // padding and the CRS pairs' G2 sides: identities
+    CUDA_TRY(cudaMemsetAsync(Y1, 0, Ktot * sizeof(g2_aff), ctx->stream));
+    LAUNCH(k_verify_assemble, nprob * (size_t)sp.K, sp, vp, ctx->crs, XP, YP, nprob);
+    LAUNCH(k_verify_assemble, nl * (size_t)sl.K, sl, vl, ctx->crs, XL, YL, nl);
+    if (int rc = rand_fold(ctx, sc, sp, vp, nprob, false, slp, drp, beta, XP, YP, Kp, X1, Y1 + nf, nullptr)) return rc;
+    if (int rc = rand_fold(ctx, sc, sl, vl, nl, false, sll, drl, beta, XL, YL, Kl, X1L, Y1L, XfixL)) return rc;
+    LAUNCH(k_zk_rand_place, nprob * 2, nprob, (int)K, Kp, (int)at_lin, X1L, Y1L, Kl, XfixL, lin_pid, nfl, X1, Y1);
+    if (int rc = side.join()) return rc;  // the folded CRS points and their lines
+    if (int rc = each_finish(ctx, sc, X1, Y1, nprob, S, c, each, nullptr, out_ok_dev + off)) return rc;
   }
   return GS_OK;
 }

@@ -6,8 +6,9 @@
 // scalar y-variable delta has the FIXED commitment W2 = 1 W2 + 0 v[0], rebuilt by the verifier from its CRS.  Under a
 // binding CRS W2 binds delta = 1, so Z_k = P_k and PPE' is the original equation; under a hiding CRS W2 = t2 v[0] is also
 // the commitment of delta = 0 with randomness t2, which is how the simulator proves L_k with Z_k = O.
-// The drivers below own this layout and run the existing impls on it: commit + prove, simulate, verify.  Arrays are
-// host arrays in the engine's proof-major layout; the only kernel of its own is the AND of the 1 + K verdicts.
+// The drivers below own this layout and run the existing impls on it: commit + prove, simulate, verify, and the randomised
+// per-statement check of verify.cu (gsi::zk_each_rand_dev).  Arrays are host arrays in the engine's proof-major layout; the
+// only kernel of its own is the AND of the 1 + K verdicts.
 #include <algorithm>
 #include <cstddef>
 
@@ -80,6 +81,63 @@ int zk_args(gs_ctx* ctx, const char* what, size_t count, size_t m, size_t n, siz
   return set ? GS_OK : GS_EARG;
 }
 
+
+// the host arrays of a verify call (proof-major)
+struct zk_host {
+  size_t m, n, K;
+  const gs_g1* a_consts;
+  const gs_com1* xcoms;
+  const gs_com2* ycoms;
+  const gs_com2* pi;
+  const gs_com1* theta;
+  const gs_com2* lin_pi;
+  const gs_com1* lin_theta;
+};
+
+// delta's commitment is never taken from the proof: W2 of the loaded CRS, once per call
+int crs_w2(gs_ctx* ctx, gs_com2* w2) {
+  CUDA_TRY(cudaMemcpyAsync(w2, &ctx->crs->w2[0], sizeof(*w2), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  return GS_OK;
+}
+
+// statements per upload: at most 4 verify passes of L_k, so that device scratch does not grow with the batch (C5 at
+// K = 1, 65,536 statements, is one chunk; within a chunk verify_impl alternates its passes between two streams)
+size_t zk_chunk(const gs_ctx* ctx, size_t K) { return std::max<size_t>(1, 4 * ctx->verify_batch_max / K); }
+
+// device copies of statements [off, off + cn) in the augmented layout, PPE''s target left out: PPE' (A, B, G, c, d, pi, th)
+// and the cn * K equations L_k (La, Lb, Lg, Lt = O, Lc, Ld = W2, Lpi, Lth)
+struct zk_dev {
+  g1_aff *A, *La, *Lt;
+  g2_aff *B, *Ld;
+  fr *G, *Lb, *Lg;
+  gs_com1 *c, *th, *Lc, *Lth;
+  gs_com2 *d, *pi, *Lpi;
+};
+int zk_upload(gs_ctx* ctx, Scratch& sc, const zk_host& h, const zk_layout& L, const gs_com2& w2, size_t off, size_t cn, zk_dev* d) {
+  const size_t m = h.m, n = h.n, K = h.K, mk = m + K, nl = cn * K;
+  const std::vector<gs_com2> lin_d(nl, w2);
+  const std::vector<gs_g1> origin(nl);
+  CUDA_TRY(upload(ctx, sc, &d->A, h.a_consts + off * n, cn * n));
+  CUDA_TRY(upload(ctx, sc, &d->B, L.b.data(), cn * mk));
+  CUDA_TRY(upload(ctx, sc, &d->G, L.gamma.data(), cn * mk * n));
+  CUDA_TRY(upload(ctx, sc, &d->c, h.xcoms + off * mk, cn * mk));
+  CUDA_TRY(upload(ctx, sc, &d->d, h.ycoms + off * n, cn * n));
+  CUDA_TRY(upload(ctx, sc, &d->pi, h.pi + off * 2, cn * 2));
+  CUDA_TRY(upload(ctx, sc, &d->th, h.theta + off * 2, cn * 2));
+  CUDA_TRY(upload(ctx, sc, &d->La, L.lin_a.data(), nl));
+  CUDA_TRY(upload(ctx, sc, &d->Lb, L.lin_b.data(), nl));
+  CUDA_TRY(upload(ctx, sc, &d->Lg, L.lin_gamma.data(), nl));
+  CUDA_TRY(upload(ctx, sc, &d->Lt, origin.data(), nl));
+  CUDA_TRY(upload(ctx, sc, &d->Ld, lin_d.data(), 2 * nl));
+  CUDA_TRY(upload(ctx, sc, &d->Lpi, h.lin_pi + off * K * 2, nl * 2));
+  CUDA_TRY(upload(ctx, sc, &d->Lth, h.lin_theta + off * K, nl));
+  // L_k's x-commitment is c_{m+k} of PPE': the last K commitments of every statement
+  CUDA_TRY(sc.alloc(&d->Lc, nl));
+  CUDA_TRY(cudaMemcpy2DAsync(d->Lc, K * sizeof(gs_com1), d->c + m, mk * sizeof(gs_com1), K * sizeof(gs_com1), cn,
+                             cudaMemcpyDeviceToDevice, ctx->stream));
+  return GS_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -145,55 +203,62 @@ int gs_zk_ppe_verify_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t
   if (int rc = zk_args(ctx, "zk_ppe_verify", count, m, n, K, set)) return rc;
   if (count == 0) return GS_OK;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  const size_t mk = m + K;
-  // delta's commitment is never taken from the proof: W2 of the loaded CRS, once per call
+  const zk_host h{m, n, K, a_consts, xcoms, ycoms, pi, theta, lin_pi, lin_theta};
   gs_com2 w2;
-  CUDA_TRY(cudaMemcpyAsync(&w2, &ctx->crs->w2[0], sizeof(w2), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  // statements per upload: at most 4 verify passes of L_k, so that device scratch does not grow with the batch (C5 at
-  // K = 1, 65,536 statements, is one chunk; within a chunk verify_impl alternates its passes between two streams)
-  const size_t chunk = std::max<size_t>(1, 4 * ctx->verify_batch_max / K);
+  if (int rc = crs_w2(ctx, &w2)) return rc;
+  const size_t mk = m + K, chunk = zk_chunk(ctx, K);
   for (size_t off = 0; off < count; off += chunk) {
     const size_t cn = std::min(chunk, count - off), nl = cn * K;
     const zk_layout L(cn, m, n, K, b_consts + off * m, gamma + off * m * n, tp + off * K, tq + off * K);
-    const std::vector<gs_com2> lin_d(nl, w2);
-    const std::vector<gs_g1> origin(nl);
     Scratch sc(ctx);
-    g1_aff *dA, *dLa, *dLt;
-    g2_aff *dB, *dLd;
+    zk_dev d;
+    if (int rc = zk_upload(ctx, sc, h, L, w2, off, cn, &d)) return rc;
     gs_gt* dT;
-    fr *dG, *dLb, *dLg;
-    gs_com1 *dc, *dth, *dLc, *dLth;
-    gs_com2 *dd, *dpi, *dLpi;
     uint8_t *ok_ppe, *ok_lin, *dok;
-    CUDA_TRY(upload(ctx, sc, &dA, a_consts + off * n, cn * n));
-    CUDA_TRY(upload(ctx, sc, &dB, L.b.data(), cn * mk));
-    CUDA_TRY(upload(ctx, sc, &dG, L.gamma.data(), cn * mk * n));
     CUDA_TRY(upload(ctx, sc, &dT, L.ones.data(), cn));
-    CUDA_TRY(upload(ctx, sc, &dc, xcoms + off * mk, cn * mk));
-    CUDA_TRY(upload(ctx, sc, &dd, ycoms + off * n, cn * n));
-    CUDA_TRY(upload(ctx, sc, &dpi, pi + off * 2, cn * 2));
-    CUDA_TRY(upload(ctx, sc, &dth, theta + off * 2, cn * 2));
-    CUDA_TRY(upload(ctx, sc, &dLa, L.lin_a.data(), nl));
-    CUDA_TRY(upload(ctx, sc, &dLb, L.lin_b.data(), nl));
-    CUDA_TRY(upload(ctx, sc, &dLg, L.lin_gamma.data(), nl));
-    CUDA_TRY(upload(ctx, sc, &dLt, origin.data(), nl));
-    CUDA_TRY(upload(ctx, sc, &dLd, lin_d.data(), 2 * nl));
-    CUDA_TRY(upload(ctx, sc, &dLpi, lin_pi + off * K * 2, nl * 2));
-    CUDA_TRY(upload(ctx, sc, &dLth, lin_theta + off * K, nl));
-    // L_k's x-commitment is c_{m+k} of PPE': the last K commitments of every statement
-    CUDA_TRY(sc.alloc(&dLc, nl));
-    CUDA_TRY(cudaMemcpy2DAsync(dLc, K * sizeof(gs_com1), dc + m, mk * sizeof(gs_com1), K * sizeof(gs_com1), cn,
-                               cudaMemcpyDeviceToDevice, ctx->stream));
     CUDA_TRY(sc.alloc(&ok_ppe, cn));
     CUDA_TRY(sc.alloc(&ok_lin, nl));
     CUDA_TRY(sc.alloc(&dok, cn));
-    int rc = verify_dev(ctx, GS_PPE, cn, mk, n, dA, dB, (const gs_fr*)dG, dT, dc, dd, dpi, dth, false, ok_ppe);
+    int rc = verify_dev(ctx, GS_PPE, cn, mk, n, d.A, d.B, (const gs_fr*)d.G, dT, d.c, d.d, d.pi, d.th, false, ok_ppe);
     if (rc) return rc;
     // every L_k has the y-commitment W2: its lines are walked once per pass
-    rc = verify_dev(ctx, GS_MSMEG1, nl, 1, 1, dLa, dLb, (const gs_fr*)dLg, dLt, dLc, (const gs_com2*)dLd, dLpi, dLth, true, ok_lin);
+    rc = verify_dev(ctx, GS_MSMEG1, nl, 1, 1, d.La, d.Lb, (const gs_fr*)d.Lg, d.Lt, d.Lc, (const gs_com2*)d.Ld, d.Lpi, d.Lth, true,
+                    ok_lin);
     if (rc) return rc;
     LAUNCH(k_zk_and, cn, ok_ppe, ok_lin, cn, (int)K, dok);
+    CUDA_TRY(cudaMemcpyAsync(out_ok + off, dok, cn, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  return GS_OK;
+}
+
+int gs_zk_ppe_verify_each_rand(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                               const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq, const gs_com1* xcoms,
+                               const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const gs_com2* lin_pi,
+                               const gs_com1* lin_theta, const uint64_t* rho, uint8_t* out_ok) {
+  const bool set =
+      a_consts && b_consts && gamma && tp && tq && xcoms && ycoms && pi && theta && lin_pi && lin_theta && rho && out_ok;
+  if (int rc = zk_args(ctx, "zk_ppe_verify_each_rand", count, m, n, K, set)) return rc;
+  if (count == 0) return GS_OK;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  const zk_host h{m, n, K, a_consts, xcoms, ycoms, pi, theta, lin_pi, lin_theta};
+  gs_com2 w2;
+  if (int rc = crs_w2(ctx, &w2)) return rc;
+  const size_t mk = m + K, chunk = zk_chunk(ctx, K);
+  // rho: PPE' of statement i at 2i, L_k at 2 count + 2(iK + k), beta last
+  const uint64_t *rho_lin = rho + 2 * count, *rho_beta = rho + 2 * count * (1 + K);
+  for (size_t off = 0; off < count; off += chunk) {
+    const size_t cn = std::min(chunk, count - off);
+    const zk_layout L(cn, m, n, K, b_consts + off * m, gamma + off * m * n, tp + off * K, tq + off * K);
+    Scratch sc(ctx);
+    zk_dev d;
+    uint8_t* dok;
+    if (int rc = zk_upload(ctx, sc, h, L, w2, off, cn, &d)) return rc;
+    CUDA_TRY(sc.alloc(&dok, cn));
+    int rc = zk_each_rand_dev(ctx, cn, mk, n, K, (const gs_g1*)d.A, (const gs_g2*)d.B, (const gs_fr*)d.G, d.c, d.d, d.pi, d.th,
+                              (const gs_g1*)d.La, (const gs_fr*)d.Lb, (const gs_fr*)d.Lg, (const gs_g1*)d.Lt, d.Lc,
+                              (const gs_com2*)d.Ld, d.Lpi, d.Lth, rho + 2 * off, rho_lin + 2 * off * K, rho_beta, dok);
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(out_ok + off, dok, cn, cudaMemcpyDeviceToHost, ctx->stream));
   }
   CUDA_TRY(cudaStreamSynchronize(ctx->stream));

@@ -17,7 +17,7 @@ EXPORTED_SYMBOLS = [
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
     "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_simulate", "gs_simulate_batch",
-    "gs_zk_ppe_prove_batch", "gs_zk_ppe_simulate_batch", "gs_zk_ppe_verify_batch", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_zk_ppe_prove_batch", "gs_zk_ppe_simulate_batch", "gs_zk_ppe_verify_batch", "gs_zk_ppe_verify_each_rand", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_each_rand", "gs_verify_each_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
@@ -83,6 +83,7 @@ def load_library():
         lib.gs_zk_ppe_prove_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 17
         lib.gs_zk_ppe_simulate_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 16
         lib.gs_zk_ppe_verify_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 12
+        lib.gs_zk_ppe_verify_each_rand.argtypes = [vp, sz, sz, sz, sz] + [vp] * 13
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_dev.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
         lib.gs_verify_batch_rand.argtypes = [vp, ci, sz, sz, sz] + [vp] * 10
@@ -389,6 +390,27 @@ class Engine:
         ok = ctypes.create_string_buffer(max(1, count))
         ks = [_buf(x) for x in named.values()]
         self._chk(self.lib.gs_zk_ppe_verify_batch(self.h, count, m, n, K, *[k[1] for k in ks], ctypes.cast(ok, ctypes.c_void_p)))
+        return ok.raw[:count]
+
+    def zk_ppe_verify_each_rand(self, count, m, n, K, a_consts, b_consts, gamma, tp, tq, xcoms, ycoms, pi, theta, lin_pi,
+                                lin_theta, rho=None) -> bytes:
+        """out_ok bytes of gs_zk_ppe_verify_each_rand: 1 iff statement i verifies (a bad statement passes with probability
+        <= 2^-62 over rho, each on its own).  rho is 2 * count * (1 + K) + 1 random 64-bit words (PPE' weights, then the
+        L_k weights, then beta), drawn from the OS CSPRNG unless the caller brings them; not bit-comparable with
+        zk_ppe_verify_batch."""
+        named = dict(a_consts=a_consts, b_consts=b_consts, gamma=gamma, tp=tp, tq=tq, xcoms=xcoms, ycoms=ycoms, pi=pi,
+                     theta=theta, lin_pi=lin_pi, lin_theta=lin_theta)
+        if count and m and n and K:
+            self._zk_sizes(count, m, n, K, named)
+        need = 8 * (2 * count * (1 + K) + 1)
+        if rho is None:
+            import secrets
+            rho = secrets.token_bytes(need)
+        if len(rho) != need:
+            raise GsError(1, f"zk_ppe_verify_each_rand: rho is {len(rho)} bytes, expected {need}")
+        ok = ctypes.create_string_buffer(max(1, count))
+        ks = [_buf(x) for x in (*named.values(), rho)]
+        self._chk(self.lib.gs_zk_ppe_verify_each_rand(self.h, count, m, n, K, *[k[1] for k in ks], ctypes.cast(ok, ctypes.c_void_p)))
         return ok.raw[:count]
 
     @staticmethod

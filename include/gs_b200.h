@@ -229,6 +229,25 @@ int gs_zk_ppe_verify_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t
                            const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
                            const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
                            const gs_com2* lin_pi, const gs_com1* lin_theta, uint8_t* out_ok);
+/* Randomised PER-STATEMENT verification of the same statements, an opt-in like gs_verify_each_rand: out_ok[i] = 1 iff
+ * statement i verifies, except with probability <= 2^-62 over `rho` for every bad statement on its own.  All 1 + K
+ * equations of statement i have target 1 (PPE' by construction, L_k with target O).  Every equation e gets weights of its
+ * own, (sigma_e, tau_e) = the low 63 bits of two words of rho, and the call one beta from a whole 64-bit word:
+ *   PPE' of statement i:  rho[2i], rho[2i + 1];
+ *   L_k of statement i:   rho[2 count + 2(iK + k)], rho[2 count + 2(iK + k) + 1];
+ *   beta:                 rho[2 count (1 + K)]            (rho has 2 count (1 + K) + 1 words).
+ * Each equation's slots are folded as gs_verify_each_rand folds them, and statement i is accepted iff
+ *     FE( prod over e in {PPE', L_1..L_K} of prod_k e( sigma_e X_k.0 + tau_e X_k.1 ,  beta Y_k.0 + Y_k.1 ) ) == 1
+ * -- one folded pairing product and ONE final exponentiation per statement, however large K is (csrc/verify.cu,
+ * "randomised per-statement verification of zk PPEs").  L_k's y-commitment is W2 of the loaded CRS, never an input.  A
+ * statement the exact check rejects passes only if a non-zero polynomial of degree 2 in the weights vanishes.  Arrays as
+ * for gs_zk_ppe_verify_batch; GS_EDIM for m, n or K = 0 or too many variables, GS_EARG for a null pointer (rho included)
+ * or no loaded CRS; count == 0 returns GS_OK and writes nothing.  An all-zero rho accepts everything (the check is then
+ * vacuous).  The verdicts are not bit-comparable with gs_zk_ppe_verify_batch's. */
+int gs_zk_ppe_verify_each_rand(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                               const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
+                               const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                               const gs_com2* lin_pi, const gs_com1* lin_theta, const uint64_t* rho, uint8_t* out_ok);
 
 /* ---- verification (src/verifier.rs)----------------------------------------------------- */
 /* Verifiable::verify :23-157 for `count` independent (equation, proof) instances of the same

@@ -86,6 +86,11 @@ extern "C" {
                                   gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, xcoms: *const GsCom1, ycoms: *const GsCom2,
                                   pi: *const GsCom2, theta: *const GsCom1, lin_pi: *const GsCom2, lin_theta: *const GsCom1,
                                   out_ok: *mut u8) -> i32;
+    // opt-in: ONE randomised verdict PER STATEMENT (rho: 2*count*(1 + K) + 1 words from the caller's CSPRNG)
+    pub fn gs_zk_ppe_verify_each_rand(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
+                                      gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, xcoms: *const GsCom1, ycoms: *const GsCom2,
+                                      pi: *const GsCom2, theta: *const GsCom1, lin_pi: *const GsCom2, lin_theta: *const GsCom1,
+                                      rho: *const u64, out_ok: *mut u8) -> i32;
     // verifier.rs:23-157
     pub fn gs_verify_batch(ctx: *mut GsCtx, ty: i32, count: usize, m: usize, n: usize, a: *const u8, b: *const u8,
                            gamma: *const GsFr, target: *const u8, xcoms: *const GsCom1, ycoms: *const GsCom2,

@@ -99,6 +99,18 @@ impl<E: Gpu> ZkPPE<E> {
 
     /// PPE' and every Z_k - delta P_k = O verify, delta's commitment being W2 of `crs`.
     pub fn verify(&self, proof: &ZkPPEProof<E>, crs: &CRS<E>) -> bool {
+        self.verify_with(proof, crs, None)
+    }
+
+    /// Not in the reference: the verdict of `verify` at close to the cost of one equation (gs_zk_ppe_verify_each_rand):
+    /// PPE' and the K equations are folded, each with its own weights from `rng` (a cryptographic RNG the prover cannot
+    /// predict), into one pairing product and ONE final exponentiation.  A bad proof is accepted with probability <= 2^-62.
+    pub fn verify_each_randomized(&self, proof: &ZkPPEProof<E>, crs: &CRS<E>, rng: &mut dyn ark_std::rand::RngCore) -> bool {
+        let rho: Vec<u64> = (0..2 * (1 + self.target_pairs.len()) + 1).map(|_| rng.next_u64()).collect();
+        self.verify_with(proof, crs, Some(&rho))
+    }
+
+    fn verify_with(&self, proof: &ZkPPEProof<E>, crs: &CRS<E>, rho: Option<&[u64]>) -> bool {
         let (m, n, k) = self.shape();
         assert_eq!((proof.xcoms.coms.len(), proof.ycoms.coms.len(), proof.lin.len()), (m + k, n, k));
         let (a, b, g, tp, tq) = self.statement();
@@ -111,8 +123,14 @@ impl<E: Gpu> ZkPPE<E> {
         assert_eq!((pi.len(), th.len(), lpi.len(), lth.len()), (2, 2, 2 * k, k));
         let mut ok = [0u8];
         with_crs(&crs.abi(), |c| check(c, unsafe {
-            gs_zk_ppe_verify_batch(c.raw(), 1, m, n, k, a.as_ptr(), b.as_ptr(), g.as_ptr(), tp.as_ptr(), tq.as_ptr(), xc.as_ptr(),
-                                   yc.as_ptr(), pi.as_ptr(), th.as_ptr(), lpi.as_ptr(), lth.as_ptr(), ok.as_mut_ptr())
+            match rho {
+                None => gs_zk_ppe_verify_batch(c.raw(), 1, m, n, k, a.as_ptr(), b.as_ptr(), g.as_ptr(), tp.as_ptr(), tq.as_ptr(),
+                                               xc.as_ptr(), yc.as_ptr(), pi.as_ptr(), th.as_ptr(), lpi.as_ptr(), lth.as_ptr(),
+                                               ok.as_mut_ptr()),
+                Some(r) => gs_zk_ppe_verify_each_rand(c.raw(), 1, m, n, k, a.as_ptr(), b.as_ptr(), g.as_ptr(), tp.as_ptr(),
+                                                      tq.as_ptr(), xc.as_ptr(), yc.as_ptr(), pi.as_ptr(), th.as_ptr(), lpi.as_ptr(),
+                                                      lth.as_ptr(), r.as_ptr(), ok.as_mut_ptr()),
+            }
         }));
         ok[0] == 1
     }
