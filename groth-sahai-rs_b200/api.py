@@ -429,6 +429,9 @@ class ZkPPE:
     def simulate(self, crs: CRS, key: SimulationKey, rng) -> "ZkPPEProof":
         return zk_simulate_batch([self], crs, key, rng)[0]
 
+    def rerandomize(self, proof: "ZkPPEProof", crs: CRS, rng) -> "ZkPPEProof":
+        return zk_rerandomize_batch([self], [proof], crs, rng)[0]
+
     def verify(self, proof: "ZkPPEProof", crs: CRS) -> bool:
         return zk_verify_batch([self], [proof], crs)[0]
 
@@ -505,6 +508,27 @@ def zk_simulate_batch(statements, crs: CRS, key: SimulationKey, rng) -> List[ZkP
     out = crs._use().zk_ppe_simulate_batch(
         len(statements), m, n, K, *arrays, cat(lambda d: _flat(d[0])), cat(lambda d: _flat(d[1])), cat(lambda d: _flat(d[2])),
         cat(lambda d: b"".join(_flat(t) for t in d[3])), key.to_bytes())
+    return _zk_proofs(out, draws, m, n, K, False)
+
+
+def zk_rerandomize_batch(statements, proofs, crs: CRS, rng) -> List[ZkPPEProof]:
+    """Fresh-looking ZkPPEProofs of the same statements from the proofs alone, real or simulated, without witnesses or
+    trapdoor (Belenkiy et al., CRYPTO 2009) in one GPU pass (gs_zk_ppe_rerandomize_batch): distributed exactly as fresh
+    zk_prove_batch output, so a presentation cannot be linked to the proof it came from.  Fresh randomness is drawn as for
+    zk_prove_batch: R' rows ((m + K) x 2), S' rows (n x 2), T' (2 x 2, row-major), then T'_1..T'_K (1 x 2 each).  The
+    input is not checked: a proof that does not verify still does not verify afterwards.  The returned Commit*.rand and
+    EquProof.rand are empty, as for rerandomize_batch."""
+    if len(proofs) != len(statements):
+        raise ValueError("zk_rerandomize_batch: one proof per statement")
+    if not statements:
+        return []
+    m, n, K, arrays = _zk_verify_arrays(statements, proofs, "zk_rerandomize_batch")
+    draws = _zk_draws(len(statements), m, n, K, rng)
+    cat = lambda f: b"".join(f(d) for d in draws)
+    a, b, g, _, tq, *coms = arrays
+    out = crs._use().zk_ppe_rerandomize_batch(
+        len(statements), m, n, K, a, b, g, tq, *coms, cat(lambda d: _flat(d[0])), cat(lambda d: _flat(d[1])),
+        cat(lambda d: _flat(d[2])), cat(lambda d: b"".join(_flat(t) for t in d[3])))
     return _zk_proofs(out, draws, m, n, K, False)
 
 

@@ -349,6 +349,12 @@ template <class F>
 int rerand_element(gs_ctx* ctx, Scratch& sc, size_t count, int rows, bool group_typed, const fr* sv, const fr* rg,
                    const void* dconst, size_t nconst, const Aff<F>* dcom, size_t ncom, bool coms_shared, int ncoef,
                    const fr* coef, const fr* e, const Aff<F>* dold, Aff<F>* dout);
+// out[i] = com[i] + s0[i * s0_stride] Base0 + s1[i * s1_stride] Base1 for n commitments of one group, both coordinates,
+// bases indexed as in the fixed-base tables (u1 u2 W1 / v1 v2 W2); device buffers (zk.cu: the linear equations of a
+// rerandomised zk PPE proof)
+template <class F>
+int fixed_com_add(gs_ctx* ctx, size_t n, int base0, int base1, const fr* s0, size_t s0_stride, const fr* s1, size_t s1_stride,
+                  const Aff<F>* dcom, Aff<F>* dout);
 template <class F>
 int com_matmul_impl(gs_ctx* ctx, size_t r, size_t k, size_t c, const gs_fr* lhs, const void* mat, void* out);
 
@@ -370,6 +376,12 @@ int theta_pi_fork(gs_ctx* ctx, bool two_streams, Theta&& theta, Pi&& pi) {
 int prove_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
                const gs_fr* gamma, const void* xvars, const void* yvars, const gs_fr* x_rand, const gs_fr* y_rand,
                const gs_fr* pf_rand, bool shared_vars, gs_com2* out_pi, gs_com1* out_theta);
+// prover.cu: `count` rerandomised committed proofs (gs_rerandomize_batch, host arrays; `shared`: one set of commitments and
+// of R', S' for every equation)
+int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                     const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,
+                     const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared, gs_com1* out_xcoms,
+                     gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta);
 // simulate.cu: `count` simulated proofs (gs_simulate_batch, host arrays), and the check of tkey against the loaded CRS
 // that gs_simulate_batch runs first (cached in ctx->tkey).  with_coms = false: the commitments of O / 0 are neither made nor
 // written (a caller that has them already); out_xcoms / out_ycoms may then be null

@@ -371,6 +371,8 @@ int gs_prove_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, cons
                     out_pi, out_theta);
 }
 
+}  // extern "C"
+
 // `count` rerandomisations of committed proofs, laid out as prove_impl's arrays (shared_coms: one set of commitments and
 // of R', S' for every equation).  With fresh R', S', T':
 //   c' = c + R' u_x                     d' = d + S' v_y
@@ -378,10 +380,10 @@ int gs_prove_batch(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, cons
 //   theta' = theta + S'^T iota_x(A) + (S'^T Gamma^T) c + T' u_x
 // -- exactly commit_and_prove of the same witnesses under R + R', S + S', T + T' + S'^T Gamma^T R.  The Fr algebra is
 // prove_impl's; the variable-base sums run over the commitments (both coordinates) instead of iota(variables).
-static int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
-                            const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
-                            const gs_com1* theta, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
-                            gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta) {
+int gsi::rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_t n, const void* a_consts, const void* b_consts,
+                          const gs_fr* gamma, const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi,
+                          const gs_com1* theta, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, bool shared,
+                          gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta) {
   if (!ctx) return GS_EARG;
   if (type < 0 || type > 3) FAIL(GS_EARG, "rerandomize: bad equation type");
   if (!ctx->crs_loaded) FAIL(GS_EARG, "rerandomize: no CRS loaded");
@@ -479,6 +481,8 @@ static int rerandomize_impl(gs_ctx* ctx, int type, size_t count, size_t m, size_
   }
   return GS_OK;
 }
+
+extern "C" {
 
 int gs_rerandomize(gs_ctx* ctx, int type, size_t m, size_t n, const void* a_consts, const void* b_consts, const gs_fr* gamma,
                    const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const gs_fr* x_rand,

@@ -10,5 +10,6 @@ template int proof_element<FpOps>(gs_ctx*, Scratch&, size_t, int, bool, const fr
 template int rerand_commit<FpOps>(gs_ctx*, size_t, int, const fr*, const Aff<FpOps>*, Aff<FpOps>*);
 template int rerand_element<FpOps>(gs_ctx*, Scratch&, size_t, int, bool, const fr*, const fr*, const void*, size_t,
                                 const Aff<FpOps>*, size_t, bool, int, const fr*, const fr*, const Aff<FpOps>*, Aff<FpOps>*);
+template int fixed_com_add<FpOps>(gs_ctx*, size_t, int, int, const fr*, size_t, const fr*, size_t, const Aff<FpOps>*, Aff<FpOps>*);
 template int com_matmul_impl<FpOps>(gs_ctx*, size_t, size_t, size_t, const gs_fr*, const void*, void*);
 }  // namespace gsi

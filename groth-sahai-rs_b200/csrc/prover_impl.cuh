@@ -376,6 +376,35 @@ __global__ void __launch_bounds__(GS_TAB_NT) k_rerand_commit(const Aff<F>* __res
   if (active) out[i * 2 + a] = r;
 }
 
+// out[i].p[a] = com[i].p[a] + s0_i Base0.a + s1_i Base1.a: a whole commitment plus two fixed-base products, the sibling of
+// k_fixed_commit (which adds iota(X) to coordinate 1 only and keeps its C2 register budget).  The linear equations
+// Z_k - delta P_k = O of a rerandomised zk PPE proof (zk.cu) are pi'_c = pi_c + R'_c W2 - T'_c v1 and
+// theta' = theta + T'_0 u1 + T'_1 u2: fixed-base terms only.
+template <class F>
+__global__ void __launch_bounds__(GS_TAB_NT) k_fixed_com_add(const Aff<F>* __restrict__ tab, int c, int W, size_t H, int base0,
+                                                             int base1, const fr* __restrict__ s0, size_t s0_stride,
+                                                             const fr* __restrict__ s1, size_t s1_stride,
+                                                             const Aff<F>* __restrict__ com, Aff<F>* __restrict__ out, size_t n) {
+  __shared__ fp sm[2 * GS_TAB_NT];
+  size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  bool active = id < 2 * n;
+  size_t i = active ? id >> 1 : 0;
+  int a = (int)(id & 1);
+  Jac<F> acc;
+  acc.set_inf();
+  if (active) {
+    acc.from_affine(com[i * 2 + a]);
+    uint32_t k[8];
+    fr_from_mont(k, s0[i * s0_stride]);
+    fixed_base_accumulate<F>(acc, tab + ((size_t)(base0 * 2 + a) * W) * H, k, c, W, H);
+    fr_from_mont(k, s1[i * s1_stride]);
+    fixed_base_accumulate<F>(acc, tab + ((size_t)(base1 * 2 + a) * W) * H, k, c, W, H);
+  }
+  Aff<F> r;
+  block_to_affine<GS_TAB_NT>(r, acc, sm);
+  if (active) out[i * 2 + a] = r;
+}
+
 // Variable-base products of a rerandomised proof element (pi': G2 over the constants B and the commitments d; theta': G1
 // over A and c).  Output row i has two coordinate rows:
 //   a = 1:  sum_{k < n0} sv[i][k] B_k + sum_j sv[i][c0 + j] com_j.1        (n0 = 0 on a scalar-typed side)
@@ -788,6 +817,17 @@ int rerand_commit(gs_ctx* ctx, size_t n, int ns, const fr* dR, const Aff<F>* dco
   if (rc) return rc;
   const gs_fixed_table<F>& T = table_of<F>(ctx);
   LAUNCH((k_rerand_commit<F>), 2 * n, T.t, T.c, T.W, T.H, dR, ns, dcom, dout, n);
+  return GS_OK;
+}
+
+// out[i] = com[i] + s0_i Base0 + s1_i Base1 for n commitments (k_fixed_com_add); device buffers
+template <class F>
+int fixed_com_add(gs_ctx* ctx, size_t n, int base0, int base1, const fr* s0, size_t s0_stride, const fr* s1, size_t s1_stride,
+                  const Aff<F>* dcom, Aff<F>* dout) {
+  int rc = fixed_table_for<F>(ctx, n);
+  if (rc) return rc;
+  const gs_fixed_table<F>& T = table_of<F>(ctx);
+  LAUNCH((k_fixed_com_add<F>), 2 * n, T.t, T.c, T.W, T.H, base0, base1, s0, s0_stride, s1, s1_stride, dcom, dout, n);
   return GS_OK;
 }
 

@@ -6,9 +6,10 @@
 // scalar y-variable delta has the FIXED commitment W2 = 1 W2 + 0 v[0], rebuilt by the verifier from its CRS.  Under a
 // binding CRS W2 binds delta = 1, so Z_k = P_k and PPE' is the original equation; under a hiding CRS W2 = t2 v[0] is also
 // the commitment of delta = 0 with randomness t2, which is how the simulator proves L_k with Z_k = O.
-// The drivers below own this layout and run the existing impls on it: commit + prove, simulate, verify, and the randomised
-// per-statement check of verify.cu (gsi::zk_each_rand_dev).  Arrays are host arrays in the engine's proof-major layout; the
-// only kernel of its own is the AND of the 1 + K verdicts.
+// The drivers below own this layout and run the existing impls on it: commit + prove, simulate, rerandomise, verify, and the
+// randomised per-statement check of verify.cu (gsi::zk_each_rand_dev).  Arrays are host arrays in the engine's proof-major
+// layout; the only kernel of its own is the AND of the 1 + K verdicts (the fixed-base sums of rerandomised L_k are
+// k_fixed_com_add of prover_impl.cuh).
 #include <algorithm>
 #include <cstddef>
 
@@ -41,11 +42,12 @@ struct zk_layout {
   std::vector<gs_g2> b;          // PPE': [count][m + K]     = B | -Q
   std::vector<gs_fr> gamma;      // PPE': [count][m + K][n]  = Gamma, then K zero rows
   std::vector<gs_gt> ones;       // PPE': [count]            target 1
-  std::vector<gs_g1> lin_a;      // L_k : [count][K]         -P_k
+  std::vector<gs_g1> lin_a;      // L_k : [count][K]         -P_k (left empty without tp: rerandomisation never reads it)
   std::vector<gs_fr> lin_b;      // L_k : [count][K]         1 (b, and delta of the real prover)
   std::vector<gs_fr> lin_gamma;  // L_k : [count][K]         0
   zk_layout(size_t count, size_t m, size_t n, size_t K, const gs_g2* b_consts, const gs_fr* gm, const gs_g1* tp, const gs_g2* tq)
-      : b(count * (m + K)), gamma(count * (m + K) * n), ones(count), lin_a(count * K), lin_b(count * K), lin_gamma(count * K) {
+      : b(count * (m + K)), gamma(count * (m + K) * n), ones(count), lin_a(tp ? count * K : 0), lin_b(count * K),
+        lin_gamma(count * K) {
     fp12 one12;
     one12.set_one();
     fr one;
@@ -56,7 +58,7 @@ struct zk_layout {
       memcpy(&ones[i], &one12, sizeof(gs_gt));
       for (size_t k = 0; k < K; k++) {
         b[i * (m + K) + m + k] = negated<Fp2Ops>(tq[i * K + k]);
-        lin_a[i * K + k] = negated<FpOps>(tp[i * K + k]);
+        if (tp) lin_a[i * K + k] = negated<FpOps>(tp[i * K + k]);
         memcpy(&lin_b[i * K + k], &one, sizeof(gs_fr));
       }
     }
@@ -138,6 +140,34 @@ int zk_upload(gs_ctx* ctx, Scratch& sc, const zk_host& h, const zk_layout& L, co
                              cudaMemcpyDeviceToDevice, ctx->stream));
   return GS_OK;
 }
+
+// The nl = count * K equations L_k of a rerandomised proof under R'_{m+k} (zr, [nl][2]) and T'_k (lin_rand, [nl][1][2]),
+// delta's fresh randomness 0.  With Gamma = 0 and b = [1], gs_rerandomize's formula leaves fixed-base terms only:
+//   lin_pi'_c = lin_pi_c + R'[m+k][c] W2 - T'_k[c] v[0]   (c = 0, 1)        lin_theta' = lin_theta + T'_k[0] u[0] + T'_k[1] u[1]
+// c_{m+k} is rerandomised with PPE'; W2 is neither recomputed nor output, and P_k is never read (its terms carry delta's 0).
+int lin_rerandomize(gs_ctx* ctx, size_t nl, const std::vector<gs_fr>& zr, const gs_fr* lin_rand, const gs_com2* lin_pi,
+                    const gs_com1* lin_theta, gs_com2* out_lin_pi, gs_com1* out_lin_theta) {
+  std::vector<gs_fr> neg_t(nl * 2);  // -T'_k[c] (r - x on the limbs; 0 stays 0)
+  for (size_t j = 0; j < nl * 2; j++) fr::neg(reinterpret_cast<fr&>(neg_t[j]), reinterpret_cast<const fr&>(lin_rand[j]));
+  Scratch sc(ctx);
+  fr *dz, *dnt, *dt;
+  g2_aff *dpi, *dpo;
+  g1_aff *dth, *dto;
+  CUDA_TRY(upload(ctx, sc, &dz, zr.data(), nl * 2));
+  CUDA_TRY(upload(ctx, sc, &dnt, neg_t.data(), nl * 2));
+  CUDA_TRY(upload(ctx, sc, &dt, lin_rand, nl * 2));
+  CUDA_TRY(upload(ctx, sc, &dpi, lin_pi, nl * 2 * 2));
+  CUDA_TRY(upload(ctx, sc, &dth, lin_theta, nl * 2));
+  CUDA_TRY(sc.alloc(&dpo, nl * 2 * 2));
+  CUDA_TRY(sc.alloc(&dto, nl * 2));
+  // pi: 2 nl Com2 (c = 0, 1 of every L_k) with bases W2 (2) and v[0] (0); theta: nl Com1 with bases u[0] (0), u[1] (1)
+  if (int rc = fixed_com_add<Fp2Ops>(ctx, nl * 2, 2, 0, dz, 1, dnt, 1, dpi, dpo)) return rc;
+  if (int rc = fixed_com_add<FpOps>(ctx, nl, 0, 1, dt, 2, dt + 1, 2, dth, dto)) return rc;
+  CUDA_TRY(cudaMemcpyAsync(out_lin_pi, dpo, nl * 2 * sizeof(gs_com2), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaMemcpyAsync(out_lin_theta, dto, nl * sizeof(gs_com1), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  return GS_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -194,6 +224,25 @@ int gs_zk_ppe_simulate_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size
   const std::vector<gs_g1> origin(count * K);
   return simulate_impl(ctx, GS_MSMEG1, count * K, 1, 1, L.lin_a.data(), L.lin_b.data(), L.lin_gamma.data(), origin.data(), zr.data(),
                        t2.data(), lin_rand, false, tkey, nullptr, nullptr, out_lin_pi, out_lin_theta, false);
+}
+
+int gs_zk_ppe_rerandomize_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                                const gs_g2* b_consts, const gs_fr* gamma, const gs_g2* tq, const gs_com1* xcoms,
+                                const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const gs_com2* lin_pi,
+                                const gs_com1* lin_theta, const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand,
+                                const gs_fr* lin_rand, gs_com1* out_xcoms, gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta,
+                                gs_com2* out_lin_pi, gs_com1* out_lin_theta) {
+  const bool set = a_consts && b_consts && gamma && tq && xcoms && ycoms && pi && theta && lin_pi && lin_theta && x_rand && y_rand &&
+                   pf_rand && lin_rand && out_xcoms && out_ycoms && out_pi && out_theta && out_lin_pi && out_lin_theta;
+  if (int rc = zk_args(ctx, "zk_ppe_rerandomize", count, m, n, K, set)) return rc;
+  if (count == 0) return GS_OK;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  const zk_layout L(count, m, n, K, b_consts, gamma, nullptr, tq);
+  // PPE': gs_rerandomize_batch of the augmented statement under R', S', T' -- c_{m+k} included
+  int rc = rerandomize_impl(ctx, GS_PPE, count, m + K, n, a_consts, L.b.data(), L.gamma.data(), xcoms, ycoms, pi, theta, x_rand,
+                            y_rand, pf_rand, false, out_xcoms, out_ycoms, out_pi, out_theta);
+  if (rc) return rc;
+  return lin_rerandomize(ctx, count * K, z_rand(x_rand, count, m, K), lin_rand, lin_pi, lin_theta, out_lin_pi, out_lin_theta);
 }
 
 int gs_zk_ppe_verify_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts, const gs_g2* b_consts,

@@ -17,7 +17,7 @@ EXPORTED_SYMBOLS = [
     "gs_crs_generate", "gs_crs_load",
     "gs_batch_commit_g1", "gs_batch_commit_g2", "gs_batch_commit_scalar_b1", "gs_batch_commit_scalar_b2",
     "gs_prove", "gs_prove_batch", "gs_rerandomize", "gs_rerandomize_batch", "gs_extract", "gs_simulate", "gs_simulate_batch",
-    "gs_zk_ppe_prove_batch", "gs_zk_ppe_simulate_batch", "gs_zk_ppe_verify_batch", "gs_zk_ppe_verify_each_rand", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
+    "gs_zk_ppe_prove_batch", "gs_zk_ppe_simulate_batch", "gs_zk_ppe_rerandomize_batch", "gs_zk_ppe_verify_batch", "gs_zk_ppe_verify_each_rand", "gs_verify_batch", "gs_verify_batch_dev", "gs_verify_batch_rand", "gs_verify_batch_rand_dev",
     "gs_verify_each_rand", "gs_verify_each_rand_dev",
     "gs_verify_partial", "gs_verify_partial_dev", "gs_verify_finish", "gs_verify_finish_dev", "gs_verify_sharded",
     "gs_comt_pairing", "gs_comt_pairing_sum", "gs_comt_linear_map", "gs_pairing",
@@ -82,6 +82,7 @@ def load_library():
         lib.gs_simulate_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 7 + [ci] + [vp] * 5
         lib.gs_zk_ppe_prove_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 17
         lib.gs_zk_ppe_simulate_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 16
+        lib.gs_zk_ppe_rerandomize_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 20
         lib.gs_zk_ppe_verify_batch.argtypes = [vp, sz, sz, sz, sz] + [vp] * 12
         lib.gs_zk_ppe_verify_each_rand.argtypes = [vp, sz, sz, sz, sz] + [vp] * 13
         lib.gs_verify_batch.argtypes = [vp, ci, sz, sz, sz] + [vp] * 9
@@ -356,7 +357,7 @@ class Engine:
                 raise GsError(1, f"zk_ppe: {nm} is {len(buf)} bytes, expected {w} for count {count}, m {m}, n {n}, K {K}")
 
     def _zk_proofs(self, fn, count, m, n, K, named):
-        """call gs_zk_ppe_prove_batch / _simulate_batch; (xcoms, ycoms, pi, theta, lin_pi, lin_theta) bytes"""
+        """call gs_zk_ppe_prove_batch / _simulate_batch / _rerandomize_batch; (xcoms, ycoms, pi, theta, lin_pi, lin_theta) bytes"""
         if count and m and n and K:
             self._zk_sizes(count, m, n, K, named)
         sizes = [count * k for k in ((m + K) * COM1, n * COM2, 2 * COM2, 2 * COM1, K * 2 * COM2, K * COM1)]
@@ -379,6 +380,15 @@ class Engine:
         return self._zk_proofs(self.lib.gs_zk_ppe_simulate_batch, count, m, n, K, dict(
             a_consts=a_consts, b_consts=b_consts, gamma=gamma, tp=tp, tq=tq, x_rand=x_rand, y_rand=y_rand, pf_rand=pf_rand,
             lin_rand=lin_rand, tkey=tkey))
+
+    def zk_ppe_rerandomize_batch(self, count, m, n, K, a_consts, b_consts, gamma, tq, xcoms, ycoms, pi, theta, lin_pi,
+                                 lin_theta, x_rand, y_rand, pf_rand, lin_rand):
+        """`count` zero-knowledge proofs rerandomised without the witness (gs_zk_ppe_rerandomize_batch) with fresh R' = x_rand,
+        S' = y_rand, T' = pf_rand and T'_k = lin_rand, laid out as for zk_ppe_prove_batch; the target pairs' P_k are not
+        needed.  Returns (xcoms, ycoms, pi, theta, lin_pi, lin_theta) bytes, proof-major."""
+        return self._zk_proofs(self.lib.gs_zk_ppe_rerandomize_batch, count, m, n, K, dict(
+            a_consts=a_consts, b_consts=b_consts, gamma=gamma, tq=tq, xcoms=xcoms, ycoms=ycoms, pi=pi, theta=theta,
+            lin_pi=lin_pi, lin_theta=lin_theta, x_rand=x_rand, y_rand=y_rand, pf_rand=pf_rand, lin_rand=lin_rand))
 
     def zk_ppe_verify_batch(self, count, m, n, K, a_consts, b_consts, gamma, tp, tq, xcoms, ycoms, pi, theta, lin_pi,
                             lin_theta) -> bytes:

@@ -225,6 +225,31 @@ int gs_zk_ppe_simulate_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size
                              const gs_fr* x_rand, const gs_fr* y_rand, const gs_fr* pf_rand, const gs_fr* lin_rand,
                              const gs_fr* tkey /* [2] = t1, t2 */, gs_com1* out_xcoms, gs_com2* out_ycoms,
                              gs_com2* out_pi, gs_com1* out_theta, gs_com2* out_lin_pi, gs_com1* out_lin_theta);
+/* Rerandomisation of zero-knowledge PPE proofs without the witness (Belenkiy et al., CRYPTO 2009; PAPERS.md): whoever
+ * holds a proof of the statements above -- real or simulated -- turns it into a fresh-looking proof of the same statement.
+ * With fresh R' = x_rand[count][m+K][2], S' = y_rand[count][n][2], T' = pf_rand[count][2][2] and T'_k =
+ * lin_rand[count][K][1][2] (the layouts of gs_zk_ppe_prove_batch):
+ *   PPE'  gs_rerandomize_batch of the augmented statement (b' = B | -Q, Gamma' = Gamma + K zero rows) under R', S', T';
+ *         this moves c_{m+k}, the x-commitment L_k shares, by row m+k of R'.
+ *   L_k   delta's fresh randomness is 0 (its commitment stays W2, which the verifier takes from the CRS), so with
+ *         Gamma = 0 and b = [1] only fixed-base terms remain:
+ *           lin_pi'_c  = lin_pi_c + R'[m+k][c] W2 - T'_k[c] v[0]   (c = 0, 1)
+ *           lin_theta' = lin_theta + T'_k[0] u[0] + T'_k[1] u[1]
+ * P_k is multiplied by delta's fresh randomness only, so tp is not an argument.  The output is byte for byte what
+ * gs_zk_ppe_prove_batch of the same witnesses makes under R + R', S + S', T + T' + S'^T Gamma'^T R and T_k + T'_k; for a
+ * simulated input, what gs_zk_ppe_simulate_batch makes under the same combined randomness (delta's randomness still t2).
+ * With uniform fresh randomness the output is distributed exactly as a fresh zk proof, so real and simulated proofs stay
+ * indistinguishable.  Rerandomisation does NOT validate its input: a proof that fails verification still fails
+ * afterwards (the verification error is unchanged).  No trapdoor is needed; binding and hiding CRSs alike.  Arrays and
+ * return codes as gs_zk_ppe_prove_batch (inputs under the verify names, outputs under out_); count == 0 returns GS_OK
+ * and writes nothing. */
+int gs_zk_ppe_rerandomize_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
+                                const gs_g2* b_consts, const gs_fr* gamma, const gs_g2* tq, const gs_com1* xcoms,
+                                const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta, const gs_com2* lin_pi,
+                                const gs_com1* lin_theta, const gs_fr* x_rand, const gs_fr* y_rand,
+                                const gs_fr* pf_rand, const gs_fr* lin_rand, gs_com1* out_xcoms,
+                                gs_com2* out_ycoms, gs_com2* out_pi, gs_com1* out_theta, gs_com2* out_lin_pi,
+                                gs_com1* out_lin_theta);
 int gs_zk_ppe_verify_batch(gs_ctx* ctx, size_t count, size_t m, size_t n, size_t K, const gs_g1* a_consts,
                            const gs_g2* b_consts, const gs_fr* gamma, const gs_g1* tp, const gs_g2* tq,
                            const gs_com1* xcoms, const gs_com2* ycoms, const gs_com2* pi, const gs_com1* theta,

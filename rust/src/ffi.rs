@@ -82,6 +82,13 @@ extern "C" {
                                     pf_rand: *const GsFr, lin_rand: *const GsFr, tkey: *const GsFr, out_xcoms: *mut GsCom1,
                                     out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1, out_lin_pi: *mut GsCom2,
                                     out_lin_theta: *mut GsCom1) -> i32;
+    // not in the reference: zk proofs rerandomised without the witness (fresh x_rand, y_rand, pf_rand, lin_rand as for prove)
+    pub fn gs_zk_ppe_rerandomize_batch(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
+                                       gamma: *const GsFr, tq: *const GsG2, xcoms: *const GsCom1, ycoms: *const GsCom2,
+                                       pi: *const GsCom2, theta: *const GsCom1, lin_pi: *const GsCom2, lin_theta: *const GsCom1,
+                                       x_rand: *const GsFr, y_rand: *const GsFr, pf_rand: *const GsFr, lin_rand: *const GsFr,
+                                       out_xcoms: *mut GsCom1, out_ycoms: *mut GsCom2, out_pi: *mut GsCom2, out_theta: *mut GsCom1,
+                                       out_lin_pi: *mut GsCom2, out_lin_theta: *mut GsCom1) -> i32;
     pub fn gs_zk_ppe_verify_batch(ctx: *mut GsCtx, count: usize, m: usize, n: usize, k: usize, a: *const GsG1, b: *const GsG2,
                                   gamma: *const GsFr, tp: *const GsG1, tq: *const GsG2, xcoms: *const GsCom1, ycoms: *const GsCom2,
                                   pi: *const GsCom2, theta: *const GsCom1, lin_pi: *const GsCom2, lin_theta: *const GsCom1,

@@ -2,7 +2,8 @@
 //! sum_k e(P_k, Q_k) (Groth & Sahai, EUROCRYPT 2008).  The statement is augmented to a target-1 PPE' over (X | Z) with
 //! constants (B | -Q) and K equations Z_k - delta P_k = O whose delta has the fixed commitment W2 (include/gs_b200.h,
 //! `gs_zk_ppe_prove_batch`).  `prove` makes real proofs, `simulate` makes proofs for any target pairs with the hiding
-//! CRS's trapdoor, `verify` checks both; real and simulated proofs are identically distributed under a hiding CRS.
+//! CRS's trapdoor, `verify` checks both, `rerandomize` refreshes either without witness or trapdoor; real and simulated
+//! proofs are identically distributed under a hiding CRS.
 use crate::data_structures::{Com1, Com2};
 use crate::ffi::*;
 use crate::generator::CRS;
@@ -97,6 +98,34 @@ impl<E: Gpu> ZkPPE<E> {
         self.proof(d, o, false)
     }
 
+    /// Not in the reference: a fresh-looking proof of the same statement from `proof` alone, real or simulated, without
+    /// witness or trapdoor (Belenkiy et al., CRYPTO 2009; gs_zk_ppe_rerandomize_batch).  Fresh randomness is drawn as for
+    /// `prove`; the openings are not returned.  The input is not checked: a proof that fails `verify` still fails.
+    pub fn rerandomize<R: Rng>(&self, proof: &ZkPPEProof<E>, crs: &CRS<E>, rng: &mut R) -> ZkPPEProof<E> {
+        let (m, n, k) = self.shape();
+        assert_eq!((proof.xcoms.coms.len(), proof.ycoms.coms.len(), proof.lin.len()), (m + k, n, k));
+        let (a, b, g, _, tq) = self.statement();
+        let (xc, yc, pi, th, lpi, lth) = Self::proof_abi(proof);
+        assert_eq!((pi.len(), th.len(), lpi.len(), lth.len()), (2, 2, 2 * k, k));
+        let d = self.draws(rng);
+        let r: Vec<Vec<GsFr>> = d.iter().map(|mat| fr_matrix::<E>(mat)).collect();
+        let mut o = self.outs();
+        with_crs(&crs.abi(), |c| check(c, unsafe {
+            gs_zk_ppe_rerandomize_batch(c.raw(), 1, m, n, k, a.as_ptr(), b.as_ptr(), g.as_ptr(), tq.as_ptr(), xc.as_ptr(),
+                                        yc.as_ptr(), pi.as_ptr(), th.as_ptr(), lpi.as_ptr(), lth.as_ptr(), r[0].as_ptr(),
+                                        r[1].as_ptr(), r[2].as_ptr(), r[3].as_ptr(), o.0.as_mut_ptr(), o.1.as_mut_ptr(),
+                                        o.2.as_mut_ptr(), o.3.as_mut_ptr(), o.4.as_mut_ptr(), o.5.as_mut_ptr())
+        }));
+        self.proof(d, o, false)
+    }
+
+    fn proof_abi(proof: &ZkPPEProof<E>) -> (Vec<GsCom1>, Vec<GsCom2>, Vec<GsCom2>, Vec<GsCom1>, Vec<GsCom2>, Vec<GsCom1>) {
+        (proof.xcoms.coms.iter().map(|c| c.abi()).collect(), proof.ycoms.coms.iter().map(|c| c.abi()).collect(),
+         proof.ppe.pi.iter().map(|c| c.abi()).collect(), proof.ppe.theta.iter().map(|c| c.abi()).collect(),
+         proof.lin.iter().flat_map(|e| e.pi.iter().map(|c| c.abi())).collect(),
+         proof.lin.iter().flat_map(|e| e.theta.iter().map(|c| c.abi())).collect())
+    }
+
     /// PPE' and every Z_k - delta P_k = O verify, delta's commitment being W2 of `crs`.
     pub fn verify(&self, proof: &ZkPPEProof<E>, crs: &CRS<E>) -> bool {
         self.verify_with(proof, crs, None)
@@ -114,12 +143,7 @@ impl<E: Gpu> ZkPPE<E> {
         let (m, n, k) = self.shape();
         assert_eq!((proof.xcoms.coms.len(), proof.ycoms.coms.len(), proof.lin.len()), (m + k, n, k));
         let (a, b, g, tp, tq) = self.statement();
-        let xc: Vec<GsCom1> = proof.xcoms.coms.iter().map(|c| c.abi()).collect();
-        let yc: Vec<GsCom2> = proof.ycoms.coms.iter().map(|c| c.abi()).collect();
-        let pi: Vec<GsCom2> = proof.ppe.pi.iter().map(|c| c.abi()).collect();
-        let th: Vec<GsCom1> = proof.ppe.theta.iter().map(|c| c.abi()).collect();
-        let lpi: Vec<GsCom2> = proof.lin.iter().flat_map(|e| e.pi.iter().map(|c| c.abi())).collect();
-        let lth: Vec<GsCom1> = proof.lin.iter().flat_map(|e| e.theta.iter().map(|c| c.abi())).collect();
+        let (xc, yc, pi, th, lpi, lth) = Self::proof_abi(proof);
         assert_eq!((pi.len(), th.len(), lpi.len(), lth.len()), (2, 2, 2 * k, k));
         let mut ok = [0u8];
         with_crs(&crs.abi(), |c| check(c, unsafe {
